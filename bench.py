@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- train samples/sec (fwd + BPTT), ALIF 784-128-10 recurrent, batch 256 per GPU, T = 100.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 One step = one pass of the hot path over one batch: input projection, fused recurrence + readout, fused
 max-over-time/log-softmax/NLL head, reverse-time BPTT, weight-gradient contraction, [gradient all-reduce],
@@ -15,6 +15,10 @@ Adam step (reference snn.py:384-415).  Reported on the ONE JSON line:
 
 --impl reference times that CPU restatement alone (the reference itself is pure Python and cannot travel to the
 GPU box; oracle/torch_port.py is pinned against it by tests/test_oracle_golden.py).
+
+--dump-outputs DIR writes what the timed resident step handed its caller after the last of the K timed steps -- the
+batch loss and every updated parameter -- as DIR/<name>.npy (float32).  Inputs and initial weights are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -140,7 +144,11 @@ def main():
 	ap.add_argument("--no-large-batch", action="store_true")
 	ap.add_argument("--no-configs", action="store_true", help="skip the c1/c3/c4/c5 sub-lines")
 	ap.add_argument("--quick-sweep", action="store_true", help="c5: ALIF and T in {10, 100} only")
+	ap.add_argument("--dump-outputs", metavar="DIR",
+		help="write the loss and the parameters after the last timed step as DIR/<name>.npy")
 	args = ap.parse_args()
+	if args.steps < 1:
+		ap.error("--steps must be at least 1")
 	args.warmup = max(args.warmup, 3)
 
 	rank = int(os.environ.get("RANK", "0"))
@@ -214,6 +222,8 @@ def main():
 		step_resident(i)        # the first NVML query returns (a 30 ms timed region alone sometimes caught a single sample)
 	ms = timed(step_resident, args.steps)
 	clocks = sampler.stop()
+	if args.dump_outputs and rank == 0:      # before the measurements below train the same network further
+		dump_outputs(args.dump_outputs, graphs[(args.steps - 1) % N_POOL].loss, net)
 	timeline = None
 	if dp_fused:     # last resident step on every rank, rank-local device clocks, us since kernel start
 		timeline = [None] * world
@@ -650,6 +660,15 @@ def large_batch_rooflines(net, enc, dev, B=4096, iters=5):
 	out["bit_packed_input"] = bits
 	del xb
 	return out
+
+
+def dump_outputs(out_dir, loss, net):
+	"""The last timed step's batch loss and the parameters its Adam update left, one float32 .npy file each."""
+	os.makedirs(out_dir, exist_ok=True)
+	arrays = {"loss": loss.detach().reshape(1)}
+	arrays.update({f"param.{name}": p.detach() for name, p in net.named_parameters()})
+	for name, t in arrays.items():
+		np.save(os.path.join(out_dir, f"{name}.npy"), t.float().cpu().numpy())
 
 
 def finish(world):

@@ -247,14 +247,19 @@ def test_packed_raster_tagging_and_passthrough():
 		fp32._encode_if_needed(torch.zeros(2, 5, 25, dtype=torch.int32))
 
 
-def test_bench_parses_the_committed_ncu_summary():
-	"""bench.py takes `roofline.traffic` / `roofline.smem_frac` from profiles/r02_ncu_full_summary.csv (unit row respected):
-	the headline kernels' rows must be found (lean kernels first) and carry sane numbers."""
+def _bench_module():
 	import importlib.util
 	root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 	spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(root, "bench.py"))
 	bench = importlib.util.module_from_spec(spec)
 	spec.loader.exec_module(bench)
+	return bench
+
+
+def test_bench_parses_the_committed_ncu_summary():
+	"""bench.py takes `roofline.traffic` / `roofline.smem_frac` from profiles/r02_ncu_full_summary.csv (unit row respected):
+	the headline kernels' rows must be found (lean kernels first) and carry sane numbers."""
+	bench = _bench_module()
 	k3 = bench.ncu_evidence("K3")
 	assert k3 is not None and "k_recur_bwd_lean" in k3["kernel"]
 	assert 20e6 < k3["traffic"] < 60e6                     # bytes per launch: V, a read once (26 MB), gI mostly stays in L2
@@ -265,3 +270,19 @@ def test_bench_parses_the_committed_ncu_summary():
 	assert bench.ncu_evidence("K1") is not None and bench.ncu_evidence("nope") is None
 	flops, byts = bench.per_sample_work(128, True, True, True)
 	assert abs(flops - 50.7e6) < 0.5e6 and abs(byts - 942e3) < 5e3      # SURVEY.md 8d: c2 = 50.7 MFLOP, 942 KB per sample
+
+
+def test_bench_dump_outputs_writes_loss_and_parameters(tmp_path):
+	"""bench.py --dump-outputs: the loss and every parameter, one float32 .npy file each, values unchanged."""
+	bench = _bench_module()
+	torch.manual_seed(0)
+	net = SNN(20, 10, 24, hidden_layer_type=LayerType.ALIF, use_recurrent_connection=True, learn_beta=True, device=CPU,
+		int_time_steps=5)
+	out = tmp_path / "out"
+	bench.dump_outputs(str(out), torch.tensor(1.25), net)
+	params = dict(net.named_parameters())
+	assert sorted(os.listdir(out)) == sorted(["loss.npy"] + [f"param.{n}.npy" for n in params])
+	assert np.load(out / "loss.npy").tolist() == [1.25]
+	for n, p in params.items():
+		a = np.load(out / f"param.{n}.npy")
+		assert a.dtype == np.float32 and np.array_equal(a, p.detach().numpy()), n
