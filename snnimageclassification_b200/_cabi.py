@@ -23,6 +23,7 @@ SNNK_LIF, SNNK_ALIF, SNNK_IZHIKEVICH = 0, 1, 2
 SNNK_FAST_SIGMOID, SNNK_PHI = 0, 1
 SNNK_F32, SNNK_F64, SNNK_U8, SNNK_I64, SNNK_BITS = 0, 1, 2, 3, 4
 SNNK_F_TRACES, SNNK_F_TENSOR_CORE, SNNK_F_INPUT_BINARY, SNNK_F_INPUT_BITS, SNNK_F_RUNS_TILED = 0x1, 0x2, 0x4, 0x8, 0x10
+SNNK_MAX_CLASSES = 16   # widest readout the kernels take (SnnkDesc.O <= 16, kOMax in csrc/common.cuh)
 
 NVCC_FLAGS = [
 	"-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

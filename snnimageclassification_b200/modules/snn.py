@@ -88,6 +88,11 @@ class SNN(torch.nn.Module):
 			**kwargs
 	):
 		super().__init__()
+		# the fused readout / head kernels hold the class dimension in 16 lanes: refuse a wider readout here rather
+		# than at the first forward call
+		if not 1 <= int(output_size) <= _cabi.SNNK_MAX_CLASSES:
+			raise ValueError(f"output_size={output_size}: the B200 kernels support readouts of 1 to "
+				f"{_cabi.SNNK_MAX_CLASSES} classes")
 		self.input_size = inputs_size
 		self.output_size = output_size
 		# keywords of the B200 build; everything else is threaded to the layers exactly as in the reference

@@ -99,6 +99,14 @@ def test_no_cpu_fallback():
 	assert float(V.min()) == float(V.max()) == -60.0 and float(u.abs().max()) == 0.0 and float(Z.abs().max()) == 0.0
 
 
+def test_readout_wider_than_16_classes_is_refused_at_construction():
+	for O in (1, 16):
+		assert SNN(16, O, 32, device=CPU, int_time_steps=4).layers["readout"].forward_weights.shape == (32, O)
+	for O in (17, 0):
+		with pytest.raises(ValueError, match="1 to 16 classes"):
+			SNN(16, O, 32, device=CPU, int_time_steps=4)
+
+
 def test_format_inputs():
 	net = SNN(6, 10, 32, device=CPU, int_time_steps=5)
 	x = torch.arange(12, dtype=torch.float64).reshape(2, 6)
