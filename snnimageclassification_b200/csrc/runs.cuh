@@ -289,20 +289,6 @@ __global__ void __launch_bounds__(256) k_gather_rows_tiled(const float* __restri
     }
 }
 
-// I_in[row] = I_u[compact(row)]: H/4 threads per dense row
-__global__ void __launch_bounds__(256) k_expand_rows(const float* __restrict__ Iu, const int* __restrict__ table, int BT,
-                                                    int H, float* __restrict__ I_in)
-{
-    if (table[1] != 1) return;
-    const int per_row = H / 4;
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long row = idx / per_row;
-    if (row >= BT) return;
-    const int q = (int)(idx - row * per_row);
-    const int r = table[kRunHdr + row];
-    reinterpret_cast<float4*>(I_in + (size_t)row * H)[q] = __ldg(reinterpret_cast<const float4*>(Iu + (size_t)r * H) + q);
-}
-
 // The run sums of gI (compact rows of the dW_in contraction) are produced by the BPTT sweep itself: recur_bwd.cuh.
 
 }  // namespace snnk

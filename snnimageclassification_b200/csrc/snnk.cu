@@ -9,6 +9,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <algorithm>
+#include <type_traits>
 
 #include "common.cuh"
 #include "encode_head.cuh"
@@ -65,33 +66,93 @@ struct ProfScope {
     ~ProfScope() { if (slot >= 0) cudaEventRecord(g_prof[slot].b, st); }
 };
 
+// Set the kernel's dynamic shared-memory limit (when it uses any), launch it inside the profiler bracket `id` and
+// check the launch.
+template <class... P, class... A>
+int launch(int id, void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, const A&... args)
+{
+    if (smem) SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    { ProfScope ps(id, st); kern<<<grid, block, smem, st>>>(args...); }
+    SNNK_CUDA(cudaGetLastError());
+    return SNNK_OK;
+}
+
 // Fork / join onto a helper stream (one per device, created on first use) so that two independent kernels of one call
 // overlap.  Event record / wait are legal during stream capture: the helper stream joins the capture and the graph
-// gets two parallel branches.  The call still returns with everything ordered behind the caller's stream.
+// gets two parallel branches.  The call still returns with everything ordered behind the caller's stream.  A call
+// with parallel work has no serial form: it fails if the helper stream cannot be had.
 struct Fork {
     cudaStream_t side = nullptr;
     cudaEvent_t forked = nullptr, joined = nullptr, mid = nullptr, forked2 = nullptr, forked3 = nullptr, joined3 = nullptr;
     bool ok = false;
 };
-Fork* fork_for_device()
+int fork_for_device(Fork** out)
 {
     static Fork forks[64];
-    static const char* env = getenv("SNNK_FORK");
-    if (env && env[0] == '0') return nullptr;
     int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess && (dev < 0 || dev >= 64)) e = cudaErrorInvalidDevice;
+    if (e != cudaSuccess) return cuda_fail(e, "helper stream for the parallel branches of the call");
     Fork& f = forks[dev];
     if (!f.ok) {
-        if (cudaStreamCreateWithFlags(&f.side, cudaStreamNonBlocking) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.forked, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.joined, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.mid, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.forked2, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.forked3, cudaEventDisableTiming) != cudaSuccess) return nullptr;
-        if (cudaEventCreateWithFlags(&f.joined3, cudaEventDisableTiming) != cudaSuccess) return nullptr;
+        e = cudaStreamCreateWithFlags(&f.side, cudaStreamNonBlocking);
+        for (cudaEvent_t* ev : {&f.forked, &f.joined, &f.mid, &f.forked2, &f.forked3, &f.joined3})
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(ev, cudaEventDisableTiming);
+        if (e != cudaSuccess) return cuda_fail(e, "creating the helper stream for the parallel branches of the call");
         f.ok = true;
     }
-    return &f;
+    *out = &f;
+    return SNNK_OK;
+}
+
+// Measuring switches ("0" turns a default off, anything else on), read on every call so that one process can compare
+// kernel families: SNNK_LEAN (lean recurrence kernels) and SNNK_MMA_RECUR (tensor-core recurrence at any batch).
+bool env_switch(const char* name, bool dflt)
+{
+    const char* env = getenv(name);
+    return env ? env[0] != '0' : dflt;
+}
+
+// Run-time values -> template arguments.  Each selector lists every instantiation its callers are built with.
+template <int V> using Int = std::integral_constant<int, V>;
+template <bool V> using Bool = std::integral_constant<bool, V>;
+
+template <class F> int by_width(int w, F&& f)   // tile width of the tensor-core GEMMs, hidden width of narrow layers
+{
+    switch (w) {
+    case 32: return f(Int<32>{});
+    case 64: return f(Int<64>{});
+    default: return f(Int<128>{});
+    }
+}
+
+// (layer, surrogate): mode 0 LIF, 1 ALIF, 2 Izhikevich (only the SIMT kernels have an Izhikevich body: the other
+// families are passed mode 0 / 1 and read ALIF as mode == 1).
+template <class F> int by_cell(int mode, int surrogate, F&& f)
+{
+    switch (mode * 2 + (surrogate ? 1 : 0)) {
+    case 0: return f(Int<0>{}, Int<0>{});
+    case 1: return f(Int<0>{}, Int<1>{});
+    case 2: return f(Int<1>{}, Int<0>{});
+    case 3: return f(Int<1>{}, Int<1>{});
+    case 4: return f(Int<2>{}, Int<0>{});
+    default: return f(Int<2>{}, Int<1>{});
+    }
+}
+
+template <class F> int by_rows_rec(int R, bool rec, F&& f)   // rows per CTA and recurrence of the SIMT kernels
+{
+    if (R == 1) return rec ? f(Int<1>{}, Bool<true>{}) : f(Int<1>{}, Bool<false>{});
+    return rec ? f(Int<2>{}, Bool<true>{}) : f(Int<2>{}, Bool<false>{});
+}
+
+template <class F> int by_nsm(int nsm, F&& f)   // SMs per n-slice of the wide weight-stationary kernels
+{
+    switch (nsm) {
+    case 4: return f(Int<4>{});
+    case 2: return f(Int<2>{});
+    default: return f(Int<1>{});
+    }
 }
 
 int device_ok()
@@ -113,12 +174,22 @@ int sm_count()
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-constexpr bool kPdlDefault = true;    // programmatic dependent launch of the lean forward recurrence behind the projection
 constexpr int kBitsMT = 2;   // row / feature tiles per CTA of the bit-fed GEMMs (both accumulators fit TMEM)
+
+// The kernel family of the recurrence (forward sweep and BPTT sweep), chosen from the descriptor by make_plan.
+enum class Family {
+    Simt,     // register-resident SIMT kernels (recur_fwd.cuh / recur_bwd.cuh; lean variants in recur_lean.cuh)
+    TcRec,    // tensor-core recurrence (recur_tc.cuh)
+    NonRec,   // non-recurrent layer on the lean scan kernels (recur_nr.cuh)
+    WideTc,   // H > 128 on the weight-stationary tensor-core kernels (recur_wide.cuh)
+    WideGen,  // H > 128 on the fp32 kernels (recur_gen.cuh)
+};
 
 // How the batch is cut into CTAs and how the weight-gradient GEMM is split; shared by the workspace
 // query and the launches so they can never disagree.
 struct Plan {
+    Family family;
+    bool lean_fwd;    // Simt: the lean forward kernel (recur_lean.cuh)
     int R;            // batch rows per recurrence CTA
     int grid_rows;    // recurrence CTAs
     int m_total;      // rows of the stacked weight gradient [dW_in ; dW_rec]
@@ -129,11 +200,8 @@ struct Plan {
     bool check;       // tensor-core path must verify on the device that x is tf32-exact (caller did not vouch)
     bool bits;        // x is the bit-packed raster (SNNK_F_INPUT_BITS): k_proj_bits / k_wgrad_bits
     int kpad;         // K of the projection padded to the k-block
-    bool wide;        // H > 128: generic recurrence kernels (recur_gen.cuh), N-tiled tensor-core GEMMs
-    bool tcrec;       // tensor-core recurrence kernels (recur_tc.cuh): gy scan + k_wout_grad beside the sweep
-    bool nr;          // non-recurrent layer on the lean scan kernels (recur_nr.cuh)
-    bool widetc;      // wide layer on the weight-stationary tensor-core kernels (recur_wide.cuh)
-    int w_nmt, w_nnt; // their grid: m-tiles of the batch x n-slices of the hidden axis
+    bool wide;        // H > 128: N-tiled tensor-core GEMMs
+    int w_nmt, w_nnt; // WideTc grid: m-tiles of the batch x n-slices of the hidden axis
     int w_nmt_b, w_npass_b;   // backward: m-tiles (its row tile differs) and passes over the batch
     size_t off_zx, off_wflags, off_gx, off_gmask, off_wflags_b;
     int tileN;        // N extent of one tensor-core tile
@@ -144,10 +212,15 @@ struct Plan {
     size_t off_weffT, off_gyscan;
     // frame-dedup variant (runs.cuh); eligible = tensor-core GEMMs on a non-wide layer
     bool runs;            // workspace for the compact kernels is reserved
+    bool dedup;           // and the call takes a run table (x is vouched {0,1}: no tf32 check)
     int run_rows;         // rows of the compact buffers: run_cap(B*T) rounded up to whole 128-row tiles
     int S_rec, sps_rec;   // split of the dW_rec-only GEMM of the variant
     int S_cmp;            // split of the dW_in GEMM over compact rows (few 32-row blocks: a handful of splits)
     size_t off_xu_f, off_iu, off_xu_b, off_gu, gu_plane, off_pwrec;
+
+    // The SIMT sweeps evaluate the readout and its adjoint themselves (fused head, dW_out / db partials per CTA); the
+    // other families run the stand-alone head, the readout-adjoint scan (k_gy_scan) and k_wout_grad beside them.
+    bool readout_in_sweep() const { return family == Family::Simt; }
 };
 
 int check_desc(const SnnkDesc* d)
@@ -172,34 +245,56 @@ IzhConsts izh_consts(const SnnkDesc* d)
     return z;
 }
 
-bool use_tc_recur(const SnnkDesc* d);
-bool use_wide_tc(const SnnkDesc* d);
-bool use_nonrec(const SnnkDesc* d);
+// The recurrence family of a checked descriptor (H is 32, 64, 128 or a multiple of 128 up to 2048).  In tensor-core
+// mode, LIF / ALIF layers take:
+// - H > 128, recurrent: the weight-stationary kernels when their shared memory fits and their grid fits the chip;
+// - H <= 128, not recurrent: the lean scan kernels;
+// - H = 128, recurrent, O <= 15 (row 15 of the readout MMA packs the spike bits): the tensor-core recurrence from
+//   B >= 1024 on.  Measured on B200 (profiles/r02_*): a step of an 8-row tile takes ~1400 (forward) / ~3000
+//   (backward) cycles on one SM whatever the batch -- bound by the dependent-issue latency of its ~200 / ~580
+//   instructions per warp, not by the 36 / 54 MMAs -- so these kernels win once the tiles fill the chip (B = 4096: K3
+//   0.58 ms vs 0.73 ms) and lose to the one-row-per-CTA SIMT kernels, which spread a small batch over all SMs (B = 256:
+//   82 / 168 us vs 55 / 72 us).  SNNK_MMA_RECUR = 0 / 1 forces the choice.
+// Everything else runs the fp32 wide kernels (H > 128) or the SIMT kernels.
+Family pick_family(const SnnkDesc* d, Plan& p)
+{
+    const bool tc_cell = d->layer_type != SNNK_IZHIKEVICH && (d->flags & SNNK_F_TENSOR_CORE) != 0;
+    if (d->H > 128) {
+        if (!tc_cell || !d->recurrent) return Family::WideGen;
+        if (wide_fwd_smem_bytes(d->H) > 225 * 1024 || wide_bwd_smem_bytes(d->H) > 225 * 1024) return Family::WideGen;
+        const int nsm = wide_nsm(d->H), mt = wide_mt(nsm), mtb = wide_bwd_mt(nsm);
+        p.w_nnt = d->H / (16 * nsm);
+        p.w_nmt = std::min(sm_count() / p.w_nnt, (d->B + mt - 1) / mt);
+        p.w_nmt_b = std::min(sm_count() / p.w_nnt, (d->B + mtb - 1) / mtb);
+        if (p.w_nmt < 1 || p.w_nmt_b < 1) return Family::WideGen;
+        p.w_npass_b = (d->B + p.w_nmt_b * mtb - 1) / (p.w_nmt_b * mtb);
+        return Family::WideTc;
+    }
+    if (!tc_cell) return Family::Simt;
+    if (!d->recurrent) return Family::NonRec;
+    if (d->H == kTcH && d->O <= 15 && env_switch("SNNK_MMA_RECUR", d->B >= 1024) &&
+        bwd_tc_smem_bytes(d->T) <= 200 * 1024 && fwd_tc_smem_bytes(d->T) <= 200 * 1024)
+        return Family::TcRec;
+    return Family::Simt;
+}
 
 Plan make_plan(const SnnkDesc* d)
 {
     Plan p{};
     p.wide = d->H > 128;
-    p.widetc = use_wide_tc(d);
-    if (p.widetc) {
-        const int nsm = wide_nsm(d->H), mt = wide_mt(nsm);
-        p.w_nnt = d->H / (16 * nsm);
-        p.w_nmt = std::min(sm_count() / p.w_nnt, (d->B + mt - 1) / mt);
-        if (p.w_nmt < 1) p.widetc = false;
-        const int mtb = wide_bwd_mt(nsm);
-        p.w_nmt_b = std::min(sm_count() / p.w_nnt, (d->B + mtb - 1) / mtb);
-        if (p.w_nmt_b < 1) p.widetc = false;
-        else p.w_npass_b = (d->B + p.w_nmt_b * mtb - 1) / (p.w_nmt_b * mtb);
-    }
-    p.nr = use_nonrec(d);
-    p.tcrec = use_tc_recur(d) && bwd_tc_smem_bytes(d->T) <= 200 * 1024 && fwd_tc_smem_bytes(d->T) <= 200 * 1024;
+    p.family = pick_family(d, p);
     p.R = p.wide ? gen_rows(d->H) : (d->B > 1024 ? 2 : 1);
+    // lean forward (recur_lean.cuh): recurrent LIF / ALIF, H = 128, one row per CTA, the row's input current resident
+    // in shared memory; SNNK_LEAN=0 keeps the general kernel
+    p.lean_fwd = p.family == Family::Simt && d->recurrent && d->layer_type != SNNK_IZHIKEVICH && d->H == 128 &&
+                 p.R == 1 && d->O <= kLeanOP && lean_fwd_smem_bytes<128>(d->T, d->O) <= 110 * 1024 &&
+                 env_switch("SNNK_LEAN", true);
     p.grid_rows = (d->B + p.R - 1) / p.R;
     const int BT = d->B * d->T;
     p.tileN = p.wide ? 128 : d->H;
     p.ntiles_tc = d->H / p.tileN;
-    p.n_pwout = (p.wide || p.tcrec || p.nr) ? (BT < 256 ? BT : 256) : p.grid_rows;
-    p.n_pdb = (p.wide || p.tcrec || p.nr) ? p.n_pwout : p.grid_rows * p.R;
+    p.n_pwout = p.readout_in_sweep() ? p.grid_rows : (BT < 256 ? BT : 256);
+    p.n_pdb = p.readout_in_sweep() ? p.grid_rows * p.R : p.n_pwout;
     p.BN = d->H >= 64 ? 64 : 32;
     p.ntiles = d->H / p.BN;
     p.mtiles_x = (d->N + kGemmBM - 1) / kGemmBM;
@@ -231,14 +326,15 @@ Plan make_plan(const SnnkDesc* d)
     p.off_pw = off;     off = align_up(off + sizeof(float) * (size_t)p.S * p.m_total * d->H, 256);
     p.off_flag = off;   off = align_up(off + 256, 256);
     p.off_weffT = off;  off = align_up(off + sizeof(float) * (size_t)d->H * d->H, 256);
-    p.off_gyscan = off; off = align_up(off + ((p.wide || p.tcrec || p.nr) ? sizeof(float) * (size_t)BT * kOMax : 0), 256);
-    if (p.widetc) {
+    p.off_gyscan = off; off = align_up(off + (p.readout_in_sweep() ? 0 : sizeof(float) * (size_t)BT * kOMax), 256);
+    if (p.family == Family::WideTc) {
         const int nsm = wide_nsm(d->H);
         p.off_gx = off;       off = align_up(off + sizeof(float) * 2 * (size_t)p.w_nmt_b * (d->H / wide_bwd_kc(nsm)) * wide_bwd_chunk_floats(nsm), 256);
         p.off_gmask = off;    off = align_up(off + sizeof(unsigned int) * (size_t)p.w_nmt_b * p.w_npass_b * d->T, 256);
         p.off_wflags_b = off; off = align_up(off + sizeof(unsigned int) * (size_t)p.w_nmt_b * kWideFlagStride, 256);
     }
     p.runs = p.tc && !p.wide && !p.bits;
+    p.dedup = p.runs && !p.check;
     if (p.runs) {
         const int cap = run_cap(BT);
         p.run_rows = (cap + 127) / 128 * 128;
@@ -255,7 +351,7 @@ Plan make_plan(const SnnkDesc* d)
     p.off_wplanes = off; off = align_up(off + (p.tc ? sizeof(float) * 3 * (size_t)d->H * p.kpad : 0), 256);
     p.off_fflag = off;   off = align_up(off + 256, 256);
     p.off_weff = off;    off = align_up(off + sizeof(float) * (size_t)d->H * d->H, 256);
-    if (p.widetc) {
+    if (p.family == Family::WideTc) {
         const int mt = wide_mt(wide_nsm(d->H));
         p.off_zx = off;     off = align_up(off + sizeof(uint32_t) * 2 * (size_t)p.w_nmt * (d->H / 32) * mt, 256);
         p.off_wflags = off; off = align_up(off + sizeof(unsigned int) * (size_t)p.w_nmt * kWideFlagStride, 256);
@@ -304,21 +400,15 @@ int make_map(CUtensorMap* m, const void* base, int rank, const cuuint64_t* dims,
 }
 
 template <int H>   // H = N extent of one CTA tile (the whole hidden width when it is <= 128)
-int launch_proj_tc(const SnnkDesc* d, const Plan& pl, const float* x, const float* W_in, float* I_in, float* planes,
-                   unsigned int* flag, cudaStream_t st, const int* run_table = nullptr, int run_variant = 0,
-                   bool split = true)
+int launch_proj_tc(const SnnkDesc* d, const Plan& pl, const float* x, float* I_in, const float* planes,
+                   unsigned int* flag, cudaStream_t st, const int* run_table, int run_variant)
 {
-    // run_variant 1: x / I_in are the compact buffers of the frame-dedup path (run_rows rows, the weight planes are
-    // already split); 0 with a table: the dense launch, which the kernel skips when the table says ok
+    // planes: W_in^T as split by k_split_w.  run_variant 1: x / I_in are the compact buffers of the frame-dedup path
+    // (run_rows rows); 0 with a table: the dense launch, which the kernel skips when the table says ok
     constexpr int P = 2;   // planes of W_in^T fed to the tensor pipe (k_split_w writes three)
     using Cfg = tc::ProjCfg<H, P>;
     const int M = run_variant == 1 ? pl.run_rows : d->B * d->T;
     const int Hf = d->H;
-    if (run_variant == 0 && split) {
-        const int n = Hf * pl.kpad;
-        tc::k_split_w<<<(n + 255) / 256, 256, 0, st>>>(W_in, d->N, Hf, pl.kpad, planes);
-        SNNK_CUDA(cudaGetLastError());
-    }
     CUtensorMap mx;
     {
         const cuuint64_t dims[2] = {(cuuint64_t)d->N, (cuuint64_t)M};
@@ -327,14 +417,9 @@ int launch_proj_tc(const SnnkDesc* d, const Plan& pl, const float* x, const floa
         int rc = make_map(&mx, x, 2, dims, str, box);
         if (rc != SNNK_OK) return rc;
     }
-    auto kern = tc::k_proj_tc<H, P>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
-    ProfScope ps(SNNK_K_PROJ, st);
-    dim3 grid((M + tc::kBlockM - 1) / tc::kBlockM, Hf / H);
-    kern<<<grid, tc::kThreads, Cfg::kSmemBytes, st>>>(mx, planes, I_in, M, pl.kpad / tc::kBlockK, Hf, flag, run_table, run_variant,
-                                                    run_variant == 1 ? x : nullptr);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    const float* xc = run_variant == 1 ? x : nullptr;
+    return launch(SNNK_K_PROJ, tc::k_proj_tc<H, P>, dim3((M + tc::kBlockM - 1) / tc::kBlockM, Hf / H), tc::kThreads,
+                  Cfg::kSmemBytes, st, mx, planes, I_in, M, pl.kpad / tc::kBlockK, Hf, flag, run_table, run_variant, xc);
 }
 
 // Geometry of one weight-gradient launch.  The dense launch contracts [x ; Z_{t-1}]^T gI over (B, T); the frame-dedup
@@ -379,13 +464,8 @@ int launch_wgrad_tc(const SnnkDesc* d, const WgradGeom& g, cudaStream_t st)
     wp.N = g.N; wp.T = g.T; wp.B = g.B; wp.mtiles_x = g.mtiles_x; wp.m_total = g.m_total; wp.H_full = d->H;
     wp.samples_per_split = g.samples_per_split; wp.part = g.part; wp.inexact_flag = g.flag;
     wp.run_table = g.run_table; wp.run_gate = g.run_gate; wp.run_clip = g.run_clip;
-    auto kern = tc::k_wgrad_tc<H, P>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
-    dim3 grid(g.mtiles_x + g.mtiles_z, g.S, d->H / H);
-    ProfScope ps(SNNK_K_WGRAD, st);
-    kern<<<grid, tc::kThreads, Cfg::kSmemBytes, st>>>(mx, mz, mg, wp);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_WGRAD, tc::k_wgrad_tc<H, P>, dim3(g.mtiles_x + g.mtiles_z, g.S, d->H / H), tc::kThreads,
+                  Cfg::kSmemBytes, st, mx, mz, mg, wp);
 }
 
 // ---- bit-packed input (SNNK_F_INPUT_BITS, gemm_bits.cuh) --------------------------------------------------------------
@@ -400,13 +480,9 @@ int launch_proj_bits(const SnnkDesc* d, const uint32_t* xbits, const float* W_in
     float* inv_scale = reinterpret_cast<float*>(planes + 2 * (size_t)kblocks * Hf * tc::kBitsBlockK);
     tc::k_split_w_h<<<Hf, 256, 0, st>>>(W_in, d->N, Hf, kblocks, planes, inv_scale);
     SNNK_CUDA(cudaGetLastError());
-    auto kern = tc::k_proj_bits<H, kBitsMT>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
-    ProfScope ps(SNNK_K_PROJ, st);
-    dim3 grid((M + kBitsMT * tc::kBlockM - 1) / (kBitsMT * tc::kBlockM), Hf / H);
-    kern<<<grid, tc::bits_threads<kBitsMT>(), Cfg::kSmemBytes, st>>>(xbits, wd, planes, inv_scale, I_in, M, kblocks, Hf);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_PROJ, tc::k_proj_bits<H, kBitsMT>,
+                  dim3((M + kBitsMT * tc::kBlockM - 1) / (kBitsMT * tc::kBlockM), Hf / H), tc::bits_threads<kBitsMT>(),
+                  Cfg::kSmemBytes, st, xbits, wd, planes, inv_scale, I_in, M, kblocks, Hf);
 }
 
 template <int H>
@@ -428,49 +504,36 @@ int launch_wgrad_bits(const SnnkDesc* d, const Plan& pl, const uint32_t* xbits, 
     wp.N = d->N; wp.T = d->T; wp.B = d->B; wp.mtiles_x = pl.mtiles_x; wp.mtiles_z = pl.mtiles_z; wp.m_total = pl.m_total;
     wp.H_full = d->H; wp.samples_per_split = pl.samples_per_split;
     wp.xbits = xbits; wp.wd_x = (d->N + 31) / 32; wp.zbits = zbits; wp.wd_z = d->H / 32; wp.part = part;
-    auto kern = tc::k_wgrad_bits<H, kBitsMT>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes));
-    dim3 grid((pl.mtiles_x + pl.mtiles_z + kBitsMT - 1) / kBitsMT, pl.S, d->H / H);
-    ProfScope ps(SNNK_K_WGRAD, st);
-    kern<<<grid, tc::bits_threads<kBitsMT>(), Cfg::kSmemBytes, st>>>(mg, wp);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_WGRAD, tc::k_wgrad_bits<H, kBitsMT>,
+                  dim3((pl.mtiles_x + pl.mtiles_z + kBitsMT - 1) / kBitsMT, pl.S, d->H / H), tc::bits_threads<kBitsMT>(),
+                  Cfg::kSmemBytes, st, mg, wp);
 }
 
 int launch_wgrad_tc_any(const SnnkDesc* d, int tileN, const WgradGeom& g, cudaStream_t st)
 {
-    switch (tileN) {
-    case 32: return launch_wgrad_tc<32>(d, g, st);
-    case 64: return launch_wgrad_tc<64>(d, g, st);
-    default: return launch_wgrad_tc<128>(d, g, st);
-    }
+    return by_width(tileN, [&](auto tn) { return launch_wgrad_tc<decltype(tn)::value>(d, g, st); });
 }
 
-template <int H, int R, bool REC>
-int launch_fwd(const FwdParams& fp, int grid, cudaStream_t st)
+// SIMT forward recurrence (recur_fwd.cuh)
+int launch_fwd_simt(const FwdParams& fp, bool rec, const Plan& pl, cudaStream_t st)
 {
-    const size_t smem = fwd_smem_bytes<H, R>(fp.T, fp.O);
-    if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-    // the Izhikevich body is a compile-time variant: a run-time branch in the step loop cost the LIF/ALIF kernels 6 %
-    auto kern = fp.iz.on ? k_recur_fwd<H, R, REC, 2> : (fp.alif ? k_recur_fwd<H, R, REC, 1> : k_recur_fwd<H, R, REC, 0>);
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    { ProfScope ps(SNNK_K_RECUR_FWD, st); kern<<<grid, H, smem, st>>>(fp); }
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return by_width(fp.H, [&](auto h) {
+        return by_rows_rec(pl.R, rec, [&](auto r, auto re) {
+            constexpr int H = decltype(h)::value, R = decltype(r)::value;
+            constexpr bool REC = decltype(re)::value;
+            const size_t smem = fwd_smem_bytes<H, R>(fp.T, fp.O);
+            if (smem > 200 * 1024) return (int)SNNK_ERR_SHAPE;
+            // the Izhikevich body is a compile-time variant: a run-time branch in the step loop cost the LIF/ALIF
+            // kernels 6 %
+            auto kern = fp.iz.on ? k_recur_fwd<H, R, REC, 2> : (fp.alif ? k_recur_fwd<H, R, REC, 1> : k_recur_fwd<H, R, REC, 0>);
+            return launch(SNNK_K_RECUR_FWD, kern, pl.grid_rows, H, smem, st, fp);
+        });
+    });
 }
 
-// Lean forward recurrence (recur_lean.cuh): recurrent LIF / ALIF, H = 128, one row per CTA, the row's input current
-// resident in shared memory.  SNNK_LEAN=0 keeps the general kernel (measuring switch, read per call).
-bool use_lean_fwd(const FwdParams& fp, bool rec, int R)
-{
-    if (!rec || fp.iz.on || fp.H != 128 || R != 1 || fp.O > kLeanOP) return false;
-    if (lean_fwd_smem_bytes<128>(fp.T, fp.O) > 110 * 1024) return false;
-    const char* env = getenv("SNNK_LEAN");
-    return !(env && env[0] == '0');
-}
-
-// pdl: launch as a programmatic dependent of the kernel queued before it on the stream (the projection GEMM, which
-// executes griddepcontrol.launch_dependents at its start): the recurrence kernel's prologue then overlaps the projection.
+// Lean forward recurrence (recur_lean.cuh; Plan::lean_fwd).  pdl: launch as a programmatic dependent of the kernel
+// queued before it on the stream (the projection GEMM, which executes griddepcontrol.launch_dependents at its start):
+// the recurrence kernel's prologue then overlaps the projection.
 int launch_fwd_lean(FwdParams fp, cudaStream_t st, bool pdl)
 {
     const size_t smem = lean_fwd_smem_bytes<128>(fp.T, fp.O);
@@ -496,36 +559,48 @@ int launch_fwd_lean(FwdParams fp, cudaStream_t st, bool pdl)
     return SNNK_OK;
 }
 
-template <int H, int R>
-int launch_fwd_rec(const FwdParams& fp, bool rec, int grid, cudaStream_t st)
+// Lean BPTT sweep (recur_lean.cuh): the training step of the headline geometry -- recurrent LIF / ALIF, H = 128, one row
+// per CTA, sparse seeds from the fused head, no seeds on V / Z.  A refinement of the SIMT family that also depends on
+// the seeds of the call; SNNK_LEAN=0 keeps the general kernel.
+bool use_lean_bwd(const BwdParams& bp, bool rec, int R)
 {
-    return rec ? launch_fwd<H, R, true>(fp, grid, st) : launch_fwd<H, R, false>(fp, grid, st);
+    if (!rec || bp.iz.on || bp.H != 128 || R != 1 || bp.g_y || bp.g_V || bp.g_Z || !bp.g_logits || !bp.tstar) return false;
+    if (bwd_smem_bytes<128, 1>(bp.T, true) > 110 * 1024 || bp.T > 128) return false;   // T * 4 spike words <= 4 per thread
+    return env_switch("SNNK_LEAN", true);
 }
 
-// Tensor-core recurrence (recur_tc.cuh): H = 128 recurrent LIF / ALIF layers in tensor-core mode.
-// Measured on B200 (profiles/r02_*): a step of an 8-row tile takes ~1400 (forward) / ~3000 (backward) cycles on one
-// SM whatever the batch -- bound by the dependent-issue latency of its ~200 / ~580 instructions per warp, not by the
-// 36 / 54 MMAs -- so these kernels win once the tiles fill the chip (B = 4096: K3 0.58 ms vs 0.73 ms) and lose to
-// the one-row-per-CTA SIMT kernels, which spread a small batch over all SMs (B = 256: 82 / 168 us vs 55 / 72 us).
-// SNNK_MMA_RECUR = 0 / 1 forces the choice (measuring switch; read per call, tools/sanitize_run.py toggles it).
-bool use_tc_recur(const SnnkDesc* d)
+int launch_bwd_lean(const BwdParams& bp, cudaStream_t st)
 {
-    if (d->layer_type == SNNK_IZHIKEVICH || !d->recurrent || d->H != kTcH || d->O > 15) return false;   // row 15 of the readout MMA packs the spike bits
-    if ((d->flags & SNNK_F_TENSOR_CORE) == 0) return false;
-    const char* env = getenv("SNNK_MMA_RECUR");
-    if (env) return env[0] != '0';
-    return d->B >= 1024;
+    const size_t smem = bwd_smem_bytes<128, 1>(bp.T, true);
+    const bool planes = bp.gI_lo != nullptr, runs = bp.run_table != nullptr;
+    return by_cell(bp.alif ? 1 : 0, bp.surrogate, [&](auto m, auto s) -> int {
+        constexpr bool A = decltype(m)::value == 1;
+        constexpr int S = decltype(s)::value;
+        auto pick = [&](auto op) {
+            constexpr int OP = decltype(op)::value;
+            return planes ? (runs ? k_recur_bwd_lean<A, S, true, true, OP> : k_recur_bwd_lean<A, S, true, false, OP>)
+                          : (runs ? k_recur_bwd_lean<A, S, false, true, OP> : k_recur_bwd_lean<A, S, false, false, OP>);
+        };
+        return launch(SNNK_K_RECUR_BWD, bp.O <= 12 ? pick(Int<12>{}) : pick(Int<16>{}), bp.B, 128, smem, st, bp);
+    });
 }
 
-// Wide layers (H > 128) in tensor-core mode: weight-stationary, grid-synchronous kernels (recur_wide.cuh).
-// SNNK_WIDE_TC=0 keeps the fp32 kernels of recur_gen.cuh (measuring switch).
-bool use_wide_tc(const SnnkDesc* d)
+// SIMT BPTT sweep (recur_bwd.cuh)
+int launch_bwd_simt(const BwdParams& bp, bool rec, const Plan& pl, cudaStream_t st)
 {
-    if (d->H <= 128 || d->H % 128 != 0 || d->H > 2048) return false;
-    if (d->layer_type == SNNK_IZHIKEVICH || !d->recurrent || (d->flags & SNNK_F_TENSOR_CORE) == 0) return false;
-    const char* env = getenv("SNNK_WIDE_TC");
-    if (env && env[0] == '0') return false;
-    return wide_fwd_smem_bytes(d->H) <= 225 * 1024 && wide_bwd_smem_bytes(d->H) <= 225 * 1024;
+    const int mode = bp.iz.on ? 2 : (bp.alif ? 1 : 0);
+    return by_width(bp.H, [&](auto h) -> int {
+        return by_rows_rec(pl.R, rec, [&](auto r, auto re) -> int {
+            constexpr int H = decltype(h)::value, R = decltype(r)::value;
+            constexpr bool REC = decltype(re)::value;
+            const size_t smem = bwd_smem_bytes<H, R>(bp.T, REC);
+            if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
+            return by_cell(mode, bp.surrogate, [&](auto m, auto s) -> int {
+                return launch(SNNK_K_RECUR_BWD, k_recur_bwd<H, R, REC, decltype(m)::value, decltype(s)::value>,
+                              pl.grid_rows, H, smem, st, bp);
+            });
+        });
+    });
 }
 
 WideParams wide_params(const FwdParams& fp, const Plan& pl, char* ws)
@@ -541,118 +616,64 @@ WideParams wide_params(const FwdParams& fp, const Plan& pl, char* ws)
     return wp;
 }
 
-template <int NSM>
-int launch_wide_fwd_t(const WideParams& wp, cudaStream_t st)
-{
-    const size_t smem = wide_fwd_smem_bytes(wp.H);
-    void* kern = wp.alif ? (void*)k_wide_fwd<NSM, true> : (void*)k_wide_fwd<NSM, false>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    SNNK_CUDA(cudaMemsetAsync(wp.flags, 0, sizeof(unsigned int) * (size_t)wp.n_mt * kWideFlagStride, st));
-    WideParams arg = wp;
-    void* args[] = {&arg};
-    ProfScope ps(SNNK_K_RECUR_FWD, st);
-    // cooperative: every CTA waits for its m-tile's peers each step, so all of them must be resident
-    SNNK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(wp.n_mt * wp.n_nt), dim3(kWideThreads), args, smem, st));
-    return SNNK_OK;
-}
-
+// Wide layers (H > 128) in tensor-core mode: weight-stationary, grid-synchronous kernels (recur_wide.cuh).  Cooperative
+// launches: every CTA waits for its m-tile's peers each step, so all of them must be resident.
 int launch_wide_fwd(const WideParams& wp, cudaStream_t st)
 {
-    switch (wide_nsm(wp.H)) {
-    case 4: return launch_wide_fwd_t<4>(wp, st);
-    case 2: return launch_wide_fwd_t<2>(wp, st);
-    default: return launch_wide_fwd_t<1>(wp, st);
-    }
-}
-
-template <int NSM>
-int launch_wide_bwd_t(const WideBwdParams& wp, int n_pass, cudaStream_t st)
-{
-    const size_t smem = wide_bwd_smem_bytes(wp.H);
-    void* kern = nullptr;
-    switch ((wp.alif ? 2 : 0) + (wp.surrogate ? 1 : 0)) {
-    case 0: kern = (void*)k_wide_bwd<NSM, false, 0>; break;
-    case 1: kern = (void*)k_wide_bwd<NSM, false, 1>; break;
-    case 2: kern = (void*)k_wide_bwd<NSM, true, 0>; break;
-    default: kern = (void*)k_wide_bwd<NSM, true, 1>; break;
-    }
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    SNNK_CUDA(cudaMemsetAsync(wp.flags, 0, sizeof(unsigned int) * (size_t)wp.n_mt * kWideFlagStride, st));
-    SNNK_CUDA(cudaMemsetAsync(wp.gmask, 0, sizeof(unsigned int) * (size_t)wp.n_mt * n_pass * wp.T, st));
-    WideBwdParams arg = wp;
-    void* args[] = {&arg};
-    ProfScope ps(SNNK_K_RECUR_BWD, st);
-    SNNK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(wp.n_mt * wp.n_nt), dim3(kWideThreads), args, smem, st));
-    return SNNK_OK;
+    return by_nsm(wide_nsm(wp.H), [&](auto nsm) -> int {
+        constexpr int NSM = decltype(nsm)::value;
+        const size_t smem = wide_fwd_smem_bytes(wp.H);
+        void* kern = wp.alif ? (void*)k_wide_fwd<NSM, true> : (void*)k_wide_fwd<NSM, false>;
+        SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        SNNK_CUDA(cudaMemsetAsync(wp.flags, 0, sizeof(unsigned int) * (size_t)wp.n_mt * kWideFlagStride, st));
+        WideParams arg = wp;
+        void* args[] = {&arg};
+        ProfScope ps(SNNK_K_RECUR_FWD, st);
+        SNNK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(wp.n_mt * wp.n_nt), dim3(kWideThreads), args, smem, st));
+        return SNNK_OK;
+    });
 }
 
 int launch_wide_bwd(const WideBwdParams& wp, int n_pass, cudaStream_t st)
 {
-    switch (wide_nsm(wp.H)) {
-    case 4: return launch_wide_bwd_t<4>(wp, n_pass, st);
-    case 2: return launch_wide_bwd_t<2>(wp, n_pass, st);
-    default: return launch_wide_bwd_t<1>(wp, n_pass, st);
-    }
+    return by_nsm(wide_nsm(wp.H), [&](auto nsm) -> int {
+        return by_cell(wp.alif ? 1 : 0, wp.surrogate, [&](auto m, auto s) -> int {
+            const size_t smem = wide_bwd_smem_bytes(wp.H);
+            void* kern = (void*)k_wide_bwd<decltype(nsm)::value, decltype(m)::value == 1, decltype(s)::value>;
+            SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            SNNK_CUDA(cudaMemsetAsync(wp.flags, 0, sizeof(unsigned int) * (size_t)wp.n_mt * kWideFlagStride, st));
+            SNNK_CUDA(cudaMemsetAsync(wp.gmask, 0, sizeof(unsigned int) * (size_t)wp.n_mt * n_pass * wp.T, st));
+            WideBwdParams arg = wp;
+            void* args[] = {&arg};
+            ProfScope ps(SNNK_K_RECUR_BWD, st);
+            SNNK_CUDA(cudaLaunchCooperativeKernel(kern, dim3(wp.n_mt * wp.n_nt), dim3(kWideThreads), args, smem, st));
+            return SNNK_OK;
+        });
+    });
 }
 
 // Non-recurrent LIF / ALIF layers of width 32 / 64 / 128 in tensor-core mode: lean scan kernels (recur_nr.cuh).
-// SNNK_NONREC=0 keeps the generic kernels (measuring switch).
-bool use_nonrec(const SnnkDesc* d)
-{
-    if (d->recurrent || d->layer_type == SNNK_IZHIKEVICH || (d->flags & SNNK_F_TENSOR_CORE) == 0) return false;
-    if (d->H != 32 && d->H != 64 && d->H != 128) return false;
-    const char* env = getenv("SNNK_NONREC");
-    return !(env && env[0] == '0');
-}
-
-template <int H>
-int launch_nonrec_fwd_t(const FwdParams& fp, cudaStream_t st)
-{
-    const size_t smem = nonrec_fwd_smem_bytes<H>(fp.T, fp.O);
-    if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-    auto kern = fp.alif ? k_nonrec_fwd<H, true> : k_nonrec_fwd<H, false>;
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ProfScope ps(SNNK_K_RECUR_FWD, st);
-    kern<<<fp.B, H, smem, st>>>(fp);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
-}
-
 int launch_nonrec_fwd(const FwdParams& fp, cudaStream_t st)
 {
-    switch (fp.H) {
-    case 32: return launch_nonrec_fwd_t<32>(fp, st);
-    case 64: return launch_nonrec_fwd_t<64>(fp, st);
-    default: return launch_nonrec_fwd_t<128>(fp, st);
-    }
-}
-
-template <int H>
-int launch_nonrec_bwd_t(const BwdParams& bp, const float* gy_scan, cudaStream_t st)
-{
-    const size_t smem = nonrec_bwd_smem_bytes<H>(bp.T);
-    if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-    void (*kern)(const BwdParams, const float*) = nullptr;
-    switch ((bp.alif ? 2 : 0) + (bp.surrogate ? 1 : 0)) {
-    case 0: kern = k_nonrec_bwd<H, false, 0>; break;
-    case 1: kern = k_nonrec_bwd<H, false, 1>; break;
-    case 2: kern = k_nonrec_bwd<H, true, 0>; break;
-    default: kern = k_nonrec_bwd<H, true, 1>; break;
-    }
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ProfScope ps(SNNK_K_RECUR_BWD, st);
-    kern<<<bp.B, H, smem, st>>>(bp, gy_scan);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return by_width(fp.H, [&](auto h) -> int {
+        constexpr int H = decltype(h)::value;
+        const size_t smem = nonrec_fwd_smem_bytes<H>(fp.T, fp.O);
+        if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
+        return launch(SNNK_K_RECUR_FWD, fp.alif ? k_nonrec_fwd<H, true> : k_nonrec_fwd<H, false>, fp.B, H, smem, st, fp);
+    });
 }
 
 int launch_nonrec_bwd(const BwdParams& bp, const float* gy_scan, cudaStream_t st)
 {
-    switch (bp.H) {
-    case 32: return launch_nonrec_bwd_t<32>(bp, gy_scan, st);
-    case 64: return launch_nonrec_bwd_t<64>(bp, gy_scan, st);
-    default: return launch_nonrec_bwd_t<128>(bp, gy_scan, st);
-    }
+    return by_width(bp.H, [&](auto h) -> int {
+        constexpr int H = decltype(h)::value;
+        const size_t smem = nonrec_bwd_smem_bytes<H>(bp.T);
+        if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
+        return by_cell(bp.alif ? 1 : 0, bp.surrogate, [&](auto m, auto s) -> int {
+            return launch(SNNK_K_RECUR_BWD, k_nonrec_bwd<H, decltype(m)::value == 1, decltype(s)::value>, bp.B, H, smem, st,
+                          bp, gy_scan);
+        });
+    });
 }
 
 // 4-D view {32, B, 4, T} of a (B, T, 128) fp32 trace (H = 4 groups of 32 neurons) with the box {32, rows, 4, steps} the
@@ -665,6 +686,7 @@ int make_trace_map(CUtensorMap* m, const float* base, int B, int T, int rows, in
     return make_map(m, base, 4, dims, str, box);
 }
 
+// Tensor-core recurrence (recur_tc.cuh): H = 128 recurrent LIF / ALIF layers in tensor-core mode.
 int launch_fwd_tc(const FwdParams& fp, cudaStream_t st)
 {
     const size_t smem = fwd_tc_smem_bytes(fp.T);
@@ -677,16 +699,8 @@ int launch_fwd_tc(const FwdParams& fp, cudaStream_t st)
         if (rc == SNNK_OK && fp.alif) rc = make_trace_map(&mA, fp.a, fp.B, fp.T, kTcRows, kTcK);
         if (rc != SNNK_OK) return rc;
     }
-    ProfScope ps(SNNK_K_RECUR_FWD, st);
-    if (fp.alif) {
-        SNNK_CUDA(cudaFuncSetAttribute(k_recur_fwd_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_recur_fwd_tc<true><<<grid, kTcFwdThreads, smem, st>>>(fp, mV, mA, mZ);
-    } else {
-        SNNK_CUDA(cudaFuncSetAttribute(k_recur_fwd_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k_recur_fwd_tc<false><<<grid, kTcFwdThreads, smem, st>>>(fp, mV, mV, mZ);
-    }
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_RECUR_FWD, fp.alif ? k_recur_fwd_tc<true> : k_recur_fwd_tc<false>, grid, kTcFwdThreads, smem, st,
+                  fp, mV, fp.alif ? mA : mV, mZ);
 }
 
 int launch_bwd_tc(const BwdParams& bp, const float* gy_scan, cudaStream_t st)
@@ -702,166 +716,58 @@ int launch_bwd_tc(const BwdParams& bp, const float* gy_scan, cudaStream_t st)
         if (rc == SNNK_OK && bp.gI_lo) rc = make_trace_map(&mGlo, bp.gI_lo, bp.B, bp.T, kTcRows, kTcKb);
         if (rc != SNNK_OK) return rc;
     }
-    void (*kern)(const BwdParams, const float*, const CUtensorMap, const CUtensorMap, const CUtensorMap, const CUtensorMap) = nullptr;
-    switch ((bp.alif ? 2 : 0) + (bp.surrogate ? 1 : 0)) {
-    case 0: kern = k_recur_bwd_tc<false, 0>; break;
-    case 1: kern = k_recur_bwd_tc<false, 1>; break;
-    case 2: kern = k_recur_bwd_tc<true, 0>; break;
-    default: kern = k_recur_bwd_tc<true, 1>; break;
-    }
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ProfScope ps(SNNK_K_RECUR_BWD, st);
-    kern<<<grid, kTcThreads, smem, st>>>(bp, gy_scan, mV, bp.alif ? mA : mV, mG, bp.gI_lo ? mGlo : mG);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return by_cell(bp.alif ? 1 : 0, bp.surrogate, [&](auto m, auto s) -> int {
+        return launch(SNNK_K_RECUR_BWD, k_recur_bwd_tc<decltype(m)::value == 1, decltype(s)::value>, grid, kTcThreads, smem,
+                      st, bp, gy_scan, mV, bp.alif ? mA : mV, mG, bp.gI_lo ? mGlo : mG);
+    });
 }
 
-template <int H>
-int launch_fwd_r(const FwdParams& fp, bool rec, int R, int grid, cudaStream_t st)
+// Readout-adjoint scan of the families whose sweep does not evaluate the readout (Plan::readout_in_sweep), and the
+// dW_out / db partials contracted from it and the spike raster
+int launch_gy_scan(const SnnkDesc* d, const BwdParams& bp, float* gy_scan, cudaStream_t st)
 {
-    return R == 1 ? launch_fwd_rec<H, 1>(fp, rec, grid, st) : launch_fwd_rec<H, 2>(fp, rec, grid, st);
+    return launch(SNNK_K_REDUCE_OUT, k_gy_scan, (d->B * kOMax + 255) / 256, 256, 0, st, d->B, d->T, d->O, d->kappa, bp.g_y,
+                  bp.g_logits, bp.tstar, bp.g_scale, gy_scan);
 }
 
-template <int H, int R, bool REC>
-int launch_bwd(const BwdParams& bp, int grid, cudaStream_t st)
+int launch_wout_grad(const SnnkDesc* d, const Plan& pl, const uint32_t* zbits, const float* gy_scan, float* pwout,
+                     float* pdb, cudaStream_t st)
 {
-    const size_t smem = bwd_smem_bytes<H, R>(bp.T, REC);
-    if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-    const int mode = bp.iz.on ? 2 : (bp.alif ? 1 : 0);
-    void (*kern)(const BwdParams) = nullptr;
-    switch (mode * 2 + (bp.surrogate ? 1 : 0)) {
-    case 0: kern = k_recur_bwd<H, R, REC, 0, 0>; break;
-    case 1: kern = k_recur_bwd<H, R, REC, 0, 1>; break;
-    case 2: kern = k_recur_bwd<H, R, REC, 1, 0>; break;
-    case 3: kern = k_recur_bwd<H, R, REC, 1, 1>; break;
-    case 4: kern = k_recur_bwd<H, R, REC, 2, 0>; break;
-    default: kern = k_recur_bwd<H, R, REC, 2, 1>; break;
-    }
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    { ProfScope ps(SNNK_K_RECUR_BWD, st); kern<<<grid, H, smem, st>>>(bp); }
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_REDUCE_OUT, k_wout_grad, dim3(pl.n_pwout, (d->H + 127) / 128), 128, 0, st, d->B * d->T, d->H,
+                  d->O, zbits, gy_scan, pwout, pdb);
 }
 
-// Lean BPTT sweep (recur_lean.cuh): the training step of the headline geometry -- recurrent LIF / ALIF, H = 128, one row
-// per CTA, sparse seeds from the fused head, no seeds on V / Z.  SNNK_LEAN=0 keeps the general kernel.
-bool use_lean_bwd(const BwdParams& bp, bool rec, int R)
-{
-    if (!rec || bp.iz.on || bp.H != 128 || R != 1 || bp.g_y || bp.g_V || bp.g_Z || !bp.g_logits || !bp.tstar) return false;
-    if (bwd_smem_bytes<128, 1>(bp.T, true) > 110 * 1024 || bp.T > 128) return false;   // T * 4 spike words <= 4 per thread
-    const char* env = getenv("SNNK_LEAN");
-    return !(env && env[0] == '0');
-}
-
-template <bool ALIF, int SURR, int OP>
-int launch_bwd_lean_o(const BwdParams& bp, cudaStream_t st)
-{
-    const size_t smem = bwd_smem_bytes<128, 1>(bp.T, true);
-    const bool planes = bp.gI_lo != nullptr, runs = bp.run_table != nullptr;
-    void (*kern)(const BwdParams) =
-        planes ? (runs ? k_recur_bwd_lean<ALIF, SURR, true, true, OP> : k_recur_bwd_lean<ALIF, SURR, true, false, OP>)
-               : (runs ? k_recur_bwd_lean<ALIF, SURR, false, true, OP> : k_recur_bwd_lean<ALIF, SURR, false, false, OP>);
-    SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    { ProfScope ps(SNNK_K_RECUR_BWD, st); kern<<<bp.B, 128, smem, st>>>(bp); }
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
-}
-
-template <bool ALIF, int SURR>
-int launch_bwd_lean_t(const BwdParams& bp, cudaStream_t st)
-{
-    return bp.O <= 12 ? launch_bwd_lean_o<ALIF, SURR, 12>(bp, st) : launch_bwd_lean_o<ALIF, SURR, 16>(bp, st);
-}
-
-int launch_bwd_lean(const BwdParams& bp, cudaStream_t st)
-{
-    if (bp.alif) return bp.surrogate ? launch_bwd_lean_t<true, 1>(bp, st) : launch_bwd_lean_t<true, 0>(bp, st);
-    return bp.surrogate ? launch_bwd_lean_t<false, 1>(bp, st) : launch_bwd_lean_t<false, 0>(bp, st);
-}
-
-template <int H, int R>
-int launch_bwd_rec(const BwdParams& bp, bool rec, int grid, cudaStream_t st)
-{
-    return rec ? launch_bwd<H, R, true>(bp, grid, st) : launch_bwd<H, R, false>(bp, grid, st);
-}
-
-template <int H>
-int launch_bwd_r(const BwdParams& bp, bool rec, int R, int grid, cudaStream_t st)
-{
-    return R == 1 ? launch_bwd_rec<H, 1>(bp, rec, grid, st) : launch_bwd_rec<H, 2>(bp, rec, grid, st);
-}
-
-// ---- wide hidden layers (H > 128): generic recurrence + separate readout / dW_out kernels -------------------------
+// ---- wide hidden layers (H > 128) on the fp32 kernels (recur_gen.cuh): generic recurrence, then the readout --------
 int launch_readout_scan(const SnnkDesc* d, const FwdParams& fp, cudaStream_t st)
 {
-    const size_t smem2 = sizeof(uint32_t) * (size_t)d->T * (d->H / 32) + sizeof(float) * ((size_t)d->H * d->O + (size_t)d->T * d->O);
-    if (smem2 > 200 * 1024) return SNNK_ERR_SHAPE;
-    SNNK_CUDA(cudaFuncSetAttribute(k_readout_scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-    ProfScope ps2(SNNK_K_HEAD, st);
-    k_readout_scan<<<d->B, 128, smem2, st>>>(d->T, d->H, d->O, d->kappa, fp.zbits, fp.W_out, fp.b_out, fp.y, fp.logits,
-                                             fp.tstar);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
-}
-
-template <int NPT, int R>
-int launch_fwd_wide_t(const SnnkDesc* d, const FwdParams& fp, bool rec, const Plan& pl, cudaStream_t st)
-{
-    const size_t smem = sizeof(float) * 2 * (size_t)d->H * R;
-    const int threads = d->H / NPT;
-    {
-        ProfScope ps(SNNK_K_RECUR_FWD, st);
-        if (rec) {
-            auto kern = k_recur_fwd_gen<NPT, R, true>;
-            SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<pl.grid_rows, threads, smem, st>>>(fp);
-        } else {
-            auto kern = k_recur_fwd_gen<NPT, R, false>;
-            SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<pl.grid_rows, threads, smem, st>>>(fp);
-        }
-    }
-    SNNK_CUDA(cudaGetLastError());
-    return launch_readout_scan(d, fp, st);
-}
-
-int launch_fwd_wide(const SnnkDesc* d, const FwdParams& fp, bool rec, const Plan& pl, cudaStream_t st)
-{
-    return gen_npt(d->H) == 1 ? launch_fwd_wide_t<1, 4>(d, fp, rec, pl, st) : launch_fwd_wide_t<2, 2>(d, fp, rec, pl, st);
-}
-
-template <int NPT, int R>
-int launch_bwd_wide_t(const SnnkDesc* d, const BwdParams& bp, bool rec, const Plan& pl, float* gy_scan,
-                      const uint32_t* zbits, cudaStream_t st)
-{
-    const size_t smem = sizeof(float) * (2 * (size_t)d->H * R + (size_t)R * d->T * kOMax);
+    const size_t smem = sizeof(uint32_t) * (size_t)d->T * (d->H / 32) + sizeof(float) * ((size_t)d->H * d->O + (size_t)d->T * d->O);
     if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-    const int threads = d->H / NPT;
-    {
-        ProfScope ps(SNNK_K_RECUR_BWD, st);
-        if (rec) {
-            auto kern = k_recur_bwd_gen<NPT, R, true>;
-            SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<pl.grid_rows, threads, smem, st>>>(bp, gy_scan);
-        } else {
-            auto kern = k_recur_bwd_gen<NPT, R, false>;
-            SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            kern<<<pl.grid_rows, threads, smem, st>>>(bp, gy_scan);
-        }
-    }
-    SNNK_CUDA(cudaGetLastError());
-    ProfScope ps2(SNNK_K_REDUCE_OUT, st);
-    k_wout_grad<<<dim3(pl.n_pwout, d->H / 128), 128, 0, st>>>(d->B * d->T, d->H, d->O, zbits, gy_scan, bp.part_wout,
-                                                             bp.part_db);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_HEAD, k_readout_scan, d->B, 128, smem, st, d->T, d->H, d->O, d->kappa, fp.zbits, fp.W_out, fp.b_out,
+                  fp.y, fp.logits, fp.tstar);
 }
 
-int launch_bwd_wide(const SnnkDesc* d, const BwdParams& bp, bool rec, const Plan& pl, float* gy_scan,
-                    const uint32_t* zbits, cudaStream_t st)
+int launch_fwd_gen(const SnnkDesc* d, const FwdParams& fp, bool rec, const Plan& pl, cudaStream_t st)
 {
-    return gen_npt(d->H) == 1 ? launch_bwd_wide_t<1, 4>(d, bp, rec, pl, gy_scan, zbits, st)
-                              : launch_bwd_wide_t<2, 2>(d, bp, rec, pl, gy_scan, zbits, st);
+    auto go = [&](auto npt, auto r) -> int {
+        constexpr int NPT = decltype(npt)::value, R = decltype(r)::value;
+        const size_t smem = sizeof(float) * 2 * (size_t)d->H * R;
+        return launch(SNNK_K_RECUR_FWD, rec ? k_recur_fwd_gen<NPT, R, true> : k_recur_fwd_gen<NPT, R, false>, pl.grid_rows,
+                      d->H / NPT, smem, st, fp);
+    };
+    return gen_npt(d->H) == 1 ? go(Int<1>{}, Int<4>{}) : go(Int<2>{}, Int<2>{});
+}
+
+// writes the readout-adjoint scan itself
+int launch_bwd_gen(const SnnkDesc* d, const BwdParams& bp, bool rec, const Plan& pl, float* gy_scan, cudaStream_t st)
+{
+    auto go = [&](auto npt, auto r) -> int {
+        constexpr int NPT = decltype(npt)::value, R = decltype(r)::value;
+        const size_t smem = sizeof(float) * (2 * (size_t)d->H * R + (size_t)R * d->T * kOMax);
+        if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
+        return launch(SNNK_K_RECUR_BWD, rec ? k_recur_bwd_gen<NPT, R, true> : k_recur_bwd_gen<NPT, R, false>, pl.grid_rows,
+                      d->H / NPT, smem, st, bp, gy_scan);
+    };
+    return gen_npt(d->H) == 1 ? go(Int<1>{}, Int<4>{}) : go(Int<2>{}, Int<2>{});
 }
 
 // pass 0: raster (+ change flags when chg != null)          k_encode
@@ -1020,10 +926,7 @@ int snnk_unpack_raster(const uint32_t* bits, int64_t n_rows, int32_t n_pix, floa
     if (!device_ok()) return SNNK_ERR_DEVICE;
     const long long total = n_rows * (long long)n_pix;
     const unsigned grid = (unsigned)std::min<long long>((total + 255) / 256, 32ll * sm_count());
-    ProfScope ps(SNNK_K_ENCODE, static_cast<cudaStream_t>(stream));
-    k_unpack_raster<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(bits, n_rows, n_pix, out);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_ENCODE, k_unpack_raster, grid, 256, 0, static_cast<cudaStream_t>(stream), bits, n_rows, n_pix, out);
 }
 
 size_t snnk_run_table_bytes(int64_t n_items, int32_t n_steps)
@@ -1170,100 +1073,83 @@ static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, co
     const Plan pl = make_plan(d);
     if (workspace_bytes < pl.fwd_bytes) return SNNK_ERR_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
+    char* ws = static_cast<char*>(workspace);
     float* I_in = static_cast<float*>(workspace);
+    // frame-dedup variant (runs.cuh): only for inputs the caller vouches to be the encoder's {0,1} raster
+    const int* runs = pl.dedup ? run_table : nullptr;
 
-    const int* compact_table = nullptr;
-    const float* compact_rows = nullptr;
-    Fork* fk = nullptr;
     // K1: input projection for all T steps at once.  Tensor-core path first (when asked for and addressable by
     // TMA); the fp32 SIMT kernel behind it only runs if x turned out not to be tf32-exact (device-side flag).
-    {
-        const int M = d->B * d->T;
-        unsigned int* flag = nullptr;
-        if ((d->flags & SNNK_F_INPUT_BITS) && !pl.bits) return SNNK_ERR_UNSUPPORTED;
-        if (pl.bits) {
-            // bit-packed raster: the words are expanded inside the GEMM's shared-memory tiles (gemm_bits.cuh)
-            void* planes_h = static_cast<char*>(workspace) + pl.off_wplanes;
-            const uint32_t* xb = reinterpret_cast<const uint32_t*>(x);
-            switch (pl.tileN) {
-            case 32: rc = launch_proj_bits<32>(d, xb, W_in, I_in, planes_h, st); break;
-            case 64: rc = launch_proj_bits<64>(d, xb, W_in, I_in, planes_h, st); break;
-            default: rc = launch_proj_bits<128>(d, xb, W_in, I_in, planes_h, st); break;
-            }
+    const int M = d->B * d->T;
+    unsigned int* flag = nullptr;
+    float* compact_rows = nullptr;
+    // With a run table the weight planes, the dense launch (which skips itself when the table says ok) and the
+    // preparation of the recurrent matrix go onto a parallel branch beside gather + compact projection; joined before K2.
+    Fork* fk = nullptr;
+    cudaStream_t side = st;
+    if ((d->flags & SNNK_F_INPUT_BITS) && !pl.bits) return SNNK_ERR_UNSUPPORTED;
+    if (pl.bits) {
+        // bit-packed raster: the words are expanded inside the GEMM's shared-memory tiles (gemm_bits.cuh)
+        const uint32_t* xb = reinterpret_cast<const uint32_t*>(x);
+        rc = by_width(pl.tileN, [&](auto tn) {
+            return launch_proj_bits<decltype(tn)::value>(d, xb, W_in, I_in, ws + pl.off_wplanes, st);
+        });
+        if (rc != SNNK_OK) return rc;
+    } else if (pl.tc) {
+        float* planes = reinterpret_cast<float*>(ws + pl.off_wplanes);
+        if (pl.check) {
+            flag = reinterpret_cast<unsigned int*>(ws + pl.off_fflag);
+            SNNK_CUDA(cudaMemsetAsync(flag, 0, sizeof(unsigned int), st));
+        }
+        if (runs) {   // side: weight planes -> [mid] -> dense launch, k_prep_rec;  main: gather -> wait mid -> compact GEMM
+            rc = fork_for_device(&fk);
             if (rc != SNNK_OK) return rc;
-        } else if (pl.tc) {
-            char* ws = static_cast<char*>(workspace);
-            float* planes = reinterpret_cast<float*>(ws + pl.off_wplanes);
-            if (pl.check) {
-                flag = reinterpret_cast<unsigned int*>(ws + pl.off_fflag);
-                SNNK_CUDA(cudaMemsetAsync(flag, 0, sizeof(unsigned int), st));
-            }
-            // frame-dedup variant (runs.cuh): only for inputs the caller vouches to be the encoder's {0,1} raster
-            const int* runs = (pl.runs && !pl.check) ? run_table : nullptr;
-            // With a run table the dense launch (which skips itself when the table says ok) and the preparation of the
-            // recurrent matrix go onto a parallel branch beside gather + compact projection; joined before K2.
-            fk = (runs && !pl.wide) ? fork_for_device() : nullptr;
-            cudaStream_t st_d = st;
-            if (fk) {   // side: weight planes -> [mid] -> dense launch, k_prep_rec;  main: gather -> wait mid -> compact GEMM
-                SNNK_CUDA(cudaEventRecord(fk->forked, st));
-                SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked, 0));
-                st_d = fk->side;
-                const int n = d->H * pl.kpad;
-                tc::k_split_w<<<(n + 255) / 256, 256, 0, st_d>>>(W_in, d->N, d->H, pl.kpad, planes);
-                SNNK_CUDA(cudaGetLastError());
-                SNNK_CUDA(cudaEventRecord(fk->mid, st_d));
-            }
-            switch (pl.tileN) {
-            case 32: rc = launch_proj_tc<32>(d, pl, x, W_in, I_in, planes, flag, st_d, runs, 0, fk == nullptr); break;
-            case 64: rc = launch_proj_tc<64>(d, pl, x, W_in, I_in, planes, flag, st_d, runs, 0, fk == nullptr); break;
-            default: rc = launch_proj_tc<128>(d, pl, x, W_in, I_in, planes, flag, st_d, runs, 0, fk == nullptr); break;
-            }
-            if (rc != SNNK_OK) return rc;
-            if (runs) {
-                float* Xu = reinterpret_cast<float*>(ws + pl.off_xu_f);
-                float* Iu = reinterpret_cast<float*>(ws + pl.off_iu);
-                if (d->flags & SNNK_F_RUNS_TILED) {
-                    // the encoder left the tiled compact rows behind the table (snnk_encode_runs, lazy & 2)
-                    Xu = reinterpret_cast<float*>(reinterpret_cast<char*>(const_cast<int32_t*>(runs)) +
-                                                  run_table_tiled_offset(d->B, d->T));
-                } else {
-                    ProfScope ps(SNNK_K_PROJ, st);
-                    k_gather_rows_tiled<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, st>>>(x, runs, M, d->N, pl.kpad, Xu);
-                    SNNK_CUDA(cudaGetLastError());
-                }
-                // few compact tiles: 32-column CTA tiles spread each over H/32 SMs (the tile time is bound by what one
-                // SM can pull in, two thirds of which are weight planes)
-                if (fk) SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));
-                rc = launch_proj_tc<32>(d, pl, Xu, W_in, Iu, planes, nullptr, st, runs, 1);
+            side = fk->side;
+            SNNK_CUDA(cudaEventRecord(fk->forked, st));
+            SNNK_CUDA(cudaStreamWaitEvent(side, fk->forked, 0));
+        }
+        const int n = d->H * pl.kpad;
+        tc::k_split_w<<<(n + 255) / 256, 256, 0, side>>>(W_in, d->N, d->H, pl.kpad, planes);
+        SNNK_CUDA(cudaGetLastError());
+        if (fk) SNNK_CUDA(cudaEventRecord(fk->mid, side));
+        rc = by_width(pl.tileN, [&](auto tn) {
+            return launch_proj_tc<decltype(tn)::value>(d, pl, x, I_in, planes, flag, side, runs, 0);
+        });
+        if (rc != SNNK_OK) return rc;
+        if (runs) {
+            float* Xu = reinterpret_cast<float*>(ws + pl.off_xu_f);
+            compact_rows = reinterpret_cast<float*>(ws + pl.off_iu);
+            if (d->flags & SNNK_F_RUNS_TILED) {
+                // the encoder left the tiled compact rows behind the table (snnk_encode_runs, lazy & 2)
+                Xu = reinterpret_cast<float*>(reinterpret_cast<char*>(const_cast<int32_t*>(runs)) +
+                                              run_table_tiled_offset(d->B, d->T));
+            } else {
+                rc = launch(SNNK_K_PROJ, k_gather_rows_tiled, std::min(pl.run_rows, 8 * sm_count()), 256, 0, st, x, runs, M,
+                            d->N, pl.kpad, Xu);
                 if (rc != SNNK_OK) return rc;
-                if (pl.wide) {   // k_recur_fwd / k_recur_fwd_tc fetch the compact rows themselves
-                    const long long nthr = (long long)M * (d->H / 4);
-                    k_expand_rows<<<(unsigned)((nthr + 255) / 256), 256, 0, st>>>(Iu, runs, M, d->H, I_in);
-                    SNNK_CUDA(cudaGetLastError());
-                } else {
-                    compact_table = runs;
-                    compact_rows = Iu;
-                }
             }
+            // few compact tiles: 32-column CTA tiles spread each over H/32 SMs (the tile time is bound by what one
+            // SM can pull in, two thirds of which are weight planes)
+            SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));
+            rc = launch_proj_tc<32>(d, pl, Xu, compact_rows, planes, nullptr, st, runs, 1);
+            if (rc != SNNK_OK) return rc;
         }
-        if (!pl.bits && (!pl.tc || pl.check)) {
-            dim3 grid((M + kGemmBM - 1) / kGemmBM, pl.ntiles);
-            ProfScope ps(pl.tc ? SNNK_K_PROJ_FALLBACK : SNNK_K_PROJ, st);
-            if (pl.BN == 64) k_proj_simt<64><<<grid, kGemmThreads, 0, st>>>(x, W_in, I_in, M, d->N, d->H, flag);
-            else k_proj_simt<32><<<grid, kGemmThreads, 0, st>>>(x, W_in, I_in, M, d->N, d->H, flag);
-            SNNK_CUDA(cudaGetLastError());
-        }
+    }
+    if (!pl.bits && (!pl.tc || pl.check)) {
+        rc = launch(pl.tc ? SNNK_K_PROJ_FALLBACK : SNNK_K_PROJ, pl.BN == 64 ? k_proj_simt<64> : k_proj_simt<32>,
+                    dim3((M + kGemmBM - 1) / kGemmBM, pl.ntiles), kGemmThreads, 0, st, x, W_in, I_in, M, d->N, d->H, flag);
+        if (rc != SNNK_OK) return rc;
     }
     // K2: fused recurrence + readout
     float* W_eff = nullptr;
     if (d->recurrent) {
-        W_eff = reinterpret_cast<float*>(static_cast<char*>(workspace) + pl.off_weff);
+        W_eff = reinterpret_cast<float*>(ws + pl.off_weff);
         const int n = d->H * d->H;
-        k_prep_rec<<<(n + 255) / 256, 256, 0, fk ? fk->side : st>>>(W_rec, rec_mask, d->H, W_eff, W_effT_out);
+        k_prep_rec<<<(n + 255) / 256, 256, 0, side>>>(W_rec, rec_mask, d->H, W_eff, W_effT_out);
         SNNK_CUDA(cudaGetLastError());
     }
     if (fk) {
-        SNNK_CUDA(cudaEventRecord(fk->joined, fk->side));
+        SNNK_CUDA(cudaEventRecord(fk->joined, side));
         SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined, 0));
     }
     FwdParams fp{};
@@ -1274,40 +1160,33 @@ static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, co
     fp.I_in = I_in; fp.W_eff = W_eff; fp.beta = beta; fp.W_out = W_out; fp.b_out = b_out;
     fp.V0 = V0; fp.a0 = a0; fp.Z0 = Z0; fp.V = V; fp.a = a; fp.Z = Z; fp.zbits = zbits; fp.y = y;
     fp.logits = logits; fp.tstar = tstar;
-    fp.run_table = compact_table; fp.I_u = compact_rows;
+    fp.run_table = runs; fp.I_u = compact_rows;   // k_recur_fwd / k_recur_fwd_tc fetch the compact rows themselves
     const bool rec = d->recurrent != 0;
     // the register-resident recurrence evaluates the head in its own tail; every other kernel family is followed by
     // the stand-alone head kernel (same arithmetic, same summation order)
-    const bool fused_head = head && !pl.wide && !pl.tcrec && !pl.nr;
+    const bool fused_head = head && pl.readout_in_sweep();
     if (fused_head) {
         fp.labels = reinterpret_cast<const long long*>(head->labels); fp.logp = head->logp; fp.g_logits = head->g_logits;
         fp.loss = head->loss; fp.part_nll = static_cast<float*>(head->head_ws);
         fp.ticket = reinterpret_cast<unsigned int*>(static_cast<float*>(head->head_ws) + d->B);
         fp.mailbox = reinterpret_cast<unsigned long long*>(head->mailbox); fp.mail_counter = head->counter;
     }
-    if (pl.wide && pl.widetc) {
-        rc = launch_wide_fwd(wide_params(fp, pl, static_cast<char*>(workspace)), st);
+    switch (pl.family) {
+    case Family::WideTc:
+        rc = launch_wide_fwd(wide_params(fp, pl, ws), st);
         if (rc == SNNK_OK) rc = launch_readout_scan(d, fp, st);
-    } else if (pl.wide) {
-        rc = launch_fwd_wide(d, fp, rec, pl, st);
-    } else if (pl.tcrec) {
-        rc = launch_fwd_tc(fp, st);
-    } else if (pl.nr) {
-        rc = launch_nonrec_fwd(fp, st);
-    } else {
-        if (use_lean_fwd(fp, rec, pl.R)) {
-            // behind a tensor-core projection on the same stream (not while the per-kernel profiler brackets launches
-            // with events); SNNK_PDL=0/1 is the measuring switch
-            const char* env = getenv("SNNK_PDL");
-            const bool pdl = pl.tc && !g_prof_on && (env ? env[0] != '0' : kPdlDefault);
-            rc = launch_fwd_lean(fp, st, pdl);
-        }
-        else switch (d->H) {
-        case 32: rc = launch_fwd_r<32>(fp, rec, pl.R, pl.grid_rows, st); break;
-        case 64: rc = launch_fwd_r<64>(fp, rec, pl.R, pl.grid_rows, st); break;
-        case 128: rc = launch_fwd_r<128>(fp, rec, pl.R, pl.grid_rows, st); break;
-        default: rc = SNNK_ERR_UNSUPPORTED;
-        }
+        break;
+    case Family::WideGen:
+        rc = launch_fwd_gen(d, fp, rec, pl, st);
+        if (rc == SNNK_OK) rc = launch_readout_scan(d, fp, st);
+        break;
+    case Family::TcRec: rc = launch_fwd_tc(fp, st); break;
+    case Family::NonRec: rc = launch_nonrec_fwd(fp, st); break;
+    case Family::Simt:
+        // the lean kernel is a programmatic dependent of a tensor-core projection on the same stream (not while the
+        // per-kernel profiler brackets launches with events)
+        rc = pl.lean_fwd ? launch_fwd_lean(fp, st, pl.tc && !g_prof_on) : launch_fwd_simt(fp, rec, pl, st);
+        break;
     }
     if (rc != SNNK_OK || !head || fused_head) return rc;
     return snnk_head_nll(d->B, d->O, logits, head->labels, head->logp, head->loss, head->g_logits, head->mailbox,
@@ -1345,13 +1224,24 @@ int snnk_head_nll(int32_t B, int32_t O, const float* logits, const int64_t* labe
     if ((loss_mailbox != nullptr) != (mailbox_counter != nullptr)) return SNNK_ERR_ARG;
     if (B <= 0 || O <= 0 || O > kOMax) return SNNK_ERR_SHAPE;
     if (!device_ok()) return SNNK_ERR_DEVICE;
-    {
-        ProfScope ps(SNNK_K_HEAD, static_cast<cudaStream_t>(stream));
-        k_head_nll<<<1, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-            B, O, logits, reinterpret_cast<const long long*>(labels), logp, loss, g_logits,
-            reinterpret_cast<unsigned long long*>(loss_mailbox), mailbox_counter);
+    return launch(SNNK_K_HEAD, k_head_nll, 1, 256, 0, static_cast<cudaStream_t>(stream), B, O, logits,
+                  reinterpret_cast<const long long*>(labels), logp, loss, g_logits,
+                  reinterpret_cast<unsigned long long*>(loss_mailbox), mailbox_counter);
+}
+
+// The tensor list of both Adam entry points (1 <= count <= kAdamMaxTensors, non-null arrays), checked and packed
+static int adam_tensors(int32_t count, float* const* params, const float* const* grads, float* const* exp_avg,
+                        float* const* exp_avg_sq, float* const* steps, const int64_t* numel, AdamTensors* t)
+{
+    *t = AdamTensors{};
+    t->count = count;
+    long long total = 0;
+    for (int k = 0; k < count; ++k) {
+        if (!params[k] || !grads[k] || !exp_avg[k] || !exp_avg_sq[k] || !steps[k] || numel[k] < 0) return SNNK_ERR_ARG;
+        t->p[k] = params[k]; t->g[k] = grads[k]; t->m[k] = exp_avg[k]; t->v[k] = exp_avg_sq[k]; t->step[k] = steps[k];
+        t->n[k] = numel[k]; t->start[k] = total; total += numel[k];
     }
-    SNNK_CUDA(cudaGetLastError());
+    t->start[count] = total;
     return SNNK_OK;
 }
 
@@ -1363,20 +1253,12 @@ int snnk_adam_step(int32_t count, float* const* params, const float* const* grad
     if (count == 0) return SNNK_OK;
     if (!params || !grads || !exp_avg || !exp_avg_sq || !steps || !numel) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
-    AdamTensors t{};
-    t.count = count;
-    long long total = 0;
-    for (int k = 0; k < count; ++k) {
-        if (!params[k] || !grads[k] || !exp_avg[k] || !exp_avg_sq[k] || !steps[k] || numel[k] < 0) return SNNK_ERR_ARG;
-        t.p[k] = params[k]; t.g[k] = grads[k]; t.m[k] = exp_avg[k]; t.v[k] = exp_avg_sq[k]; t.step[k] = steps[k];
-        t.n[k] = numel[k]; t.start[k] = total; total += numel[k];
-    }
-    t.start[count] = total;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    ProfScope ps(SNNK_K_ADAM, st);
-    k_adam_step<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(t, lr, beta1, beta2, eps, weight_decay);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    AdamTensors t;
+    const int rc = adam_tensors(count, params, grads, exp_avg, exp_avg_sq, steps, numel, &t);
+    if (rc != SNNK_OK) return rc;
+    const long long total = t.start[count];
+    return launch(SNNK_K_ADAM, k_adam_step, (unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream), t,
+                  lr, beta1, beta2, eps, weight_decay);
 }
 
 int snnk_adam_dp_buffer_bytes(int32_t world, int64_t total_numel, size_t* bytes)
@@ -1397,15 +1279,10 @@ int snnk_adam_step_dp(int32_t count, float* const* params, float* const* grads, 
     if (count == 0) return SNNK_OK;
     if (!params || !grads || !exp_avg || !exp_avg_sq || !steps || !numel || !peer_buffers || !state) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
-    AdamTensors t{};
-    t.count = count;
-    long long total = 0;
-    for (int k = 0; k < count; ++k) {
-        if (!params[k] || !grads[k] || !exp_avg[k] || !exp_avg_sq[k] || !steps[k] || numel[k] < 0) return SNNK_ERR_ARG;
-        t.p[k] = params[k]; t.g[k] = grads[k]; t.m[k] = exp_avg[k]; t.v[k] = exp_avg_sq[k]; t.step[k] = steps[k];
-        t.n[k] = numel[k]; t.start[k] = total; total += numel[k];
-    }
-    t.start[count] = total;
+    AdamTensors t;
+    const int rc = adam_tensors(count, params, grads, exp_avg, exp_avg_sq, steps, numel, &t);
+    if (rc != SNNK_OK) return rc;
+    const long long total = t.start[count];
     AdamDp dp{};
     dp.rank = rank; dp.world = world; dp.state = state;
     {   // two-phase exchange from 4 ranks on (at 2 the all-to-all IS one hop and one word); SNNK_DP_RSAG=0/1 forces it --
@@ -1418,15 +1295,12 @@ int snnk_adam_step_dp(int32_t count, float* const* params, float* const* grads, 
         if (reinterpret_cast<uintptr_t>(peer_buffers[r]) & 7) return SNNK_ERR_ARG;
         dp.slots[r] = static_cast<unsigned long long*>(peer_buffers[r]);
     }
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    ProfScope ps(SNNK_K_ADAM, st);
     // one gradient element per thread: every remote store of the step is in flight at once.  Threads only wait for
     // REMOTE data, never for another local CTA, so the grid need not be co-resident.
     const long long want = (total + 255) / 256;
     const unsigned grid = (unsigned)std::min<long long>(want, 8ll * sm_count());
-    k_adam_step_dp<<<grid, 256, 0, st>>>(t, dp, lr, beta1, beta2, eps, weight_decay);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_ADAM, k_adam_step_dp, grid, 256, 0, static_cast<cudaStream_t>(stream), t, dp, lr, beta1, beta2,
+                  eps, weight_decay);
 }
 
 int snnk_input_grad(const SnnkDesc* d, const float* gI, const float* W_in, float* gX, snnk_stream_t stream)
@@ -1435,13 +1309,9 @@ int snnk_input_grad(const SnnkDesc* d, const float* gI, const float* W_in, float
     if (rc != SNNK_OK) return rc;
     if (!gI || !W_in || !gX) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int M = d->B * d->T;
-    dim3 grid((M + kGemmBM - 1) / kGemmBM, (d->N + 63) / 64);
-    ProfScope ps(SNNK_K_INPUT_GRAD, st);
-    k_input_grad_simt<<<grid, kGemmThreads, 0, st>>>(gI, W_in, gX, M, d->H, d->N);
-    SNNK_CUDA(cudaGetLastError());
-    return SNNK_OK;
+    return launch(SNNK_K_INPUT_GRAD, k_input_grad_simt, dim3((M + kGemmBM - 1) / kGemmBM, (d->N + 63) / 64), kGemmThreads,
+                  0, static_cast<cudaStream_t>(stream), gI, W_in, gX, M, d->H, d->N);
 }
 
 int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const float* rec_mask, const float* beta,
@@ -1468,17 +1338,25 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
     float* pdb = reinterpret_cast<float*>(ws + pl.off_pdb);
     float* pw = reinterpret_cast<float*>(ws + pl.off_pw);
     const bool rec = d->recurrent != 0;
+    const int* runs = pl.dedup ? run_table : nullptr;
+    float* gy_scan = reinterpret_cast<float*>(ws + pl.off_gyscan);
 
+    // Parallel branches: the gather of the dedup variant, and the dW_out / db partials of the tensor-core and
+    // non-recurrent sweeps
+    const bool wout_beside = pl.family == Family::TcRec || pl.family == Family::NonRec;
+    Fork* fk = nullptr;
+    if (runs || wout_beside) {
+        rc = fork_for_device(&fk);
+        if (rc != SNNK_OK) return rc;
+    }
     // dedup variant: the compact rows of x for the dW_in GEMM do not depend on the sweep -- gathered beside it
-    const int* runs_b = (pl.tc && pl.runs && !pl.check) ? run_table : nullptr;
-    Fork* fkb = runs_b ? fork_for_device() : nullptr;
-    if (fkb) {
-        SNNK_CUDA(cudaEventRecord(fkb->forked, st));
-        SNNK_CUDA(cudaStreamWaitEvent(fkb->side, fkb->forked, 0));
-        k_gather_rows<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, fkb->side>>>(
-            x, runs_b, d->B * d->T, d->N, reinterpret_cast<float*>(ws + pl.off_xu_b));
+    if (runs) {
+        SNNK_CUDA(cudaEventRecord(fk->forked, st));
+        SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked, 0));
+        k_gather_rows<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, fk->side>>>(
+            x, runs, d->B * d->T, d->N, reinterpret_cast<float*>(ws + pl.off_xu_b));
         SNNK_CUDA(cudaGetLastError());
-        SNNK_CUDA(cudaEventRecord(fkb->mid, fkb->side));
+        SNNK_CUDA(cudaEventRecord(fk->mid, fk->side));
     }
     // K3: reverse-time sweep
     const float* W_effT = nullptr;
@@ -1501,21 +1379,16 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
     bp.tstar = dense ? nullptr : tstar; bp.g_scale = g_scale; bp.g_V = g_V; bp.g_Z = g_Z;
     float* gI_lo = pl.tc ? reinterpret_cast<float*>(ws + pl.off_gIlo) : nullptr;
     bp.gI = gI; bp.gI_lo = gI_lo; bp.part_wout = pwout; bp.part_db = pdb;
-    if (pl.tc && pl.runs && !pl.check && run_table) {
-        bp.run_table = run_table;
+    if (runs) {
+        bp.run_table = runs;
         bp.Gu_hi = reinterpret_cast<float*>(ws + pl.off_gu);
         bp.Gu_lo = reinterpret_cast<float*>(ws + pl.off_gu + pl.gu_plane);
     }
-    Fork* fkw = nullptr;
-    if (pl.wide && pl.widetc) {
+    switch (pl.family) {
+    case Family::WideTc: {
         // weight-stationary tensor-core sweep (recur_wide.cuh): adjoint scan, sweep, then dW_out / db from the scan
-        float* gy_scan = reinterpret_cast<float*>(ws + pl.off_gyscan);
-        {
-            ProfScope ps(SNNK_K_REDUCE_OUT, st);
-            k_gy_scan<<<(d->B * kOMax + 255) / 256, 256, 0, st>>>(d->B, d->T, d->O, d->kappa, bp.g_y, bp.g_logits, bp.tstar,
-                                                               bp.g_scale, gy_scan);
-            SNNK_CUDA(cudaGetLastError());
-        }
+        rc = launch_gy_scan(d, bp, gy_scan, st);
+        if (rc != SNNK_OK) return rc;
         WideBwdParams wp{};
         wp.B = d->B; wp.T = d->T; wp.H = d->H; wp.O = d->O; wp.alif = bp.alif; wp.surrogate = bp.surrogate;
         wp.alpha = bp.alpha; wp.theta = bp.theta; wp.gamma = bp.gamma;
@@ -1526,44 +1399,28 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
         wp.flags = reinterpret_cast<unsigned int*>(ws + pl.off_wflags_b);
         wp.n_mt = pl.w_nmt_b; wp.n_nt = pl.w_nnt;
         rc = launch_wide_bwd(wp, pl.w_npass_b, st);
-        if (rc != SNNK_OK) return rc;
-        ProfScope ps2(SNNK_K_REDUCE_OUT, st);
-        k_wout_grad<<<dim3(pl.n_pwout, d->H / 128), 128, 0, st>>>(d->B * d->T, d->H, d->O, zbits, gy_scan, pwout, pdb);
-        SNNK_CUDA(cudaGetLastError());
-    } else if (pl.wide) {
-        rc = launch_bwd_wide(d, bp, rec, pl, reinterpret_cast<float*>(ws + pl.off_gyscan), zbits, st);
-    } else if (pl.tcrec || pl.nr) {
+        if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
+        break;
+    }
+    case Family::WideGen:
+        rc = launch_bwd_gen(d, bp, rec, pl, gy_scan, st);
+        if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
+        break;
+    case Family::TcRec:
+    case Family::NonRec:
         // readout-adjoint scan first; dW_out / db (a contraction of it with the spike raster) beside the sweep
-        float* gy_scan = reinterpret_cast<float*>(ws + pl.off_gyscan);
-        {
-            ProfScope ps(SNNK_K_REDUCE_OUT, st);
-            k_gy_scan<<<(d->B * kOMax + 255) / 256, 256, 0, st>>>(d->B, d->T, d->O, d->kappa, bp.g_y, bp.g_logits, bp.tstar,
-                                                               bp.g_scale, gy_scan);
-            SNNK_CUDA(cudaGetLastError());
-        }
-        fkw = fork_for_device();
-        cudaStream_t st_w = st;
-        if (fkw) {
-            SNNK_CUDA(cudaEventRecord(fkw->forked3, st));
-            SNNK_CUDA(cudaStreamWaitEvent(fkw->side, fkw->forked3, 0));
-            st_w = fkw->side;
-        }
-        {
-            ProfScope ps(SNNK_K_REDUCE_OUT, st_w);
-            k_wout_grad<<<dim3(pl.n_pwout, (d->H + 127) / 128), 128, 0, st_w>>>(d->B * d->T, d->H, d->O, zbits, gy_scan, pwout, pdb);
-            SNNK_CUDA(cudaGetLastError());
-        }
-        if (fkw) SNNK_CUDA(cudaEventRecord(fkw->joined3, fkw->side));
-        rc = pl.tcrec ? launch_bwd_tc(bp, gy_scan, st) : launch_nonrec_bwd(bp, gy_scan, st);
-    } else if (use_lean_bwd(bp, rec, pl.R)) {
-        rc = launch_bwd_lean(bp, st);
-    } else {
-        switch (d->H) {
-        case 32: rc = launch_bwd_r<32>(bp, rec, pl.R, pl.grid_rows, st); break;
-        case 64: rc = launch_bwd_r<64>(bp, rec, pl.R, pl.grid_rows, st); break;
-        case 128: rc = launch_bwd_r<128>(bp, rec, pl.R, pl.grid_rows, st); break;
-        default: rc = SNNK_ERR_UNSUPPORTED;
-        }
+        rc = launch_gy_scan(d, bp, gy_scan, st);
+        if (rc != SNNK_OK) return rc;
+        SNNK_CUDA(cudaEventRecord(fk->forked3, st));
+        SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked3, 0));
+        rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, fk->side);
+        if (rc != SNNK_OK) return rc;
+        SNNK_CUDA(cudaEventRecord(fk->joined3, fk->side));
+        rc = pl.family == Family::TcRec ? launch_bwd_tc(bp, gy_scan, st) : launch_nonrec_bwd(bp, gy_scan, st);
+        break;
+    case Family::Simt:
+        rc = use_lean_bwd(bp, rec, pl.R) ? launch_bwd_lean(bp, st) : launch_bwd_simt(bp, rec, pl, st);
+        break;
     }
     if (rc != SNNK_OK) return rc;
     // K4: weight-gradient GEMM (split-K partials over whole samples, then a fixed-order reduction)
@@ -1573,26 +1430,22 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
         if (pl.bits) {
             const uint32_t* xb = reinterpret_cast<const uint32_t*>(x);
             const size_t gstride = pl.off_gIlo - pl.off_gI;
-            switch (pl.tileN) {
-            case 32: rc = launch_wgrad_bits<32>(d, pl, xb, zbits, gI, gstride, pw, st); break;
-            case 64: rc = launch_wgrad_bits<64>(d, pl, xb, zbits, gI, gstride, pw, st); break;
-            default: rc = launch_wgrad_bits<128>(d, pl, xb, zbits, gI, gstride, pw, st); break;
-            }
+            rc = by_width(pl.tileN, [&](auto tn) {
+                return launch_wgrad_bits<decltype(tn)::value>(d, pl, xb, zbits, gI, gstride, pw, st);
+            });
             if (rc != SNNK_OK) return rc;
         } else if (pl.tc) {
             if (pl.check) {
                 flag = reinterpret_cast<unsigned int*>(ws + pl.off_flag);
                 SNNK_CUDA(cudaMemsetAsync(flag, 0, sizeof(unsigned int), st));
             }
-            const int* runs = (pl.runs && !pl.check) ? run_table : nullptr;
             WgradGeom g{};
             g.x = x; g.Ztrace = rec ? Z : nullptr; g.g_planes = gI; g.g_plane_stride = pl.off_gIlo - pl.off_gI;
             g.T = d->T; g.B = d->B; g.N = d->N; g.mtiles_x = pl.mtiles_x; g.mtiles_z = pl.mtiles_z; g.m_total = pl.m_total;
             g.S = pl.S; g.samples_per_split = pl.samples_per_split; g.part = pw; g.flag = flag;
             g.run_table = runs; g.run_gate = 0; g.run_clip = 0;
-            Fork* fk = runs ? fkb : nullptr;
             cudaStream_t st_b = st;
-            if (fk) {   // dense (self-skipping) launch + Z-only GEMM on a parallel branch beside the compact GEMM
+            if (runs) {   // dense (self-skipping) launch + Z-only GEMM on a parallel branch beside the compact GEMM
                 SNNK_CUDA(cudaEventRecord(fk->forked2, st));
                 SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked2, 0));
                 st_b = fk->side;
@@ -1602,8 +1455,6 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
             if (runs) {
                 // dedup variant: x-only GEMM over the compact rows (run sums of gI come from the BPTT sweep) and Z-only
                 // GEMM over the dense rows; the two are independent
-                float* Xu = reinterpret_cast<float*>(ws + pl.off_xu_b);
-                float* Gu = reinterpret_cast<float*>(ws + pl.off_gu);
                 if (rec) {
                     WgradGeom gb = g;
                     gb.x = nullptr; gb.N = 0; gb.mtiles_x = 0; gb.m_total = d->H; gb.S = pl.S_rec;
@@ -1612,24 +1463,17 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
                     rc = launch_wgrad_tc_any(d, pl.tileN, gb, st_b);
                     if (rc != SNNK_OK) return rc;
                 }
-                if (!fk) {
-                    ProfScope ps(SNNK_K_WGRAD, st);
-                    k_gather_rows<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, st>>>(x, runs, d->B * d->T, d->N, Xu);
-                    SNNK_CUDA(cudaGetLastError());
-                } else {
-                    SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));   // the gather issued beside the sweep
-                }
+                SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));   // the gather issued beside the sweep
                 WgradGeom ga{};
-                ga.x = Xu; ga.Ztrace = nullptr; ga.g_planes = Gu; ga.g_plane_stride = pl.gu_plane;
+                ga.x = reinterpret_cast<float*>(ws + pl.off_xu_b); ga.Ztrace = nullptr;
+                ga.g_planes = reinterpret_cast<float*>(ws + pl.off_gu); ga.g_plane_stride = pl.gu_plane;
                 ga.T = pl.run_rows; ga.B = 1; ga.N = d->N; ga.mtiles_x = pl.mtiles_x; ga.mtiles_z = 0; ga.m_total = pl.m_total;
                 ga.S = pl.S_cmp; ga.samples_per_split = 1; ga.part = pw; ga.flag = nullptr;
                 ga.run_table = runs; ga.run_gate = 1; ga.run_clip = 1;
                 rc = launch_wgrad_tc_any(d, pl.tileN, ga, st);
                 if (rc != SNNK_OK) return rc;
-                if (fk) {
-                    SNNK_CUDA(cudaEventRecord(fk->joined, fk->side));
-                    SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined, 0));
-                }
+                SNNK_CUDA(cudaEventRecord(fk->joined, fk->side));
+                SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined, 0));
             }
         }
         WgradParams wp{};
@@ -1638,31 +1482,28 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
         wp.x = x; wp.zbits = zbits; wp.Z0 = Z0; wp.gI = gI; wp.gI_lo = gI_lo; wp.run_if_flag = flag;
         wp.part = pw; wp.m_total = pl.m_total;
         if (!pl.bits && (!pl.tc || pl.check)) {
-            dim3 grid(pl.mtiles_x + pl.mtiles_z, pl.ntiles, pl.S);
-            ProfScope ps(pl.tc ? SNNK_K_WGRAD_FALLBACK : SNNK_K_WGRAD, st);
-            if (pl.BN == 64) k_wgrad_simt<64><<<grid, kGemmThreads, 0, st>>>(wp);
-            else k_wgrad_simt<32><<<grid, kGemmThreads, 0, st>>>(wp);
-            SNNK_CUDA(cudaGetLastError());
+            rc = launch(pl.tc ? SNNK_K_WGRAD_FALLBACK : SNNK_K_WGRAD, pl.BN == 64 ? k_wgrad_simt<64> : k_wgrad_simt<32>,
+                        dim3(pl.mtiles_x + pl.mtiles_z, pl.ntiles, pl.S), kGemmThreads, 0, st, wp);
+            if (rc != SNNK_OK) return rc;
         }
-        if (fkw) SNNK_CUDA(cudaStreamWaitEvent(st, fkw->joined3, 0));      // dW_out / db partials of the side branch
+        if (wout_beside) SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined3, 0));      // dW_out / db partials of the side branch
         // every partial buffer (dW_in, dW_rec, dW_out, db) reduced by one launch
         FinalizeParams fz{};
         fz.pw = pw; fz.S = pl.S; fz.w_stride = (size_t)pl.m_total * d->H; fz.n_in = d->N * d->H;
         fz.n_rec = rec ? d->H * d->H : 0; fz.rec_mask = rec_mask; fz.dW_in = dW_in; fz.dW_rec = dW_rec;
         fz.pwout = pwout; fz.P_out = pl.n_pwout; fz.n_out = d->H * d->O; fz.dW_out = dW_out;
         fz.pdb = pdb; fz.P_b = pl.n_pdb; fz.n_b = d->O; fz.db = db;
-        if (pl.tc && pl.runs && !pl.check && run_table && rec) {
-            fz.run_table = run_table; fz.pw_rec = reinterpret_cast<float*>(ws + pl.off_pwrec); fz.S_rec = pl.S_rec;
-            fz.rec_stride = (size_t)d->H * d->H;
+        if (runs) {
+            fz.run_table = runs; fz.S_cmp = pl.S_cmp;
+            if (rec) {
+                fz.pw_rec = reinterpret_cast<float*>(ws + pl.off_pwrec); fz.S_rec = pl.S_rec;
+                fz.rec_stride = (size_t)d->H * d->H;
+            }
         }
-        if (pl.tc && pl.runs && !pl.check && run_table) { fz.run_table = run_table; fz.S_cmp = pl.S_cmp; }
         fz.blocks_a = (fz.n_in + fz.n_rec + 255) / 256;
         const int blocks_b = (fz.n_out + fz.n_b + 7) / 8;
-        ProfScope ps2(SNNK_K_REDUCE_W, st);
-        k_finalize_grads<<<fz.blocks_a + blocks_b, 256, 0, st>>>(fz);
-        SNNK_CUDA(cudaGetLastError());
+        return launch(SNNK_K_REDUCE_W, k_finalize_grads, fz.blocks_a + blocks_b, 256, 0, st, fz);
     }
-    return SNNK_OK;
 }
 
 }  // extern "C"

@@ -154,8 +154,6 @@ class ToSpikes:
 			images = images.reshape(images.shape[0], int(np.prod(images.shape[1:])))
 		x2, _, _, _ = self._stage(images)
 		n_items, n_pix = x2.shape
-		if os.environ.get("SNNK_FRAME_RUNS", "1") == "0":     # switch for measuring the dense kernels
-			frame_runs = False
 		nbytes = _cabi.lib().snnk_run_table_bytes(n_items, self.n_steps) if (frame_runs and n_items > 0 and n_pix > 0) else 0
 		if nbytes == 0:
 			out, _ = self._run(x2, self.use_periods, out_dtype, want_periods=False)
