@@ -47,8 +47,10 @@ typedef void* snnk_stream_t; /* cudaStream_t */
 /* LayerType, src/modules/spiking_layers.py:11-14.  SNNK_IZHIKEVICH (spiking_layers.py:246-353; wider than 128: the fp32 kernels of recur_gen.cuh): the
  * `a` trace and the a0 state hold the recovery variable u; V0 == NULL starts the membrane at v_rest (:309). */
 enum { SNNK_LIF = 0, SNNK_ALIF = 1, SNNK_IZHIKEVICH = 2 };
-/* SpikeFuncType, src/modules/spike_funcs.py:7-9 */
-enum { SNNK_FAST_SIGMOID = 0, SNNK_PHI = 1 };
+/* SpikeFuncType, src/modules/spike_funcs.py:7-9.  SNNK_SURROGATE_TRACE: a user-defined SpikeFunction subclass whose
+ * derivative the caller evaluates itself and hands to snnk_backward as a trace (see there); snnk_forward and
+ * snnk_forward_nll accept it and ignore it (the forward is the same Heaviside step), snnk_spike_backward refuses it. */
+enum { SNNK_FAST_SIGMOID = 0, SNNK_PHI = 1, SNNK_SURROGATE_TRACE = 2 };
 /* element types accepted by snnk_encode */
 enum { SNNK_F32 = 0, SNNK_F64 = 1, SNNK_U8 = 2, SNNK_I64 = 3, SNNK_BITS = 4 };
 
@@ -92,7 +94,7 @@ typedef struct SnnkDesc {
     int32_t H;          /* hidden neurons                                     */
     int32_t O;          /* readout units (10); O <= 16                        */
     int32_t layer_type; /* SNNK_LIF | SNNK_ALIF | SNNK_IZHIKEVICH             */
-    int32_t surrogate;  /* SNNK_FAST_SIGMOID | SNNK_PHI                       */
+    int32_t surrogate;  /* SNNK_FAST_SIGMOID | SNNK_PHI | SNNK_SURROGATE_TRACE */
     int32_t recurrent;  /* use_recurrent_connection                           */
     float alpha;        /* exp(-dt/tau_m),  spiking_layers.py:119             */
     float rho;          /* exp(-dt/tau_a),  spiking_layers.py:199 (ALIF)      */
@@ -266,6 +268,11 @@ int snnk_forward_nll(const SnnkDesc* d, const float* x, const float* W_in, const
  * must be given.  g_V, g_Z (B,T,H) are optional extra seeds on the hidden traces.
  * V, a (ALIF), Z (B,T,H) and zbits are the traces the forward wrote (Z, the fp32 spike trace, is read by the
  * tensor-core weight-gradient GEMM only and may be NULL without SNNK_F_TENSOR_CORE).
+ * With surrogate SNNK_SURROGATE_TRACE, `a` instead holds sigma'_t = dZ_t/dV_t (B,T,H), the surrogate derivative the
+ * caller evaluated on the saved traces (threshold theta for LIF, theta + beta a_t for ALIF, v_peak for Izhikevich);
+ * the sweep streams it where it would evaluate the built-in formula.  V may then be NULL for LIF / ALIF (the
+ * derivative was its only use) and is required for Izhikevich (its membrane Jacobian reads V); beta is unused; a NULL
+ * `a` is SNNK_ERR_ARG.
  * Outputs: dW_in (N,H), dW_rec (H,H, masked; NULL iff !recurrent), dW_out (H,O), db (O); they are
  * OVERWRITTEN.  beta receives no gradient (the threshold input of the spike function has none,
  * spike_funcs.py:62).  workspace: on return its first B*T*H floats hold gI, the gradient w.r.t. the

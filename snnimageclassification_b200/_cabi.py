@@ -20,7 +20,7 @@ LIB_PATH = os.environ.get("SNNK_LIB_PATH", LIB_PATH)
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include", "snnk.h")
 
 SNNK_LIF, SNNK_ALIF, SNNK_IZHIKEVICH = 0, 1, 2
-SNNK_FAST_SIGMOID, SNNK_PHI = 0, 1
+SNNK_FAST_SIGMOID, SNNK_PHI, SNNK_SURROGATE_TRACE = 0, 1, 2
 SNNK_F32, SNNK_F64, SNNK_U8, SNNK_I64, SNNK_BITS = 0, 1, 2, 3, 4
 SNNK_F_TRACES, SNNK_F_TENSOR_CORE, SNNK_F_INPUT_BINARY, SNNK_F_INPUT_BITS, SNNK_F_RUNS_TILED = 0x1, 0x2, 0x4, 0x8, 0x10
 SNNK_MAX_CLASSES = 16   # widest readout the kernels take (SnnkDesc.O <= 16, kOMax in csrc/common.cuh)

@@ -92,6 +92,18 @@ __device__ __forceinline__ float surrogate_grad(int kind, float gamma, float v, 
     return __fmul_rn(__fdiv_rn(gamma, te), r);
 }
 
+// SNNK_SURROGATE_TRACE: the caller evaluated sigma' of a user-defined surrogate itself and snnk_backward streams it in
+// place of the V trace (include/snnk.h).
+constexpr int kSurrTrace = 2;
+
+// The same with the kind fixed at compile time, as the BPTT sweeps instantiate it; for kSurrTrace v already is sigma'.
+template <int SURR>
+__device__ __forceinline__ float surrogate_grad(float gamma, float v, float thr)
+{
+    if constexpr (SURR == kSurrTrace) return v;
+    else return surrogate_grad(SURR, gamma, v, thr);
+}
+
 // sum_k w[k] * z[k] with sixteen accumulators over k mod 16 (the order oracle/snn_oracle.c fixes), held as eight
 // float2 and advanced with the packed FFMA2 of sm_100: H/2 FMA instructions instead of H, and eight independent
 // dependency chains per warp so the FMA latency is covered without help from other warps.  Each lane of an FFMA2

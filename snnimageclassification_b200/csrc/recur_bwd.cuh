@@ -38,11 +38,13 @@ constexpr size_t bwd_smem_bytes(int T, bool rec)
     return loop > stage ? loop : stage;
 }
 
-// MODE: 0 LIF, 1 ALIF, 2 Izhikevich; SURR: 0 FastSigmoid, 1 Phi -- compile-time for the same reason as in k_recur_fwd
+// MODE: 0 LIF, 1 ALIF, 2 Izhikevich; SURR: 0 FastSigmoid, 1 Phi, 2 sigma' trace -- compile-time for the same reason as
+// in k_recur_fwd.  With the trace, LIF / ALIF run MODE 0 with sigma' in the V slot; Izhikevich streams sigma' from `a`.
 template <int H, int R, bool REC, int MODE = 1, int SURR = 0>
 __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
 {
     constexpr bool IZH = MODE == 2, ALIF = MODE == 1;
+    constexpr bool TWO = ALIF || (IZH && SURR == kSurrTrace);   // a second trace streams beside V
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int W32 = H / 32;
     const int T = p.T, O = p.O, B = p.B;
@@ -76,7 +78,7 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
     uint32_t* s_mask = reinterpret_cast<uint32_t*>(s_g + 2 * R * H);       // [R][T][W32]
     float* s_gy = reinterpret_cast<float*>(s_mask + ((R * T * W32 + 3) & ~3));   // [R][T][kOMax], 16-B aligned
     float* s_v = s_gy + R * T * kOMax;                                           // [kRing][R][kChunk][H]  V trace ring
-    float* s_a = s_v + kRing * R * kChunk * H;                                   // [kRing][R][kChunk][H]  a trace ring
+    float* s_a = s_v + kRing * R * kChunk * H;                                   // [kRing][R][kChunk][H]  a / sigma' ring
     uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_a + kRing * R * kChunk * H); // [kRing]
     uint32_t* s_start = reinterpret_cast<uint32_t*>(s_bar + kRing);              // [R][ceil(T/32)] run-start bits
     const bool run_sums = p.run_table != nullptr && p.run_table[1] == 1;
@@ -88,11 +90,11 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
     auto issue_chunk = [&](int k) {
         const int slot = k % kRing, t0 = (nchunks - 1 - k) * kChunk;
         const uint32_t bytes = (uint32_t)(min(kChunk, T - t0) * H * sizeof(float));
-        tc::mbar_expect_tx(s_bar + slot, bytes * nvalid * (ALIF ? 2 : 1));
+        tc::mbar_expect_tx(s_bar + slot, bytes * nvalid * (TWO ? 2 : 1));
         for (int r = 0; r < nvalid; ++r) {
             const size_t g = ((size_t)(b0 + r) * T + t0) * H;
             tc::bulk_g2s(s_v + ((slot * R + r) * kChunk) * H, p.V + g, bytes, s_bar + slot);
-            if (ALIF) tc::bulk_g2s(s_a + ((slot * R + r) * kChunk) * H, p.a + g, bytes, s_bar + slot);
+            if (TWO) tc::bulk_g2s(s_a + ((slot * R + r) * kChunk) * H, p.a + g, bytes, s_bar + slot);
         }
     };
     if (i == 0) {   // the staging area above aliases the ring: the first copies start only now
@@ -194,7 +196,7 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
                 for (int r = 0; r < R; ++r) {
                     const int o = ((slot * R + r) * kChunk + tt) * H + i;
                     vt[r] = valid[r] ? s_v[o] : 0.f;
-                    at[r] = (valid[r] && ALIF) ? s_a[o] : 0.f;
+                    at[r] = (valid[r] && TWO) ? s_a[o] : 0.f;
                 }
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
@@ -228,7 +230,7 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
                         //   dV'/dV = (1 + dt k ((V-vr) + (V-vth)) / C)(1-Z)   dV'/du = -(dt/C)(1-Z)   dV'/dI = (dt/C)(1-Z)
                         //   du'/dV = dt a b                                    du'/du = 1 - dt a
                         const float v = vt[r];
-                        const float sg = surrogate_grad(SURR, p.gamma, v, p.iz.vpeak);
+                        const float sg = surrogate_grad<SURR>(p.gamma, SURR == kSurrTrace ? at[r] : v, p.iz.vpeak);
                         const float dq = __fmul_rn(p.iz.k, __fadd_rn(__fsub_rn(v, p.iz.vr), __fsub_rn(v, p.iz.vth)));
                         const float A = __fmul_rn(__fadd_rn(1.0f, __fdiv_rn(__fmul_rn(p.iz.dt, dq), p.iz.C)), __fsub_rn(1.0f, zt));
                         const float dtC = __fdiv_rn(p.iz.dt, p.iz.C);
@@ -241,7 +243,7 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_bwd(const BwdParams p)
                     } else {
                         float thr = p.theta;
                         if (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at[r]));
-                        const float sg = surrogate_grad(SURR, p.gamma, vt[r], thr);
+                        const float sg = surrogate_grad<SURR>(p.gamma, vt[r], thr);
                         const float carry = __fmul_rn(__fmul_rn(p.alpha, gv[r]), __fsub_rn(1.0f, zt));
                         g = __fadd_rn(__fmul_rn(s, sg), carry);
                         if (p.g_V && valid[r]) g = __fadd_rn(g, __ldg(p.g_V + o));

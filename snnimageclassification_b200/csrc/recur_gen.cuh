@@ -235,7 +235,8 @@ __global__ void __launch_bounds__(128) k_readout_scan(int T, int H, int O, float
 // ---- backward -------------------------------------------------------------------------------------------------------
 // grid = ceil(B / R), block = H / NPT, dynamic smem = 2*H*R floats + R*T*kOMax floats.
 // Writes gI (one or two tf32 planes) and the scanned readout adjoint gy (B,T,kOMax) for k_wout_grad.
-template <int NPT, int R, bool REC>
+// TRACE: surrogate SNNK_SURROGATE_TRACE -- sigma' is read from the V slot (LIF / ALIF, run as LIF) or from `a` (Izhikevich).
+template <int NPT, int R, bool REC, bool TRACE = false>
 __global__ void __launch_bounds__(kGenMaxThreads) k_recur_bwd_gen(const BwdParams p, float* __restrict__ gy_scan)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -321,7 +322,8 @@ __global__ void __launch_bounds__(kGenMaxThreads) k_recur_bwd_gen(const BwdParam
                 float g, gi;
                 if (p.iz.on) {
                     // the coupled (gV, gu) adjoint of spiking_layers.py:345-348, operation order of k_recur_bwd
-                    const float sg = surrogate_grad(p.surrogate, p.gamma, vt, p.iz.vpeak);
+                    const float sg = TRACE ? (valid[r] ? __ldg(p.a + o) : 0.f)
+                                           : surrogate_grad(p.surrogate, p.gamma, vt, p.iz.vpeak);
                     const float dq = __fmul_rn(p.iz.k, __fadd_rn(__fsub_rn(vt, p.iz.vr), __fsub_rn(vt, p.iz.vth)));
                     const float A = __fmul_rn(__fadd_rn(1.0f, __fdiv_rn(__fmul_rn(p.iz.dt, dq), p.iz.C)), __fsub_rn(1.0f, zt));
                     const float dtC = __fdiv_rn(p.iz.dt, p.iz.C);
@@ -334,7 +336,7 @@ __global__ void __launch_bounds__(kGenMaxThreads) k_recur_bwd_gen(const BwdParam
                 } else {
                     float thr = p.theta;
                     if (p.alif) thr = __fadd_rn(p.theta, __fmul_rn(beta, valid[r] ? __ldg(p.a + o) : 0.f));
-                    const float sg = surrogate_grad(p.surrogate, p.gamma, vt, thr);
+                    const float sg = TRACE ? vt : surrogate_grad(p.surrogate, p.gamma, vt, thr);
                     const float carry = __fmul_rn(__fmul_rn(p.alpha, gv[j][r]), __fsub_rn(1.0f, zt));
                     g = __fadd_rn(__fmul_rn(s, sg), carry);
                     if (p.g_V && valid[r]) g = __fadd_rn(g, __ldg(p.g_V + o));

@@ -499,7 +499,7 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
         s = __fadd_rn(s, dot_rec16_cb<H>(w, PAR ? g0 : g1, i & 3));   // gI_{t+1} (W_rec . M)^T
         float thr = p.theta;
         if (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at));
-        const float sg = surrogate_grad(SURR, p.gamma, vt, thr);
+        const float sg = surrogate_grad<SURR>(p.gamma, vt, thr);
         const float carry = __fmul_rn(__fmul_rn(p.alpha, gv), __fsub_rn(1.0f, zt));
         const float g = __fadd_rn(__fmul_rn(s, sg), carry);
         gv = g;

@@ -242,7 +242,7 @@ __global__ void __launch_bounds__(H) k_nonrec_bwd(const BwdParams p, const float
                 const float zprev = (float)((s_zw[t * W32 + warp] >> lane) & 1u);
                 float thr = p.theta;
                 if constexpr (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at[u]));
-                const float sg = surrogate_grad(SURR, p.gamma, vt[u], thr);
+                const float sg = surrogate_grad<SURR>(p.gamma, vt[u], thr);
                 const float carry = __fmul_rn(__fmul_rn(p.alpha, gv), __fsub_rn(1.0f, zt));
                 float g = __fadd_rn(__fmul_rn(s, sg), carry);
                 if (p.g_V) g = __fadd_rn(g, __ldg(p.g_V + o));

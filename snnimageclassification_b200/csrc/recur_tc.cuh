@@ -573,7 +573,9 @@ __device__ __forceinline__ float rcp_fast(float x)
 template <int SURR>
 __device__ __forceinline__ float surrogate_grad_fast(float gamma, float v, float thr)
 {
-    if constexpr (SURR == 0) {      // spike_funcs.py:59-62
+    if constexpr (SURR == kSurrTrace) {
+        return v;                   // the streamed value is sigma' (common.cuh)
+    } else if constexpr (SURR == 0) {      // spike_funcs.py:59-62
         const float d = fmaf(gamma, fabsf(__fsub_rn(v, thr)), 1.0f);
         return rcp_fast(__fmul_rn(d, d));
     } else {                        // spike_funcs.py:75-79

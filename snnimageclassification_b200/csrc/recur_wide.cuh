@@ -576,7 +576,7 @@ __global__ void __launch_bounds__(kWideThreads, 1) k_wide_bwd(const WideBwdParam
                             if constexpr (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at[mt][nt][e]));
                             const float zcur = (float)((zt[mt][nt][rh] >> (g + 8 * nh)) & 1u);
                             const float zprev = (float)((zp[mt][nt][rh] >> (g + 8 * nh)) & 1u);
-                            const float sgr = surrogate_grad(SURR, p.gamma, vt[mt][nt][e], thr);
+                            const float sgr = surrogate_grad<SURR>(p.gamma, vt[mt][nt][e], thr);
                             const float carry = __fmul_rn(__fmul_rn(p.alpha, gv[mt][nt][e]), __fsub_rn(1.0f, zcur));
                             float gq = __fadd_rn(__fmul_rn(sum, sgr), carry);
                             if (p.g_V && o_) gq = __fadd_rn(gq, __ldg(p.g_V + o));

@@ -127,9 +127,11 @@ template <class F> int by_width(int w, F&& f)   // tile width of the tensor-core
 }
 
 // (layer, surrogate): mode 0 LIF, 1 ALIF, 2 Izhikevich (only the SIMT kernels have an Izhikevich body: the other
-// families are passed mode 0 / 1 and read ALIF as mode == 1).
+// families are passed mode 0 / 1 and read ALIF as mode == 1).  A sigma' trace (SNNK_SURROGATE_TRACE) replaces the only
+// read of the ALIF threshold, so snnk_backward hands it over as mode 0 with sigma' in the V slot.
 template <class F> int by_cell(int mode, int surrogate, F&& f)
 {
+    if (surrogate == SNNK_SURROGATE_TRACE) return mode == 2 ? f(Int<2>{}, Int<kSurrTrace>{}) : f(Int<0>{}, Int<kSurrTrace>{});
     switch (mode * 2 + (surrogate ? 1 : 0)) {
     case 0: return f(Int<0>{}, Int<0>{});
     case 1: return f(Int<0>{}, Int<1>{});
@@ -229,7 +231,8 @@ int check_desc(const SnnkDesc* d)
     if (d->B <= 0 || d->T <= 0 || d->N <= 0 || d->H <= 0 || d->O <= 0) return SNNK_ERR_SHAPE;
     if (d->layer_type != SNNK_LIF && d->layer_type != SNNK_ALIF && d->layer_type != SNNK_IZHIKEVICH) return SNNK_ERR_ARG;
     if (d->layer_type == SNNK_IZHIKEVICH && !(d->iz_C != 0.0f)) return SNNK_ERR_ARG;
-    if (d->surrogate != SNNK_FAST_SIGMOID && d->surrogate != SNNK_PHI) return SNNK_ERR_ARG;
+    if (d->surrogate != SNNK_FAST_SIGMOID && d->surrogate != SNNK_PHI && d->surrogate != SNNK_SURROGATE_TRACE)
+        return SNNK_ERR_ARG;
     if (d->O > kOMax) return SNNK_ERR_SHAPE;
     if (d->H != 32 && d->H != 64 && d->H != 128 && !(d->H % 128 == 0 && d->H <= 2048)) return SNNK_ERR_UNSUPPORTED;
     if ((long long)d->B * d->T >= (1ll << 31) / 4) return SNNK_ERR_SHAPE;
@@ -764,8 +767,10 @@ int launch_bwd_gen(const SnnkDesc* d, const BwdParams& bp, bool rec, const Plan&
         constexpr int NPT = decltype(npt)::value, R = decltype(r)::value;
         const size_t smem = sizeof(float) * (2 * (size_t)d->H * R + (size_t)R * d->T * kOMax);
         if (smem > 200 * 1024) return SNNK_ERR_SHAPE;
-        return launch(SNNK_K_RECUR_BWD, rec ? k_recur_bwd_gen<NPT, R, true> : k_recur_bwd_gen<NPT, R, false>, pl.grid_rows,
-                      d->H / NPT, smem, st, bp, gy_scan);
+        auto kern = bp.surrogate == SNNK_SURROGATE_TRACE
+                        ? (rec ? k_recur_bwd_gen<NPT, R, true, true> : k_recur_bwd_gen<NPT, R, false, true>)
+                        : (rec ? k_recur_bwd_gen<NPT, R, true> : k_recur_bwd_gen<NPT, R, false>);
+        return launch(SNNK_K_RECUR_BWD, kern, pl.grid_rows, d->H / NPT, smem, st, bp, gy_scan);
     };
     return gen_npt(d->H) == 1 ? go(Int<1>{}, Int<4>{}) : go(Int<2>{}, Int<2>{});
 }
@@ -1322,10 +1327,14 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
 {
     int rc = check_desc(d);
     if (rc != SNNK_OK) return rc;
-    if (!x || !W_out || !V || !zbits || !dW_in || !dW_out || !db || !workspace) return SNNK_ERR_ARG;
+    // sigma' trace: it arrives in `a` and is the only trace of V a LIF / ALIF sweep reads (Izhikevich still needs V)
+    const bool trace = d->surrogate == SNNK_SURROGATE_TRACE, izh = d->layer_type == SNNK_IZHIKEVICH;
+    if (!x || !W_out || !zbits || !dW_in || !dW_out || !db || !workspace) return SNNK_ERR_ARG;
+    if ((!trace || izh) && !V) return SNNK_ERR_ARG;
+    if (trace && !a) return SNNK_ERR_ARG;
     if (d->recurrent && (!W_rec || !dW_rec)) return SNNK_ERR_ARG;
     if (d->recurrent && (d->flags & SNNK_F_TENSOR_CORE) && !Z) return SNNK_ERR_ARG;
-    if (d->layer_type == SNNK_ALIF && (!beta || !a)) return SNNK_ERR_ARG;
+    if (!trace && d->layer_type == SNNK_ALIF && (!beta || !a)) return SNNK_ERR_ARG;
     const bool dense = g_y != nullptr, sparse = g_logits != nullptr && tstar != nullptr;
     if (dense == sparse) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
@@ -1371,11 +1380,13 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
     }
     BwdParams bp{};
     bp.B = d->B; bp.T = d->T; bp.H = d->H; bp.O = d->O;
-    bp.alif = d->layer_type == SNNK_ALIF; bp.surrogate = d->surrogate;
+    bp.alif = d->layer_type == SNNK_ALIF && !trace; bp.surrogate = d->surrogate;
     bp.iz = izh_consts(d);
     bp.alpha = d->alpha; bp.theta = d->theta; bp.gamma = d->gamma; bp.kappa = d->kappa;
     bp.W_effT = W_effT; bp.beta = beta; bp.W_out = W_out; bp.Z0 = Z0;
-    bp.V = V; bp.a = a; bp.zbits = zbits; bp.g_y = g_y; bp.g_logits = dense ? nullptr : g_logits;
+    const bool sg_in_v = trace && !izh;     // LIF / ALIF: the LIF-mode sweep reads sigma' in the V slot
+    bp.V = sg_in_v ? a : V; bp.a = sg_in_v ? nullptr : a; bp.zbits = zbits; bp.g_y = g_y;
+    bp.g_logits = dense ? nullptr : g_logits;
     bp.tstar = dense ? nullptr : tstar; bp.g_scale = g_scale; bp.g_V = g_V; bp.g_Z = g_Z;
     float* gI_lo = pl.tc ? reinterpret_cast<float*>(ws + pl.off_gIlo) : nullptr;
     bp.gI = gI; bp.gI_lo = gI_lo; bp.part_wout = pwout; bp.part_db = pdb;

@@ -14,6 +14,7 @@ libsnnk.so.  Nothing in this file has a CPU or eager fallback.
 from __future__ import annotations
 
 import ctypes
+import types
 from dataclasses import dataclass
 from typing import Optional, Tuple
 
@@ -26,7 +27,7 @@ from .. import _cabi
 class LayerConsts:
 	"""Scalar constants of the hidden layer + readout (python floats, rounded to fp32 by the ABI struct)."""
 	layer_type: int      # _cabi.SNNK_LIF | SNNK_ALIF | SNNK_IZHIKEVICH
-	surrogate: int       # _cabi.SNNK_FAST_SIGMOID | SNNK_PHI
+	surrogate: int       # _cabi.SNNK_FAST_SIGMOID | SNNK_PHI | SNNK_SURROGATE_TRACE (spike_funcs.fused_surrogate)
 	recurrent: bool
 	alpha: float
 	rho: float
@@ -35,6 +36,7 @@ class LayerConsts:
 	kappa: float
 	tensor_core: bool = False
 	izh: Optional[Tuple[float, ...]] = None    # Izhikevich only: (dt, C, v_rest, v_th, k, a, b, c, d, v_peak)
+	spike_func: Optional[type] = None          # the SpikeFunction class; its backward gives sigma' for SNNK_SURROGATE_TRACE
 
 
 BINARY_TAG = "_snnk_binary"   # python attribute on tensors known to hold exactly {0,1} (encoder output, spike traces)
@@ -248,8 +250,11 @@ def run_backward(
 		g_V=None, g_Z=None, Z0=None, Z=None, g_scale=None, binary_input: bool = False, runs=None, W_effT=None,
 ):
 	"""Calls ``snnk_backward``.  Returns dict(dW_in, dW_rec, dW_out, db, gI) -- ``gI`` is a zero-argument callable
-	(the tensor-core mode stores it as two planes; summing them is only worth it when somebody asks)."""
+	(the tensor-core mode stores it as two planes; summing them is only worth it when somebody asks).  For a
+	user-defined surrogate the ``a`` argument of the call is sigma' (surrogate_trace) instead of the saved ``a``."""
 	lib = _cabi.lib()
+	if c.surrogate == _cabi.SNNK_SURROGATE_TRACE:
+		a = surrogate_trace(c, V, a, beta)
 	B, T, N = x.shape
 	nbits = bits_width(x)
 	if nbits is not None:
@@ -319,6 +324,26 @@ def run_head_nll(logits: torch.Tensor, labels: torch.Tensor, want_grad: bool = T
 			_cabi.stream_ptr())
 	_cabi.check(rc, "snnk_head_nll")
 	return loss, logp, g
+
+
+def surrogate_trace(c: LayerConsts, V: torch.Tensor, a: Optional[torch.Tensor], beta: Optional[torch.Tensor]):
+	"""sigma'_t = dZ_t/dV_t (B,T,H) of the user-defined surrogate ``c.spike_func`` over the saved traces, for the
+	``a`` argument of ``snnk_backward`` with SNNK_SURROGATE_TRACE: its ``backward`` is called once on a stand-in ctx
+	holding (V, threshold, gamma), as SpikeFunction.forward saves them, with an all-ones gradient.  The threshold is
+	theta (LIF), theta + beta a_t rounded twice as the kernels do (ALIF) or v_peak (Izhikevich, ``c.theta``).  Nothing
+	here waits for the device, so a captured training step records the user's operations too."""
+	dev = V.device
+	thr = _const_scalar(c.theta, dev)
+	if c.layer_type == _cabi.SNNK_ALIF:
+		thr = thr + beta * a
+	ctx = types.SimpleNamespace(saved_tensors=(V, thr, _const_scalar(c.gamma, dev).reshape(1)))
+	out = c.spike_func.backward(ctx, _const_scalar(1.0, dev).expand(V.shape))
+	sg = out[0] if isinstance(out, (tuple, list)) else out
+	if not isinstance(sg, torch.Tensor) or sg.shape != V.shape or sg.dtype != torch.float32 or sg.device != dev:
+		got = f"{tuple(sg.shape)} {sg.dtype} on {sg.device}" if isinstance(sg, torch.Tensor) else type(sg).__name__
+		raise TypeError(f"{c.spike_func.__name__}.backward must return a float32 tensor of the input's shape "
+			f"{tuple(V.shape)} on {dev} as its first element, got {got}")
+	return sg.detach().contiguous()
 
 
 class SpikingSequence(torch.autograd.Function):

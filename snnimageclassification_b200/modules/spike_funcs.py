@@ -3,7 +3,9 @@
 Same names and calling convention (``Func.apply(V, threshold, gamma)``); the arithmetic runs in libsnnk.so
 (``snnk_spike_forward`` / ``snnk_spike_backward``).  Inside ``SNN.forward`` these classes are only *tags*: the
 fused kernels apply the Heaviside step and its surrogate derivative in-register, and the class selects which
-derivative (``SURROGATE_ID``).
+derivative (``SURROGATE_ID``).  A user-defined subclass (``SURROGATE_ID = None``, own ``backward``, the base
+``forward``) trains too: its ``backward`` is evaluated once over the saved membrane trace and the BPTT kernels stream
+the result (see ``SpikeFunction`` and ``fused_surrogate``).
 """
 from __future__ import annotations
 
@@ -27,7 +29,16 @@ def _as_f32_cuda(t: torch.Tensor, like: torch.Tensor) -> torch.Tensor:
 
 
 class SpikeFunction(torch.autograd.Function):
-	"""Heaviside forward ``out = (inputs >= threshold)`` (reference spike_funcs.py:12-29)."""
+	"""Heaviside forward ``out = (inputs >= threshold)`` (reference spike_funcs.py:12-29).
+
+	A user-defined surrogate is a subclass that keeps this ``forward`` and overrides ``backward(ctx, grad)``:
+	it reads ``inputs, threshold, gamma = ctx.saved_tensors`` (what this ``forward`` saves) and returns
+	``(grad * f(inputs, threshold, gamma), None, None)``, with ``f`` elementwise.  Inside ``SNN`` that ``backward``
+	is called once per backward pass with ``grad`` = ones over the whole saved (B, T, H) membrane trace and the
+	per-step threshold (theta for LIF, theta + beta a_t for ALIF, v_peak for Izhikevich); it must not synchronise
+	with the host if the training step is to be captured in a CUDA graph.  The base class itself has no surrogate:
+	inference runs, training raises ``NotImplementedError`` as in the reference.
+	"""
 	SURROGATE_ID = None
 
 	@staticmethod
@@ -81,6 +92,20 @@ class HeavisidePhiApprox(SpikeFunction):
 	@staticmethod
 	def backward(ctx: Any, grad_outputs):
 		return HeavisidePhiApprox._surrogate_backward(ctx, grad_outputs)
+
+
+def fused_surrogate(func) -> int:
+	"""The surrogate kind the fused kernels run for the spike function class ``func`` (SnnkDesc.surrogate): the
+	built-ins' ``SURROGATE_ID``, otherwise ``SNNK_SURROGATE_TRACE`` -- the derivative is ``func.backward``'s, handed
+	to the BPTT sweep as a trace.  The fused forward is the Heaviside step ``V >= threshold``, so a class with its
+	own ``forward`` is refused."""
+	if not (isinstance(func, type) and issubclass(func, SpikeFunction)):
+		raise TypeError(f"spike function {func!r} is not a SpikeFunction subclass")
+	if func.forward is not SpikeFunction.forward:
+		raise NotImplementedError(
+			f"spike function {func.__name__} overrides forward: the fused B200 kernels fire on the Heaviside step "
+			"V >= threshold of SpikeFunction.forward; only backward (the surrogate) may be user-defined")
+	return _cabi.SNNK_SURROGATE_TRACE if func.SURROGATE_ID is None else func.SURROGATE_ID
 
 
 SpikeFuncType2Func = {

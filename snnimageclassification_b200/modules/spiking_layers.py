@@ -17,7 +17,7 @@ from torch import nn
 
 from .. import _cabi
 from . import functional as F_
-from .spike_funcs import HeavisideSigmoidApprox, SpikeFunction
+from .spike_funcs import HeavisideSigmoidApprox, SpikeFunction, fused_surrogate
 
 
 class LayerType(enum.Enum):
@@ -143,15 +143,11 @@ class LIFLayer(RNNLayer):
 
 	# -- constants handed to the C ABI ----------------------------------------------------------------------------
 	def snnk_consts(self, kappa: float = 0.0, tensor_core: bool = False) -> F_.LayerConsts:
-		sid = getattr(self.spike_func, "SURROGATE_ID", None)
-		if sid is None:
-			raise RuntimeError(
-				f"spike function {self.spike_func!r} has no fused surrogate on the B200 path (supported: "
-				"HeavisideSigmoidApprox, HeavisidePhiApprox)")
 		return F_.LayerConsts(
-			layer_type=self.SNNK_LAYER_TYPE, surrogate=sid, recurrent=bool(self.use_recurrent_connection),
-			alpha=float(self.alpha), rho=float(getattr(self, "rho", 0.0)), theta=float(self.threshold),
-			gamma=float(self.gamma), kappa=kappa, tensor_core=tensor_core)
+			layer_type=self.SNNK_LAYER_TYPE, surrogate=fused_surrogate(self.spike_func),
+			recurrent=bool(self.use_recurrent_connection), alpha=float(self.alpha), rho=float(getattr(self, "rho", 0.0)),
+			theta=float(self.threshold), gamma=float(self.gamma), kappa=kappa, tensor_core=tensor_core,
+			spike_func=self.spike_func)
 
 	def _beta_tensor(self) -> Optional[torch.Tensor]:
 		return None
@@ -256,17 +252,12 @@ class IzhikevichLayer(RNNLayer):
 		return V, u, Z
 
 	def snnk_consts(self, kappa: float = 0.0, tensor_core: bool = False) -> F_.LayerConsts:
-		sid = getattr(self.spike_func, "SURROGATE_ID", None)
-		if sid is None:
-			raise RuntimeError(
-				f"spike function {self.spike_func!r} has no fused surrogate on the B200 path (supported: "
-				"HeavisideSigmoidApprox, HeavisidePhiApprox)")
 		izh = tuple(float(v) for v in (self.dt, self.C, self.v_rest, self.v_th, self.k, self.a, self.b, self.c, self.d,
 			self.v_peak))
 		return F_.LayerConsts(
-			layer_type=self.SNNK_LAYER_TYPE, surrogate=sid, recurrent=bool(self.use_recurrent_connection),
-			alpha=0.0, rho=0.0, theta=float(self.v_peak), gamma=float(self.gamma), kappa=kappa, tensor_core=tensor_core,
-			izh=izh)
+			layer_type=self.SNNK_LAYER_TYPE, surrogate=fused_surrogate(self.spike_func),
+			recurrent=bool(self.use_recurrent_connection), alpha=0.0, rho=0.0, theta=float(self.v_peak),
+			gamma=float(self.gamma), kappa=kappa, tensor_core=tensor_core, izh=izh, spike_func=self.spike_func)
 
 	def _beta_tensor(self) -> Optional[torch.Tensor]:
 		return None
