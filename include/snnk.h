@@ -40,7 +40,7 @@
 extern "C" {
 #endif
 
-#define SNNK_ABI_VERSION 8   /* 8: SNNK_F_RUNS_TILED, snnk_run_table_tiled_bytes; 7: snnk_forward_nll; 6: SNNK_F_INPUT_BITS; 5: loss mailbox of snnk_head_nll; 4: W_effT_out / W_effT_in; 2: run_table argument of snnk_forward / snnk_backward, snnk_encode_runs, snnk_adam_step_dp; 3: Izhikevich fields of SnnkDesc */
+#define SNNK_ABI_VERSION 8   /* 8: SNNK_F_RUNS_TILED, snnk_run_table_tiled_bytes, and later the additions snnk_forward_nll_sweep / SNNK_F_SWEEP_DONE, which change no existing call; 7: snnk_forward_nll; 6: SNNK_F_INPUT_BITS; 5: loss mailbox of snnk_head_nll; 4: W_effT_out / W_effT_in; 2: run_table argument of snnk_forward / snnk_backward, snnk_encode_runs, snnk_adam_step_dp; 3: Izhikevich fields of SnnkDesc */
 
 typedef void* snnk_stream_t; /* cudaStream_t */
 
@@ -85,6 +85,10 @@ enum {
 #define SNNK_F_RUNS_TILED 0x10u /* the run table passed to snnk_forward / snnk_forward_nll is followed by the compact rows
                                   tiled for the projection (snnk_run_table_tiled_bytes, snnk_encode_runs with lazy & 2):
                                   the per-step gather of those rows is skipped */
+
+#define SNNK_F_SWEEP_DONE 0x20u /* snnk_backward only: snnk_forward_nll_sweep of the same call already ran the BPTT sweep
+                                  into this workspace; only the weight-gradient contraction and the reductions remain
+                                  (V and a may then be NULL) */
 
 /* Geometry and constants of one hidden spiking layer + leaky readout. */
 typedef struct SnnkDesc {
@@ -258,6 +262,28 @@ int snnk_forward_nll(const SnnkDesc* d, const float* x, const float* W_in, const
                      size_t workspace_bytes, const int32_t* run_table, float* W_effT_out, const int64_t* labels,
                      float* logp, float* loss, float* g_logits, void* head_ws, uint64_t* loss_mailbox,
                      uint32_t* mailbox_counter, snnk_stream_t stream);
+
+/*
+ * snnk_forward_nll followed by the BPTT sweep of snnk_backward, for a training step whose caller already knows the
+ * gradient of the loss it will backpropagate (g_scale, a device scalar read by the kernel: dL/dloss).  Same arguments and
+ * results as snnk_forward_nll, plus: the sweep's outputs (gI, the run sums of the frame-dedup variant, the dW_out / db
+ * partials) are left in bwd_workspace (>= snnk_backward_workspace_bytes), and a later snnk_backward of the same
+ * descriptor with SNNK_F_SWEEP_DONE, the same workspace, x, Z, zbits, tstar, g_logits and run table finishes the
+ * gradients -- with the results snnk_forward_nll + snnk_backward(g_scale) give, bit for bit.
+ * Where the register-resident lean kernels run (recurrent LIF / ALIF, H = 128, the batch below the tensor-core
+ * recurrence's threshold, O <= 12, T <= 128, FastSigmoid or Phi, no SNNK_F_TRACES) one kernel per row runs the
+ * forward, the head and the sweep, and the V / a traces never exist: V and a are not written and may be NULL.  Z
+ * (written: the weight-gradient GEMM reads it), g_logits and W_effT_out (may be NULL) are as for snnk_forward_nll.
+ * Anything else returns SNNK_ERR_UNSUPPORTED before launching any work.
+ */
+int snnk_forward_nll_sweep(const SnnkDesc* d, const float* x, const float* W_in, const float* W_rec,
+                           const float* rec_mask, const float* beta, const float* W_out, const float* b_out,
+                           const float* V0, const float* a0, const float* Z0, float* V, float* a, float* Z,
+                           uint32_t* zbits, float* y, float* logits, int32_t* tstar, void* workspace,
+                           size_t workspace_bytes, const int32_t* run_table, float* W_effT_out, const int64_t* labels,
+                           float* logp, float* loss, float* g_logits, void* head_ws, uint64_t* loss_mailbox,
+                           uint32_t* mailbox_counter, const float* g_scale, void* bwd_workspace,
+                           size_t bwd_workspace_bytes, snnk_stream_t stream);
 
 /*
  * Reverse-time BPTT.  Replaces autograd's sweep for batch_loss.backward() (snn.py:413) over the graph

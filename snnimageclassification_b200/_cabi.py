@@ -23,6 +23,8 @@ SNNK_LIF, SNNK_ALIF, SNNK_IZHIKEVICH = 0, 1, 2
 SNNK_FAST_SIGMOID, SNNK_PHI, SNNK_SURROGATE_TRACE = 0, 1, 2
 SNNK_F32, SNNK_F64, SNNK_U8, SNNK_I64, SNNK_BITS = 0, 1, 2, 3, 4
 SNNK_F_TRACES, SNNK_F_TENSOR_CORE, SNNK_F_INPUT_BINARY, SNNK_F_INPUT_BITS, SNNK_F_RUNS_TILED = 0x1, 0x2, 0x4, 0x8, 0x10
+SNNK_F_SWEEP_DONE = 0x20
+SNNK_ERR_UNSUPPORTED = -6
 SNNK_MAX_CLASSES = 16   # widest readout the kernels take (SnnkDesc.O <= 16, kOMax in csrc/common.cuh)
 
 NVCC_FLAGS = [
@@ -90,6 +92,8 @@ _SIGNATURES = {
 		ctypes.c_double, ctypes.c_double, ctypes.c_int32, _p, ctypes.c_int32, _p, _p, _p, ctypes.c_int32, _p]),
 	"snnk_forward": (ctypes.c_int, [ctypes.POINTER(SnnkDesc)] + [_p] * 18 + [ctypes.c_size_t, _p, _p, _p]),
 	"snnk_forward_nll": (ctypes.c_int, [ctypes.POINTER(SnnkDesc)] + [_p] * 18 + [ctypes.c_size_t, _p, _p] + [_p] * 7 + [_p]),
+	"snnk_forward_nll_sweep": (ctypes.c_int, [ctypes.POINTER(SnnkDesc)] + [_p] * 18 + [ctypes.c_size_t, _p, _p] + [_p] * 7
+		+ [_p, _p, ctypes.c_size_t, _p]),
 	"snnk_head_nll": (ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, _p, _p, _p, _p, _p, _p, _p, _p]),
 	"snnk_input_grad": (ctypes.c_int, [ctypes.POINTER(SnnkDesc), _p, _p, _p, _p]),
 	"snnk_backward": (ctypes.c_int, [ctypes.POINTER(SnnkDesc)] + [_p] * 21 + [ctypes.c_size_t, _p, _p, _p]),

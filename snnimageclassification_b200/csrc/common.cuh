@@ -43,6 +43,7 @@ struct FwdParams {
     // 1: launched as a programmatic dependent of the projection kernel (k_recur_fwd_lean): the kernel may start while the
     // projection still runs and must execute griddepcontrol.wait before it touches I_in / I_u
     int pdl;
+    float gamma;            // surrogate scale: the fused training kernel (k_train_lean) evaluates sigma' in its forward
 };
 
 struct BwdParams {

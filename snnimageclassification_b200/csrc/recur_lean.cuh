@@ -14,6 +14,7 @@
 //   * the double-buffer parity of the spike vector is compile-time (two steps per loop iteration);
 //   * layer type and trace output are template parameters.
 // The recurrent matrix is staged through shared memory in two halves (32 KB) so that two CTAs still fit an SM.
+// k_recur_bwd_lean below is the matching BPTT sweep, and k_train_lean runs forward, head and sweep of a row in one CTA.
 #pragma once
 #include <type_traits>
 
@@ -57,10 +58,12 @@ __device__ __forceinline__ void load_w_cb_half(float (&w)[H], const float* __res
 //     class order as k_head_nll forms it.
 constexpr int kLeanOP = 12;     // row pitch of the readout matrix in shared memory (O <= 12)
 
+// Returns, to thread c < O, the first arg-max step of class c (tstar); -1 to the other threads.
 template <int H>
-__device__ __forceinline__ void fwd_tail_lean(const FwdParams& p, const uint32_t* s_mask, const float* s_wout, float* s_s,
-                                              float* s_logit, int b, int tid)
+__device__ __forceinline__ int fwd_tail_lean(const FwdParams& p, const uint32_t* s_mask, const float* s_wout, float* s_s,
+                                             float* s_logit, int b, int tid)
 {
+    int ts = -1;
     constexpr int W32 = H / 32;
     const int T = p.T, O = p.O;
     for (int idx = tid; idx < T * W32; idx += H) p.zbits[(size_t)b * T * W32 + idx] = s_mask[idx];
@@ -113,19 +116,23 @@ __device__ __forceinline__ void fwd_tail_lean(const FwdParams& p, const uint32_t
         p.logits[(size_t)b * O + c] = mx;
         p.tstar[(size_t)b * O + c] = mt;
         s_logit[c] = mx;
+        ts = mt;
     }
     __syncthreads();
     for (int idx = tid; idx < T * O; idx += H) p.y[(size_t)b * T * O + idx] = s_s[idx];
+    return ts;
 }
 
-__device__ __forceinline__ void head_tail_lean(const FwdParams& p, const float* s_logit, int* s_hd, double* s_hp, int b, int tid,
-                                               int nthr)
+// Returns, to thread c < O, the row's dL/dlogits of class c (when p.g_logits is set); 0 to the other threads.
+__device__ __forceinline__ float head_tail_lean(const FwdParams& p, const float* s_logit, int* s_hd, double* s_hp, int b, int tid,
+                                                int nthr)
 {
     constexpr long long kIgnore = -100;
     const int O = p.O, B = p.B;
     const int n_valid = s_hd[0];
     const bool bad = s_hd[1] != 0;
     const int lane = tid & 31;
+    float g_row = 0.f;
     if (tid < 32) {
         const float lg = lane < O ? s_logit[lane] : -INFINITY;
         float mx = lg;
@@ -144,6 +151,7 @@ __device__ __forceinline__ void head_tail_lean(const FwdParams& p, const float* 
                 float g = row_ok ? __fdiv_rn(expf(lp) - (lane == lab ? 1.0f : 0.0f), (float)n_valid) : 0.0f;
                 if (row_bad) g = __int_as_float(0x7fc00000);
                 p.g_logits[(size_t)b * O + lane] = g;
+                g_row = g;
             }
         }
         const float nll = -__shfl_sync(0xffffffffu, lp, row_ok ? (int)lab : 0);
@@ -154,51 +162,72 @@ __device__ __forceinline__ void head_tail_lean(const FwdParams& p, const float* 
         }
     }
     __syncthreads();
-    if (!s_hd[2]) return;
-    __threadfence();
-    for (int vw = tid >> 5; vw < 8; vw += nthr >> 5) {
-        double acc = 0.0;
-        for (int bb = vw * 32 + lane; bb < B; bb += 256) acc += (double)__ldcg(p.part_nll + bb);
+    if (s_hd[2]) {      // the last CTA to finish: the loss (block-uniform branch)
+        __threadfence();
+        for (int vw = tid >> 5; vw < 8; vw += nthr >> 5) {
+            double acc = 0.0;
+            for (int bb = vw * 32 + lane; bb < B; bb += 256) acc += (double)__ldcg(p.part_nll + bb);
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-        if (lane == 0) s_hp[vw] = acc;
-    }
-    __syncthreads();
-    if (tid == 0) {
-        double sum = 0.0;
-        for (int q = 0; q < 8; ++q) sum += s_hp[q];
-        const float lossf = bad ? __int_as_float(0x7fc00000) : (float)(sum / (double)n_valid);
-        *p.loss = lossf;
-        *p.ticket = 0u;
-        if (p.mailbox) {
-            const unsigned int seq = *p.mail_counter + 1u;
-            *p.mail_counter = seq;
-            *reinterpret_cast<volatile unsigned long long*>(p.mailbox) =
-                (static_cast<unsigned long long>(seq) << 32) | __float_as_uint(lossf);
-            __threadfence_system();
+            for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+            if (lane == 0) s_hp[vw] = acc;
+        }
+        __syncthreads();
+        if (tid == 0) {
+            double sum = 0.0;
+            for (int q = 0; q < 8; ++q) sum += s_hp[q];
+            const float lossf = bad ? __int_as_float(0x7fc00000) : (float)(sum / (double)n_valid);
+            *p.loss = lossf;
+            *p.ticket = 0u;
+            if (p.mailbox) {
+                const unsigned int seq = *p.mail_counter + 1u;
+                *p.mail_counter = seq;
+                *reinterpret_cast<volatile unsigned long long*>(p.mailbox) =
+                    (static_cast<unsigned long long>(seq) << 32) | __float_as_uint(lossf);
+                __threadfence_system();
+            }
         }
     }
+    return g_row;
 }
 
-template <int H, bool ALIF, bool TRACES>
-__global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    constexpr int W32 = H / 32;
-    const int T = p.T, O = p.O;
-    const int i = threadIdx.x, lane = i & 31, warp = i >> 5;
-    const int b = blockIdx.x;                                                       // one row per CTA
+// Dynamic shared memory of the lean forward kernel (lean_fwd_smem_bytes)
+template <int H>
+struct LeanFwdSmem {
+    float* s_z;         // [2][H] spike vector of the previous / current step
+    uint32_t* s_mask;   // [T][W32] spike words of the row
+    float* s_wout;      // [H][12]: rows of W_out padded with zeros
+    float* s_s;         // [T][O] (tail); compact rows of the steps (prologue)
+    float* s_cur;       // [T][H] input current of the row
+    float* s_w;         // [H/2][H] staging of the recurrent matrix
+    uint64_t* s_bar;    // [0] weights, [1] input current
+    __device__ __forceinline__ LeanFwdSmem(unsigned char* raw, int T)
+    {
+        s_z = reinterpret_cast<float*>(raw);
+        s_mask = reinterpret_cast<uint32_t*>(s_z + 2 * H);
+        s_wout = reinterpret_cast<float*>(s_mask + ((T * (H / 32) + 3) & ~3));
+        s_s = s_wout + H * kLeanOP;
+        s_cur = s_wout + ((H * kLeanOP + T * kOMax + 3) & ~3);
+        s_w = s_cur + (size_t)T * H;
+        s_bar = reinterpret_cast<uint64_t*>(s_w + (H / 2) * H);
+    }
+};
 
-    float* s_z = reinterpret_cast<float*>(smem_raw);                                // [2][H]
-    uint32_t* s_mask = reinterpret_cast<uint32_t*>(s_z + 2 * H);                    // [T][W32]
-    float* s_wout = reinterpret_cast<float*>(s_mask + ((T * W32 + 3) & ~3));        // [H][12]: rows of W_out padded with zeros
-    float* s_s = s_wout + H * kLeanOP;                                              // [T][O] (tail); compact rows of the steps (prologue)
-    float* s_cur = s_wout + ((H * kLeanOP + T * kOMax + 3) & ~3);                   // [T][H] input current of the row
-    float* s_w = s_cur + (size_t)T * H;                                             // [H/2][H] staging, prologue only
-    uint64_t* s_bar = reinterpret_cast<uint64_t*>(s_w + (H / 2) * H);               // [0] weights, [1] input current
-    __shared__ int s_hd[4];
-    __shared__ double s_hp[8];
-    __shared__ float s_logit[kOMax];
+// Prologue of the lean forward (one row per CTA): W_eff in registers (column-blocked), the row's input current in s_cur,
+// W_out in s_wout, the initial state, and the head's count of valid rows.  FENCE_W: this thread's reads of the staging
+// area are also ordered before async-proxy writes that the caller issues there after the closing barrier.
+template <int H, bool ALIF, bool FENCE_W>
+__device__ __forceinline__ void lean_fwd_prologue(const FwdParams& p, const LeanFwdSmem<H>& sm, int* s_hd, float (&w)[H],
+                                                  float& beta, float& v, float& a, float& zp)
+{
+    const int T = p.T, O = p.O;
+    const int i = threadIdx.x;
+    const int b = blockIdx.x;
+    float* const s_z = sm.s_z;
+    float* const s_wout = sm.s_wout;
+    float* const s_s = sm.s_s;
+    float* const s_cur = sm.s_cur;
+    float* const s_w = sm.s_w;
+    uint64_t* const s_bar = sm.s_bar;
 
     const bool compact = p.run_table != nullptr && p.run_table[1] == 1;
     constexpr uint32_t kHalfBytes = (uint32_t)((H / 2) * H * sizeof(float));
@@ -242,7 +271,6 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p
     __syncthreads();
     if (p.labels) head_count(p, s_hd, i, H);
 
-    float w[H];
     tc::mbar_wait(s_bar, 0);
     load_w_cb_half<H>(w, s_w, i, 0);
     // The second half is written into the same staging area by the ASYNC proxy, the reads above went through the generic
@@ -254,10 +282,10 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p
         tc::mbar_expect_tx(s_bar, kHalfBytes);
         tc::bulk_g2s(s_w, p.W_eff + (size_t)(H / 2) * H, kHalfBytes, s_bar);
     }
-    const float beta = (ALIF && p.beta) ? __ldg(p.beta) : 0.f;
-    float v = p.V0 ? p.V0[(size_t)b * H + i] : 0.f;
-    float a = p.a0 ? p.a0[(size_t)b * H + i] : 0.f;
-    float zp = p.Z0 ? p.Z0[(size_t)b * H + i] : 0.f;
+    beta = (ALIF && p.beta) ? __ldg(p.beta) : 0.f;
+    v = p.V0 ? p.V0[(size_t)b * H + i] : 0.f;
+    a = p.a0 ? p.a0[(size_t)b * H + i] : 0.f;
+    zp = p.Z0 ? p.Z0[(size_t)b * H + i] : 0.f;
     s_z[H + i] = zp;                               // step 0 reads buffer 1
     for (int idx = i; idx < H * kLeanOP; idx += H) {
         const int j = idx / kLeanOP, c = idx - j * kLeanOP;
@@ -265,6 +293,7 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p
     }
     tc::mbar_wait(s_bar, 1);
     load_w_cb_half<H>(w, s_w, i, 1);
+    if constexpr (FENCE_W) tc::fence_proxy_async_smem();
     if (i == 0 && p.pdl) issue_current();
     tc::mbar_wait(s_bar + 1, 0);
     if (compact) {
@@ -281,53 +310,84 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p
         }
     }
     __syncthreads();
+}
 
-    const float* curp = s_cur + i;
-    uint32_t* maskp = s_mask + warp;
+// What a forward step leaves in memory besides the spike words: nothing, the traces V, Z (and a), or -- for the fused
+// training kernel -- Z and, in the step's own input-current slot, sigma'_t = surrogate'(V_t, threshold_t), the only
+// thing the reverse sweep of a LIF / ALIF layer needs from V and a.
+constexpr int kLeanOutNone = 0, kLeanOutTraces = 1, kLeanOutSweep = 2;
+
+// One step of the lean forward for neuron i = threadIdx.x; BUF = buffer of s_z the step WRITES (it reads the other one).
+template <int H, bool ALIF, int OUT, int SURR, int BUF>
+__device__ __forceinline__ void lean_fwd_step(const FwdParams& p, const float (&w)[H], float* s_z, float*& curp,
+                                              uint32_t*& maskp, size_t& tro, float& v, float& a, float& zp, float beta)
+{
+    constexpr int W32 = H / 32;
+    const int i = threadIdx.x, lane = i & 31;
+    float* const slot = curp;
+    const float cur = *curp;
+    curp += H;
+    const float rec = dot_rec16_cb<H>(w, reinterpret_cast<const float4*>(s_z + (BUF ? 0 : H)), i & 3);
+    // V' = (alpha V + I_in + I_rec) (1 - Z.detach())     spiking_layers.py:169/239
+    const float t1 = __fmul_rn(p.alpha, v);
+    const float t2 = __fadd_rn(t1, cur);
+    const float t3 = __fadd_rn(t2, rec);
+    const float vn = __fmul_rn(t3, __fsub_rn(1.0f, zp));
+    float thr = p.theta;
+    if constexpr (ALIF) {
+        a = __fadd_rn(__fmul_rn(p.rho, a), zp);                    // :240
+        thr = __fadd_rn(p.theta, __fmul_rn(beta, a));              // :241
+    }
+    const float zn = vn >= thr ? 1.0f : 0.0f;                      // spike_funcs.py:27-28
+    s_z[BUF * H + i] = zn;
+    if constexpr (OUT == kLeanOutTraces) {
+        p.V[tro] = vn;
+        p.Z[tro] = zn;
+        if constexpr (ALIF) p.a[tro] = a;
+        tro += H;
+    }
+    if constexpr (OUT == kLeanOutSweep) {
+        *slot = surrogate_grad<SURR>(p.gamma, vn, thr);     // slot t is read by this thread only, and already was
+        p.Z[tro] = zn;
+        tro += H;
+    }
+    const unsigned m = __ballot_sync(0xffffffffu, zn != 0.f);
+    if (lane == 0) *maskp = m;
+    maskp += W32;
+    v = vn;
+    zp = zn;
+    __syncthreads();
+}
+
+template <int H, bool ALIF, bool TRACES>
+__global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p)
+{
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int T = p.T;
+    const int i = threadIdx.x, warp = i >> 5;
+    const int b = blockIdx.x;                                                       // one row per CTA
+    const LeanFwdSmem<H> sm(smem_raw, T);
+    __shared__ int s_hd[4];
+    __shared__ double s_hp[8];
+    __shared__ float s_logit[kOMax];
+
+    float w[H];
+    float beta, v, a, zp;
+    lean_fwd_prologue<H, ALIF, false>(p, sm, s_hd, w, beta, v, a, zp);
+
+    float* curp = sm.s_cur + i;
+    uint32_t* maskp = sm.s_mask + warp;
     size_t tro = (size_t)b * T * H + i;
-    const float4* z0 = reinterpret_cast<const float4*>(s_z);
-    const float4* z1 = reinterpret_cast<const float4*>(s_z + H);
-
-    // one step; BUF = buffer the step WRITES (it reads the other one)
-    auto step = [&](auto buf_tag) {
-        constexpr int BUF = decltype(buf_tag)::value;
-        const float cur = *curp;
-        curp += H;
-        const float rec = dot_rec16_cb<H>(w, BUF ? z0 : z1, i & 3);
-        // V' = (alpha V + I_in + I_rec) (1 - Z.detach())     spiking_layers.py:169/239
-        const float t1 = __fmul_rn(p.alpha, v);
-        const float t2 = __fadd_rn(t1, cur);
-        const float t3 = __fadd_rn(t2, rec);
-        const float vn = __fmul_rn(t3, __fsub_rn(1.0f, zp));
-        float thr = p.theta;
-        if constexpr (ALIF) {
-            a = __fadd_rn(__fmul_rn(p.rho, a), zp);                    // :240
-            thr = __fadd_rn(p.theta, __fmul_rn(beta, a));              // :241
-        }
-        const float zn = vn >= thr ? 1.0f : 0.0f;                      // spike_funcs.py:27-28
-        s_z[BUF * H + i] = zn;
-        if constexpr (TRACES) {
-            p.V[tro] = vn;
-            p.Z[tro] = zn;
-            if constexpr (ALIF) p.a[tro] = a;
-            tro += H;
-        }
-        const unsigned m = __ballot_sync(0xffffffffu, zn != 0.f);
-        if (lane == 0) *maskp = m;
-        maskp += W32;
-        v = vn;
-        zp = zn;
-        __syncthreads();
-    };
+    constexpr int OUT = TRACES ? kLeanOutTraces : kLeanOutNone;
     int t = 0;
     for (; t + 1 < T; t += 2) {
-        step(std::integral_constant<int, 0>{});
-        step(std::integral_constant<int, 1>{});
+        lean_fwd_step<H, ALIF, OUT, 0, 0>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
+        lean_fwd_step<H, ALIF, OUT, 0, 1>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
     }
-    if (t < T) step(std::integral_constant<int, 0>{});
+    if (t < T) lean_fwd_step<H, ALIF, OUT, 0, 0>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
     __syncthreads();
 
-    fwd_tail_lean<H>(p, s_mask, s_wout, s_s, s_logit, b, i);
+    fwd_tail_lean<H>(p, sm.s_mask, sm.s_wout, sm.s_s, s_logit, b, i);
     if (p.labels) head_tail_lean(p, s_logit, s_hd, s_hp, b, i, H);
 }
 
@@ -342,6 +402,113 @@ __global__ void __launch_bounds__(H, 256 / H) k_recur_fwd_lean(const FwdParams p
 // step of the general kernel contain ~70 of uniform-datapath bookkeeping and branches (profiles/r02_*).
 // OP: readout width padded to whole float4 (12 for ten classes): columns >= O of the adjoint rows and of W_out are zero,
 // so leaving them out of the two FMA chains changes nothing but the instruction count.
+// Frame-dedup variant: the run of step t = i and of step i - 1, and the run of the row's last step.
+__device__ __forceinline__ void lean_run_rows(const int* run_table, int T, int b, int i, int& rc_t, int& rc_p, int& crow)
+{
+    const int* rc = run_table + kRunHdrInts + (size_t)b * T;
+    if (i < T) {
+        rc_t = __ldg(rc + i);
+        if (i > 0) rc_p = __ldg(rc + i - 1);
+    }
+    crow = __ldg(rc + T - 1);
+}
+
+// Frame-dedup variant: the row's run-start bits, and (CTA 0) zeros in the tail of the last 32-row block of the run sums
+__device__ __forceinline__ void lean_run_starts(const BwdParams& p, uint32_t* s_start, int rc_t, int rc_p, int i)
+{
+    const int T = p.T, TW = (T + 31) >> 5;
+    if (i < TW) s_start[i] = 0u;
+    __syncthreads();
+    // bit t of the word: step t is the first of its run of equal input frames
+    if (i < T && (i == 0 || rc_t != rc_p)) atomicOr(s_start + (i >> 5), 1u << (i & 31));
+    if (blockIdx.x == 0) {   // the weight-gradient GEMM contracts whole 32-row blocks: zero the tail of the last one
+        const int n_rows = p.run_table[0], n_pad = (n_rows + 31) & ~31;
+        for (int idx = i; idx < (n_pad - n_rows) * 128; idx += 128) {
+            p.Gu_hi[(size_t)n_rows * 128 + idx] = 0.f;
+            p.Gu_lo[(size_t)n_rows * 128 + idx] = 0.f;
+        }
+    }
+}
+
+// readout adjoint scan gy_t = seed_t + kappa gy_{t+1}  (spiking_layers.py:407 backwards) and db: the seed of a class
+// sits at one step (its arg-max over time), so the chain runs in registers -- the same two operations per step as
+// the general kernel's scan over shared memory -- and fills the class's whole column, padding columns with zeros
+__device__ __forceinline__ void lean_gy_scan(const BwdParams& p, float* s_gy, float seed, int ts, int i)
+{
+    const int T = p.T, O = p.O;
+    if (i < kOMax) {
+        float g = 0.f, sum = 0.f;
+        for (int t = T - 1; t >= 0; --t) {
+            g = __fadd_rn(t == ts ? seed : 0.f, __fmul_rn(p.kappa, g));
+            s_gy[t * kOMax + i] = g;
+            sum += g;
+        }
+        if (i < O) p.part_db[(size_t)blockIdx.x * O + i] = sum;
+    }
+}
+
+// One reverse step t of the lean sweep for neuron i = threadIdx.x.  PAR = t & 1 (the buffer gI_t is written to; gI_{t+1}
+// is read from the other one); sigma() yields sigma'_t.
+template <int OP, bool PLANES, bool RUNS, int PAR, class Sigma>
+__device__ __forceinline__ void lean_bwd_step(const BwdParams& p, int t, const float (&w)[128], const float (&wo)[OP],
+                                              float (&dwo)[OP], float* s_g, const uint32_t* s_start, bool run_sums,
+                                              const float4*& gyp, const uint32_t*& mkp, uint32_t& mword, float& gv,
+                                              float& racc, uint32_t& sbits, int& crow, size_t& tro, Sigma&& sigma)
+{
+    constexpr int H = 128, W32 = H / 32;
+    const int i = threadIdx.x, lane = i & 31;
+    const int b = blockIdx.x;
+    float gy[OP];
+#pragma unroll
+    for (int q = 0; q < OP / 4; ++q) {
+        const float4 g4 = gyp[q];
+        gy[4 * q + 0] = g4.x; gy[4 * q + 1] = g4.y; gy[4 * q + 2] = g4.z; gy[4 * q + 3] = g4.w;
+    }
+    gyp -= kOMax / 4;
+    const float zt = (float)((mword >> lane) & 1u);
+    float zprev;
+    if (t > 0) {
+        mkp -= W32;
+        mword = *mkp;
+        zprev = (float)((mword >> lane) & 1u);
+    } else {
+        zprev = p.Z0 ? __ldg(p.Z0 + (size_t)b * H + i) : 0.f;
+    }
+    float s = 0.f;
+#pragma unroll
+    for (int c = 0; c < OP; ++c) {
+        s = fmaf(gy[c], wo[c], s);               // gy_t W_out^T
+        dwo[c] = fmaf(zt, gy[c], dwo[c]);        // dW_out += Z_t^T gy_t
+    }
+    s = __fadd_rn(s, dot_rec16_cb<H>(w, reinterpret_cast<const float4*>(s_g + (PAR ? 0 : H)), i & 3));   // gI_{t+1} (W_rec . M)^T
+    const float sg = sigma();
+    const float carry = __fmul_rn(__fmul_rn(p.alpha, gv), __fsub_rn(1.0f, zt));
+    const float g = __fadd_rn(__fmul_rn(s, sg), carry);
+    gv = g;
+    const float gi = __fmul_rn(g, __fsub_rn(1.0f, zprev));
+    if (PLANES) {   // tensor-core mode: exact two-plane tf32 split for the weight-gradient GEMM
+        const float hi = __uint_as_float(__float_as_uint(gi) & 0xFFFFE000u);
+        p.gI[tro] = hi;
+        p.gI_lo[tro] = __fsub_rn(gi, hi);
+    } else {
+        p.gI[tro] = gi;
+    }
+    tro -= H;
+    s_g[PAR * H + i] = gi;
+    if (RUNS && run_sums) {   // sum of gI over the run of equal input frames this step belongs to
+        racc = __fadd_rn(racc, gi);
+        if (t == p.T - 1 || (t & 31) == 31) sbits = s_start[t >> 5];
+        if ((sbits >> (t & 31)) & 1u) {
+            const float hi = __uint_as_float(__float_as_uint(racc) & 0xFFFFE000u);
+            p.Gu_hi[(size_t)crow * H + i] = hi;
+            p.Gu_lo[(size_t)crow * H + i] = __fsub_rn(racc, hi);
+            racc = 0.f;
+            --crow;
+        }
+    }
+    __syncthreads();
+}
+
 template <bool ALIF, int SURR, bool PLANES, bool RUNS, int OP>
 __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
 {
@@ -350,14 +517,13 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
     static_assert(kChunk % 2 == 0, "compile-time parity of the gI double buffer");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int T = p.T, O = p.O;
-    const int i = threadIdx.x, lane = i & 31, warp = i >> 5;
+    const int i = threadIdx.x, warp = i >> 5;
     const int b = blockIdx.x;
 
     // Everything the prologue needs from global memory is requested FIRST, into registers: the weight staging below
     // (64 KB through shared memory, which the loop buffers alias) then overlaps those round trips instead of
     // preceding six of them one after the other (ncu: 15 % of the general kernel was prologue).
     const bool run_sums = RUNS && p.run_table != nullptr && p.run_table[1] == 1;
-    const int TW = (T + 31) >> 5;
     uint32_t zw[4];                                        // spike words i, i+H, ... of the row (T * W32 <= 4 H)
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
@@ -365,14 +531,7 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
         zw[q] = idx < T * W32 ? __ldg(p.zbits + (size_t)b * T * W32 + idx) : 0u;
     }
     int rc_t = 0, rc_p = -1, crow = 0;                     // run of step t = i and of step i-1; run of the last step
-    if (run_sums) {
-        const int* rc = p.run_table + kRunHdrInts + (size_t)b * T;
-        if (i < T) {
-            rc_t = __ldg(rc + i);
-            if (i > 0) rc_p = __ldg(rc + i - 1);
-        }
-        crow = __ldg(rc + T - 1);
-    }
+    if (run_sums) lean_run_rows(p.run_table, T, b, i, rc_t, rc_p, crow);
     float seed = 0.f;                                      // thread c < O: the seed of class c at its arg-max step
     int ts = -1;
     if (i < O) {
@@ -433,31 +592,8 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
 #pragma unroll
     for (int q = 0; q < 4; ++q)
         if (i + q * H < T * W32) s_mask[i + q * H] = zw[q];
-    if (run_sums) {
-        if (i < TW) s_start[i] = 0u;
-        __syncthreads();
-        // bit t of the word: step t is the first of its run of equal input frames
-        if (i < T && (i == 0 || rc_t != rc_p)) atomicOr(s_start + (i >> 5), 1u << (i & 31));
-        if (blockIdx.x == 0) {   // the weight-gradient GEMM contracts whole 32-row blocks: zero the tail of the last one
-            const int n_rows = p.run_table[0], n_pad = (n_rows + 31) & ~31;
-            for (int idx = i; idx < (n_pad - n_rows) * H; idx += H) {
-                p.Gu_hi[(size_t)n_rows * H + idx] = 0.f;
-                p.Gu_lo[(size_t)n_rows * H + idx] = 0.f;
-            }
-        }
-    }
-    // readout adjoint scan gy_t = seed_t + kappa gy_{t+1}  (spiking_layers.py:407 backwards) and db: the seed of a class
-    // sits at one step (its arg-max over time), so the chain runs in registers -- the same two operations per step as
-    // the general kernel's scan over shared memory -- and fills the class's whole column, padding columns with zeros
-    if (i < kOMax) {
-        float g = 0.f, sum = 0.f;
-        for (int t = T - 1; t >= 0; --t) {
-            g = __fadd_rn(t == ts ? seed : 0.f, __fmul_rn(p.kappa, g));
-            s_gy[t * kOMax + i] = g;
-            sum += g;
-        }
-        if (i < O) p.part_db[(size_t)blockIdx.x * O + i] = sum;
-    }
+    if (run_sums) lean_run_starts(p, s_start, rc_t, rc_p, i);
+    lean_gy_scan(p, s_gy, seed, ts, i);
     __syncthreads();
 
     float gv = 0.f, racc = 0.f;
@@ -466,65 +602,17 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
     const float4* gyp = reinterpret_cast<const float4*>(s_gy + (T - 1) * kOMax);
     const uint32_t* mkp = s_mask + (T - 1) * W32 + warp;
     uint32_t mword = *mkp;                                 // spike word of step t (carried: it is step t+1's "previous")
-    const float4* g0 = reinterpret_cast<const float4*>(s_g);
-    const float4* g1 = reinterpret_cast<const float4*>(s_g + H);
-
     // one step.  PAR = t & 1 (the buffer gI_t is written to; gI_{t+1} is read from the other one)
     auto step = [&](int t, const float* vrow, const float* arow, auto par_tag) {
         constexpr int PAR = decltype(par_tag)::value;
         const float vt = vrow[i];
         const float at = ALIF ? arow[i] : 0.f;
-        float gy[OP];
-#pragma unroll
-        for (int q = 0; q < OP / 4; ++q) {
-            const float4 g4 = gyp[q];
-            gy[4 * q + 0] = g4.x; gy[4 * q + 1] = g4.y; gy[4 * q + 2] = g4.z; gy[4 * q + 3] = g4.w;
-        }
-        gyp -= kOMax / 4;
-        const float zt = (float)((mword >> lane) & 1u);
-        float zprev;
-        if (t > 0) {
-            mkp -= W32;
-            mword = *mkp;
-            zprev = (float)((mword >> lane) & 1u);
-        } else {
-            zprev = p.Z0 ? __ldg(p.Z0 + (size_t)b * H + i) : 0.f;
-        }
-        float s = 0.f;
-#pragma unroll
-        for (int c = 0; c < OP; ++c) {
-            s = fmaf(gy[c], wo[c], s);               // gy_t W_out^T
-            dwo[c] = fmaf(zt, gy[c], dwo[c]);        // dW_out += Z_t^T gy_t
-        }
-        s = __fadd_rn(s, dot_rec16_cb<H>(w, PAR ? g0 : g1, i & 3));   // gI_{t+1} (W_rec . M)^T
-        float thr = p.theta;
-        if (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at));
-        const float sg = surrogate_grad<SURR>(p.gamma, vt, thr);
-        const float carry = __fmul_rn(__fmul_rn(p.alpha, gv), __fsub_rn(1.0f, zt));
-        const float g = __fadd_rn(__fmul_rn(s, sg), carry);
-        gv = g;
-        const float gi = __fmul_rn(g, __fsub_rn(1.0f, zprev));
-        if (PLANES) {   // tensor-core mode: exact two-plane tf32 split for the weight-gradient GEMM
-            const float hi = __uint_as_float(__float_as_uint(gi) & 0xFFFFE000u);
-            p.gI[tro] = hi;
-            p.gI_lo[tro] = __fsub_rn(gi, hi);
-        } else {
-            p.gI[tro] = gi;
-        }
-        tro -= H;
-        s_g[PAR * H + i] = gi;
-        if (RUNS && run_sums) {   // sum of gI over the run of equal input frames this step belongs to
-            racc = __fadd_rn(racc, gi);
-            if (t == T - 1 || (t & 31) == 31) sbits = s_start[t >> 5];
-            if ((sbits >> (t & 31)) & 1u) {
-                const float hi = __uint_as_float(__float_as_uint(racc) & 0xFFFFE000u);
-                p.Gu_hi[(size_t)crow * H + i] = hi;
-                p.Gu_lo[(size_t)crow * H + i] = __fsub_rn(racc, hi);
-                racc = 0.f;
-                --crow;
-            }
-        }
-        __syncthreads();
+        lean_bwd_step<OP, PLANES, RUNS, PAR>(p, t, w, wo, dwo, s_g, s_start, run_sums, gyp, mkp, mword, gv, racc, sbits,
+                                             crow, tro, [&] {
+                                                 float thr = p.theta;
+                                                 if (ALIF) thr = __fadd_rn(p.theta, __fmul_rn(beta, at));
+                                                 return surrogate_grad<SURR>(p.gamma, vt, thr);
+                                             });
     };
 
     for (int k = 0; k < nchunks; ++k) {
@@ -550,6 +638,108 @@ __global__ void __launch_bounds__(128, 2) k_recur_bwd_lean(const BwdParams p)
 #pragma unroll
     for (int c = 0; c < OP; ++c)
         if (c < O) p.part_wout[((size_t)blockIdx.x * H + i) * O + c] = dwo[c];
+}
+
+// ---- forward, head and BPTT sweep of a row in one CTA ----------------------------------------------------------------
+// k_recur_fwd_lean with its head, then k_recur_bwd_lean<.., kLeanOP> in LIF mode, in the CTA that owns the row: the
+// row's dL/dlogits depends on that row alone (every CTA counts n_valid in its prologue), so no CTA waits for another
+// and the sweep needs no second launch.  Same arithmetic in the same order as the two kernels (bit-identical results):
+//   * the forward overwrites step t's slot of the row's input current, which it reads once at step t, with sigma'_t of
+//     the V_t and threshold it just computed, and stores Z (the weight-gradient GEMM reads it) but neither V nor a: the
+//     reverse loop reads sigma'_t from shared memory where k_recur_bwd_lean streams V and a back through its ring;
+//   * the spike words, W_out, tstar and the seeds stay on chip;
+//   * W_effT goes through the forward's weight staging area in two halves: the first while the forward loop runs,
+//     the second behind the tail.
+// Shared memory is the forward kernel's (lean_fwd_smem_bytes): s_g aliases s_z and s_gy the tail's s_s.
+template <bool ALIF, int SURR, bool PLANES, bool RUNS>
+__global__ void __launch_bounds__(128, 2) k_train_lean(const FwdParams p, const BwdParams q)
+{
+    constexpr int H = 128, W32 = H / 32, OP = kLeanOP;
+    constexpr uint32_t kHalfBytes = (uint32_t)((H / 2) * H * sizeof(float));
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int T = p.T, O = p.O;
+    const int i = threadIdx.x, warp = i >> 5;
+    const int b = blockIdx.x;
+    const LeanFwdSmem<H> sm(smem_raw, T);
+    __shared__ int s_hd[4];
+    __shared__ double s_hp[8];
+    __shared__ float s_logit[kOMax];
+    __shared__ uint32_t s_start[4];                        // run-start bits of the row (T <= 128)
+
+    const bool run_sums = RUNS && q.run_table != nullptr && q.run_table[1] == 1;
+    int rc_t = 0, rc_p = -1, crow = 0;                     // run of step t = i and of step i-1; run of the last step
+    if (run_sums) lean_run_rows(q.run_table, T, b, i, rc_t, rc_p, crow);
+    const float scale = __ldg(q.g_scale);
+
+    float w[H];
+    float beta, v, a, zp;
+    lean_fwd_prologue<H, ALIF, true>(p, sm, s_hd, w, beta, v, a, zp);
+    if (i == 0) {
+        tc::mbar_expect_tx(sm.s_bar, kHalfBytes);
+        tc::bulk_g2s(sm.s_w, q.W_effT, kHalfBytes, sm.s_bar);
+    }
+
+    float* curp = sm.s_cur + i;
+    uint32_t* maskp = sm.s_mask + warp;
+    size_t tro = (size_t)b * T * H + i;
+    int t = 0;
+    for (; t + 1 < T; t += 2) {
+        lean_fwd_step<H, ALIF, kLeanOutSweep, SURR, 0>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
+        lean_fwd_step<H, ALIF, kLeanOutSweep, SURR, 1>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
+    }
+    if (t < T) lean_fwd_step<H, ALIF, kLeanOutSweep, SURR, 0>(p, w, sm.s_z, curp, maskp, tro, v, a, zp, beta);
+    __syncthreads();
+
+    // the forward's weights are dead: first half of W_effT into registers, the second half's copy overlaps the tail
+    tc::mbar_wait(sm.s_bar, 0);
+    load_w_cb_half<H>(w, sm.s_w, i, 0);
+    tc::fence_proxy_async_smem();
+    __syncthreads();
+    if (i == 0) {
+        tc::mbar_expect_tx(sm.s_bar, kHalfBytes);
+        tc::bulk_g2s(sm.s_w, q.W_effT + (size_t)(H / 2) * H, kHalfBytes, sm.s_bar);
+    }
+    const int ts = fwd_tail_lean<H>(p, sm.s_mask, sm.s_wout, sm.s_s, s_logit, b, i);
+    const float g_row = head_tail_lean(p, s_logit, s_hd, s_hp, b, i, H);
+    const float seed = i < O ? __fmul_rn(g_row, scale) : 0.f;     // thread c < O: the seed of class c at step ts
+
+    float wo[OP], dwo[OP];
+#pragma unroll
+    for (int c = 0; c < OP; ++c) {
+        wo[c] = sm.s_wout[i * kLeanOP + c];               // zero for c >= O
+        dwo[c] = 0.f;
+    }
+    float* s_g = sm.s_z;                                   // [2][H]
+    float* s_gy = sm.s_s;                                  // [T][kOMax]
+    for (int idx = i; idx < 2 * H; idx += H) s_g[idx] = 0.f;
+    if (run_sums) lean_run_starts(q, s_start, rc_t, rc_p, i);
+    lean_gy_scan(q, s_gy, seed, ts, i);
+    tc::mbar_wait(sm.s_bar, 1);
+    load_w_cb_half<H>(w, sm.s_w, i, 1);
+    __syncthreads();
+
+    float gv = 0.f, racc = 0.f;
+    uint32_t sbits = 0u;
+    size_t gro = ((size_t)b * T + (T - 1)) * H + i;
+    const float4* gyp = reinterpret_cast<const float4*>(s_gy + (T - 1) * kOMax);
+    const uint32_t* mkp = sm.s_mask + (T - 1) * W32 + warp;
+    uint32_t mword = *mkp;                                 // spike word of step t (carried: it is step t+1's "previous")
+    const float* sgp = sm.s_cur + (size_t)(T - 1) * H + i;
+    auto step = [&](int tt, auto par_tag) {
+        constexpr int PAR = decltype(par_tag)::value;
+        lean_bwd_step<OP, PLANES, RUNS, PAR>(q, tt, w, wo, dwo, s_g, s_start, run_sums, gyp, mkp, mword, gv, racc, sbits,
+                                             crow, gro, [&] { return *sgp; });
+        sgp -= H;
+    };
+    t = T - 1;
+    if (!(t & 1)) step(t--, std::integral_constant<int, 0>{});
+    for (; t > 0; t -= 2) {
+        step(t, std::integral_constant<int, 1>{});
+        step(t - 1, std::integral_constant<int, 0>{});
+    }
+#pragma unroll
+    for (int c = 0; c < OP; ++c)
+        if (c < O) q.part_wout[((size_t)b * H + i) * O + c] = dwo[c];
 }
 
 }  // namespace snnk

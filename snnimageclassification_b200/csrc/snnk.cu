@@ -537,29 +537,59 @@ int launch_fwd_simt(const FwdParams& fp, bool rec, const Plan& pl, cudaStream_t 
 // Lean forward recurrence (recur_lean.cuh; Plan::lean_fwd).  pdl: launch as a programmatic dependent of the kernel
 // queued before it on the stream (the projection GEMM, which executes griddepcontrol.launch_dependents at its start):
 // the recurrence kernel's prologue then overlaps the projection.
-int launch_fwd_lean(FwdParams fp, cudaStream_t st, bool pdl)
+template <class... P>
+int launch_lean(void (*kern)(P...), size_t smem, cudaStream_t st, bool pdl, int B, const P&... args)
 {
-    const size_t smem = lean_fwd_smem_bytes<128>(fp.T, fp.O);
-    void (*kern)(const FwdParams) = fp.alif ? (fp.traces ? k_recur_fwd_lean<128, true, true> : k_recur_fwd_lean<128, true, false>)
-                                            : (fp.traces ? k_recur_fwd_lean<128, false, true> : k_recur_fwd_lean<128, false, false>);
     SNNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    fp.pdl = pdl ? 1 : 0;
     {
         ProfScope ps(SNNK_K_RECUR_FWD, st);
         if (pdl) {
             cudaLaunchConfig_t cfg{};
-            cfg.gridDim = dim3(fp.B); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+            cfg.gridDim = dim3(B); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = smem; cfg.stream = st;
             cudaLaunchAttribute attr[1];
             attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             attr[0].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = attr; cfg.numAttrs = 1;
-            SNNK_CUDA(cudaLaunchKernelEx(&cfg, kern, (const FwdParams)fp));
+            SNNK_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
         } else {
-            kern<<<fp.B, 128, smem, st>>>(fp);
+            kern<<<B, 128, smem, st>>>(args...);
         }
     }
     SNNK_CUDA(cudaGetLastError());
     return SNNK_OK;
+}
+
+int launch_fwd_lean(FwdParams fp, cudaStream_t st, bool pdl)
+{
+    void (*kern)(const FwdParams) = fp.alif ? (fp.traces ? k_recur_fwd_lean<128, true, true> : k_recur_fwd_lean<128, true, false>)
+                                            : (fp.traces ? k_recur_fwd_lean<128, false, true> : k_recur_fwd_lean<128, false, false>);
+    fp.pdl = pdl ? 1 : 0;
+    return launch_lean(kern, lean_fwd_smem_bytes<128>(fp.T, fp.O), st, pdl, fp.B, (const FwdParams)fp);
+}
+
+// Fused training kernel (recur_lean.cuh, k_train_lean): where both lean kernels run, with a built-in surrogate.  The
+// readout (O <= kLeanOP) and T (<= 128: the sweep's spike words) limits are those of the two lean kernels.
+bool sweep_eligible(const SnnkDesc* d, const Plan& pl)
+{
+    return pl.lean_fwd && d->surrogate != SNNK_SURROGATE_TRACE && d->T <= 128 &&
+           bwd_smem_bytes<128, 1>(d->T, true) <= 110 * 1024;
+}
+
+template <bool A, int S>
+void (*train_lean_kernel(bool planes, bool runs))(const FwdParams, const BwdParams)
+{
+    return planes ? (runs ? k_train_lean<A, S, true, true> : k_train_lean<A, S, true, false>)
+                  : (runs ? k_train_lean<A, S, false, true> : k_train_lean<A, S, false, false>);
+}
+
+int launch_train_lean(FwdParams fp, const BwdParams& bp, cudaStream_t st, bool pdl)
+{
+    const bool planes = bp.gI_lo != nullptr, runs = bp.run_table != nullptr, phi = bp.surrogate == SNNK_PHI;
+    void (*kern)(const FwdParams, const BwdParams) =
+        fp.alif ? (phi ? train_lean_kernel<true, 1>(planes, runs) : train_lean_kernel<true, 0>(planes, runs))
+                : (phi ? train_lean_kernel<false, 1>(planes, runs) : train_lean_kernel<false, 0>(planes, runs));
+    fp.pdl = pdl ? 1 : 0;
+    return launch_lean(kern, lean_fwd_smem_bytes<128>(fp.T, fp.O), st, pdl, fp.B, (const FwdParams)fp, bp);
 }
 
 // Lean BPTT sweep (recur_lean.cuh): the training step of the headline geometry -- recurrent LIF / ALIF, H = 128, one row
@@ -1061,11 +1091,36 @@ struct HeadArgs {
     const int64_t* labels; float* logp; float* loss; float* g_logits; void* head_ws; uint64_t* mailbox; uint32_t* counter;
 };
 
+// Sweep arguments of snnk_forward_nll_sweep (null otherwise): the seed scale and the backward workspace
+struct SweepArgs {
+    const float* g_scale; void* workspace; size_t workspace_bytes;
+};
+
+// Constants of the BPTT sweep and its outputs in the backward workspace: gI (planes), dW_out / db partials, run sums
+BwdParams sweep_params(const SnnkDesc* d, const Plan& pl, char* ws, const int* runs)
+{
+    BwdParams bp{};
+    bp.B = d->B; bp.T = d->T; bp.H = d->H; bp.O = d->O;
+    bp.alif = d->layer_type == SNNK_ALIF && d->surrogate != SNNK_SURROGATE_TRACE; bp.surrogate = d->surrogate;
+    bp.iz = izh_consts(d);
+    bp.alpha = d->alpha; bp.theta = d->theta; bp.gamma = d->gamma; bp.kappa = d->kappa;
+    bp.gI = reinterpret_cast<float*>(ws + pl.off_gI);
+    bp.gI_lo = pl.tc ? reinterpret_cast<float*>(ws + pl.off_gIlo) : nullptr;
+    bp.part_wout = reinterpret_cast<float*>(ws + pl.off_pwout);
+    bp.part_db = reinterpret_cast<float*>(ws + pl.off_pdb);
+    if (runs) {
+        bp.run_table = runs;
+        bp.Gu_hi = reinterpret_cast<float*>(ws + pl.off_gu);
+        bp.Gu_lo = reinterpret_cast<float*>(ws + pl.off_gu + pl.gu_plane);
+    }
+    return bp;
+}
+
 static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, const float* W_rec, const float* rec_mask,
                  const float* beta, const float* W_out, const float* b_out, const float* V0, const float* a0,
                  const float* Z0, float* V, float* a, float* Z, uint32_t* zbits, float* y, float* logits,
                  int32_t* tstar, void* workspace, size_t workspace_bytes, const int32_t* run_table, float* W_effT_out,
-                 snnk_stream_t stream, const HeadArgs* head)
+                 snnk_stream_t stream, const HeadArgs* head, const SweepArgs* sweep = nullptr)
 {
     int rc = check_desc(d);
     if (rc != SNNK_OK) return rc;
@@ -1076,9 +1131,12 @@ static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, co
     if (traces && (!V || !Z || (d->layer_type != SNNK_LIF && !a))) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
     const Plan pl = make_plan(d);
+    if (sweep && (!head || traces || !sweep_eligible(d, pl))) return SNNK_ERR_UNSUPPORTED;
     if (workspace_bytes < pl.fwd_bytes) return SNNK_ERR_WORKSPACE;
+    if (sweep && sweep->workspace_bytes < pl.bwd_bytes) return SNNK_ERR_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     char* ws = static_cast<char*>(workspace);
+    char* ws_b = sweep ? static_cast<char*>(sweep->workspace) : nullptr;
     float* I_in = static_cast<float*>(workspace);
     // frame-dedup variant (runs.cuh): only for inputs the caller vouches to be the encoder's {0,1} raster
     const int* runs = pl.dedup ? run_table : nullptr;
@@ -1147,21 +1205,30 @@ static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, co
     }
     // K2: fused recurrence + readout
     float* W_eff = nullptr;
+    // the fused training kernel reads the transposed matrix too: the caller's W_effT_out, else the backward workspace's
+    float* W_effT = W_effT_out ? W_effT_out : (sweep ? reinterpret_cast<float*>(ws_b + pl.off_weffT) : nullptr);
     if (d->recurrent) {
         W_eff = reinterpret_cast<float*>(ws + pl.off_weff);
         const int n = d->H * d->H;
-        k_prep_rec<<<(n + 255) / 256, 256, 0, side>>>(W_rec, rec_mask, d->H, W_eff, W_effT_out);
+        k_prep_rec<<<(n + 255) / 256, 256, 0, side>>>(W_rec, rec_mask, d->H, W_eff, W_effT);
         SNNK_CUDA(cudaGetLastError());
     }
     if (fk) {
         SNNK_CUDA(cudaEventRecord(fk->joined, side));
         SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined, 0));
     }
+    // dedup variant of the fused training kernel: the compact rows of x for the dW_in GEMM, gathered beside it
+    if (sweep && runs) {
+        k_gather_rows<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, side>>>(
+            x, runs, d->B * d->T, d->N, reinterpret_cast<float*>(ws_b + pl.off_xu_b));
+        SNNK_CUDA(cudaGetLastError());
+        SNNK_CUDA(cudaEventRecord(fk->joined3, side));
+    }
     FwdParams fp{};
     fp.B = d->B; fp.T = d->T; fp.H = d->H; fp.O = d->O;
     fp.alif = d->layer_type == SNNK_ALIF; fp.traces = traces;
     fp.iz = izh_consts(d);
-    fp.alpha = d->alpha; fp.rho = d->rho; fp.theta = d->theta; fp.kappa = d->kappa;
+    fp.alpha = d->alpha; fp.rho = d->rho; fp.theta = d->theta; fp.kappa = d->kappa; fp.gamma = d->gamma;
     fp.I_in = I_in; fp.W_eff = W_eff; fp.beta = beta; fp.W_out = W_out; fp.b_out = b_out;
     fp.V0 = V0; fp.a0 = a0; fp.Z0 = Z0; fp.V = V; fp.a = a; fp.Z = Z; fp.zbits = zbits; fp.y = y;
     fp.logits = logits; fp.tstar = tstar;
@@ -1190,7 +1257,15 @@ static int forward_impl(const SnnkDesc* d, const float* x, const float* W_in, co
     case Family::Simt:
         // the lean kernel is a programmatic dependent of a tensor-core projection on the same stream (not while the
         // per-kernel profiler brackets launches with events)
-        rc = pl.lean_fwd ? launch_fwd_lean(fp, st, pl.tc && !g_prof_on) : launch_fwd_simt(fp, rec, pl, st);
+        if (sweep) {
+            BwdParams bp = sweep_params(d, pl, ws_b, runs);
+            bp.W_effT = W_effT; bp.beta = beta; bp.W_out = W_out; bp.Z0 = Z0; bp.zbits = zbits;
+            bp.g_logits = head->g_logits; bp.tstar = tstar; bp.g_scale = sweep->g_scale;
+            rc = launch_train_lean(fp, bp, st, pl.tc && !g_prof_on);
+            if (rc == SNNK_OK && runs) SNNK_CUDA(cudaStreamWaitEvent(st, fk->joined3, 0));
+        } else {
+            rc = pl.lean_fwd ? launch_fwd_lean(fp, st, pl.tc && !g_prof_on) : launch_fwd_simt(fp, rec, pl, st);
+        }
         break;
     }
     if (rc != SNNK_OK || !head || fused_head) return rc;
@@ -1220,6 +1295,22 @@ int snnk_forward_nll(const SnnkDesc* d, const float* x, const float* W_in, const
     const HeadArgs h{labels, logp, loss, g_logits, head_ws, loss_mailbox, mailbox_counter};
     return forward_impl(d, x, W_in, W_rec, rec_mask, beta, W_out, b_out, V0, a0, Z0, V, a, Z, zbits, y, logits, tstar,
                         workspace, workspace_bytes, run_table, W_effT_out, stream, &h);
+}
+
+int snnk_forward_nll_sweep(const SnnkDesc* d, const float* x, const float* W_in, const float* W_rec, const float* rec_mask,
+                           const float* beta, const float* W_out, const float* b_out, const float* V0, const float* a0,
+                           const float* Z0, float* V, float* a, float* Z, uint32_t* zbits, float* y, float* logits,
+                           int32_t* tstar, void* workspace, size_t workspace_bytes, const int32_t* run_table,
+                           float* W_effT_out, const int64_t* labels, float* logp, float* loss, float* g_logits,
+                           void* head_ws, uint64_t* loss_mailbox, uint32_t* mailbox_counter, const float* g_scale,
+                           void* bwd_workspace, size_t bwd_workspace_bytes, snnk_stream_t stream)
+{
+    if (!labels || !loss || !head_ws || !g_logits || !Z || !g_scale || !bwd_workspace) return SNNK_ERR_ARG;
+    if ((loss_mailbox != nullptr) != (mailbox_counter != nullptr)) return SNNK_ERR_ARG;
+    const HeadArgs h{labels, logp, loss, g_logits, head_ws, loss_mailbox, mailbox_counter};
+    const SweepArgs sw{g_scale, bwd_workspace, bwd_workspace_bytes};
+    return forward_impl(d, x, W_in, W_rec, rec_mask, beta, W_out, b_out, V0, a0, Z0, V, a, Z, zbits, y, logits, tstar,
+                        workspace, workspace_bytes, run_table, W_effT_out, stream, &h, &sw);
 }
 
 int snnk_head_nll(int32_t B, int32_t O, const float* logits, const int64_t* labels, float* logp, float* loss,
@@ -1329,20 +1420,24 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
     if (rc != SNNK_OK) return rc;
     // sigma' trace: it arrives in `a` and is the only trace of V a LIF / ALIF sweep reads (Izhikevich still needs V)
     const bool trace = d->surrogate == SNNK_SURROGATE_TRACE, izh = d->layer_type == SNNK_IZHIKEVICH;
+    // the sweep already ran in snnk_forward_nll_sweep: its outputs are in the workspace, the traces are not read
+    const bool done = (d->flags & SNNK_F_SWEEP_DONE) != 0;
     if (!x || !W_out || !zbits || !dW_in || !dW_out || !db || !workspace) return SNNK_ERR_ARG;
-    if ((!trace || izh) && !V) return SNNK_ERR_ARG;
+    if ((!trace || izh) && !V && !done) return SNNK_ERR_ARG;
     if (trace && !a) return SNNK_ERR_ARG;
     if (d->recurrent && (!W_rec || !dW_rec)) return SNNK_ERR_ARG;
     if (d->recurrent && (d->flags & SNNK_F_TENSOR_CORE) && !Z) return SNNK_ERR_ARG;
-    if (!trace && d->layer_type == SNNK_ALIF && (!beta || !a)) return SNNK_ERR_ARG;
+    if (!trace && d->layer_type == SNNK_ALIF && (!beta || !a) && !done) return SNNK_ERR_ARG;
     const bool dense = g_y != nullptr, sparse = g_logits != nullptr && tstar != nullptr;
     if (dense == sparse) return SNNK_ERR_ARG;
     if (!device_ok()) return SNNK_ERR_DEVICE;
     const Plan pl = make_plan(d);
+    if (done && (dense || !sweep_eligible(d, pl))) return SNNK_ERR_UNSUPPORTED;
     if (workspace_bytes < pl.bwd_bytes) return SNNK_ERR_WORKSPACE;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     char* ws = static_cast<char*>(workspace);
     float* gI = reinterpret_cast<float*>(ws + pl.off_gI);
+    float* gI_lo = pl.tc ? reinterpret_cast<float*>(ws + pl.off_gIlo) : nullptr;
     float* pwout = reinterpret_cast<float*>(ws + pl.off_pwout);
     float* pdb = reinterpret_cast<float*>(ws + pl.off_pdb);
     float* pw = reinterpret_cast<float*>(ws + pl.off_pw);
@@ -1359,7 +1454,7 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
         if (rc != SNNK_OK) return rc;
     }
     // dedup variant: the compact rows of x for the dW_in GEMM do not depend on the sweep -- gathered beside it
-    if (runs) {
+    if (runs && !done) {
         SNNK_CUDA(cudaEventRecord(fk->forked, st));
         SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked, 0));
         k_gather_rows<<<std::min(pl.run_rows, 8 * sm_count()), 256, 0, fk->side>>>(
@@ -1367,71 +1462,61 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
         SNNK_CUDA(cudaGetLastError());
         SNNK_CUDA(cudaEventRecord(fk->mid, fk->side));
     }
-    // K3: reverse-time sweep
-    const float* W_effT = nullptr;
-    if (rec && W_effT_in) {
-        W_effT = W_effT_in;      // prepared by snnk_forward of the same weights (its W_effT_out)
-    } else if (rec) {
-        float* wt = reinterpret_cast<float*>(ws + pl.off_weffT);
-        const int n = d->H * d->H;
-        k_prep_rec<<<(n + 255) / 256, 256, 0, st>>>(W_rec, rec_mask, d->H, nullptr, wt);
-        SNNK_CUDA(cudaGetLastError());
-        W_effT = wt;
-    }
-    BwdParams bp{};
-    bp.B = d->B; bp.T = d->T; bp.H = d->H; bp.O = d->O;
-    bp.alif = d->layer_type == SNNK_ALIF && !trace; bp.surrogate = d->surrogate;
-    bp.iz = izh_consts(d);
-    bp.alpha = d->alpha; bp.theta = d->theta; bp.gamma = d->gamma; bp.kappa = d->kappa;
-    bp.W_effT = W_effT; bp.beta = beta; bp.W_out = W_out; bp.Z0 = Z0;
-    const bool sg_in_v = trace && !izh;     // LIF / ALIF: the LIF-mode sweep reads sigma' in the V slot
-    bp.V = sg_in_v ? a : V; bp.a = sg_in_v ? nullptr : a; bp.zbits = zbits; bp.g_y = g_y;
-    bp.g_logits = dense ? nullptr : g_logits;
-    bp.tstar = dense ? nullptr : tstar; bp.g_scale = g_scale; bp.g_V = g_V; bp.g_Z = g_Z;
-    float* gI_lo = pl.tc ? reinterpret_cast<float*>(ws + pl.off_gIlo) : nullptr;
-    bp.gI = gI; bp.gI_lo = gI_lo; bp.part_wout = pwout; bp.part_db = pdb;
-    if (runs) {
-        bp.run_table = runs;
-        bp.Gu_hi = reinterpret_cast<float*>(ws + pl.off_gu);
-        bp.Gu_lo = reinterpret_cast<float*>(ws + pl.off_gu + pl.gu_plane);
-    }
-    switch (pl.family) {
-    case Family::WideTc: {
-        // weight-stationary tensor-core sweep (recur_wide.cuh): adjoint scan, sweep, then dW_out / db from the scan
-        rc = launch_gy_scan(d, bp, gy_scan, st);
-        if (rc != SNNK_OK) return rc;
-        WideBwdParams wp{};
-        wp.B = d->B; wp.T = d->T; wp.H = d->H; wp.O = d->O; wp.alif = bp.alif; wp.surrogate = bp.surrogate;
-        wp.alpha = bp.alpha; wp.theta = bp.theta; wp.gamma = bp.gamma;
-        wp.W = bp.W_effT; wp.beta = bp.beta; wp.W_out = bp.W_out; wp.V = bp.V; wp.a = bp.a; wp.zbits = bp.zbits; wp.Z0 = bp.Z0;
-        wp.gy_scan = gy_scan; wp.g_V = bp.g_V; wp.g_Z = bp.g_Z; wp.gI = bp.gI; wp.gI_lo = bp.gI_lo;
-        wp.gx = reinterpret_cast<float*>(ws + pl.off_gx);
-        wp.gmask = reinterpret_cast<unsigned int*>(ws + pl.off_gmask);
-        wp.flags = reinterpret_cast<unsigned int*>(ws + pl.off_wflags_b);
-        wp.n_mt = pl.w_nmt_b; wp.n_nt = pl.w_nnt;
-        rc = launch_wide_bwd(wp, pl.w_npass_b, st);
-        if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
-        break;
-    }
-    case Family::WideGen:
-        rc = launch_bwd_gen(d, bp, rec, pl, gy_scan, st);
-        if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
-        break;
-    case Family::TcRec:
-    case Family::NonRec:
-        // readout-adjoint scan first; dW_out / db (a contraction of it with the spike raster) beside the sweep
-        rc = launch_gy_scan(d, bp, gy_scan, st);
-        if (rc != SNNK_OK) return rc;
-        SNNK_CUDA(cudaEventRecord(fk->forked3, st));
-        SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked3, 0));
-        rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, fk->side);
-        if (rc != SNNK_OK) return rc;
-        SNNK_CUDA(cudaEventRecord(fk->joined3, fk->side));
-        rc = pl.family == Family::TcRec ? launch_bwd_tc(bp, gy_scan, st) : launch_nonrec_bwd(bp, gy_scan, st);
-        break;
-    case Family::Simt:
-        rc = use_lean_bwd(bp, rec, pl.R) ? launch_bwd_lean(bp, st) : launch_bwd_simt(bp, rec, pl, st);
-        break;
+    if (!done) {   // K3: reverse-time sweep
+        const float* W_effT = nullptr;
+        if (rec && W_effT_in) {
+            W_effT = W_effT_in;      // prepared by snnk_forward of the same weights (its W_effT_out)
+        } else if (rec) {
+            float* wt = reinterpret_cast<float*>(ws + pl.off_weffT);
+            const int n = d->H * d->H;
+            k_prep_rec<<<(n + 255) / 256, 256, 0, st>>>(W_rec, rec_mask, d->H, nullptr, wt);
+            SNNK_CUDA(cudaGetLastError());
+            W_effT = wt;
+        }
+        BwdParams bp = sweep_params(d, pl, ws, runs);
+        bp.W_effT = W_effT; bp.beta = beta; bp.W_out = W_out; bp.Z0 = Z0;
+        const bool sg_in_v = trace && !izh;     // LIF / ALIF: the LIF-mode sweep reads sigma' in the V slot
+        bp.V = sg_in_v ? a : V; bp.a = sg_in_v ? nullptr : a; bp.zbits = zbits; bp.g_y = g_y;
+        bp.g_logits = dense ? nullptr : g_logits;
+        bp.tstar = dense ? nullptr : tstar; bp.g_scale = g_scale; bp.g_V = g_V; bp.g_Z = g_Z;
+        switch (pl.family) {
+        case Family::WideTc: {
+            // weight-stationary tensor-core sweep (recur_wide.cuh): adjoint scan, sweep, then dW_out / db from the scan
+            rc = launch_gy_scan(d, bp, gy_scan, st);
+            if (rc != SNNK_OK) return rc;
+            WideBwdParams wp{};
+            wp.B = d->B; wp.T = d->T; wp.H = d->H; wp.O = d->O; wp.alif = bp.alif; wp.surrogate = bp.surrogate;
+            wp.alpha = bp.alpha; wp.theta = bp.theta; wp.gamma = bp.gamma;
+            wp.W = bp.W_effT; wp.beta = bp.beta; wp.W_out = bp.W_out; wp.V = bp.V; wp.a = bp.a; wp.zbits = bp.zbits; wp.Z0 = bp.Z0;
+            wp.gy_scan = gy_scan; wp.g_V = bp.g_V; wp.g_Z = bp.g_Z; wp.gI = bp.gI; wp.gI_lo = bp.gI_lo;
+            wp.gx = reinterpret_cast<float*>(ws + pl.off_gx);
+            wp.gmask = reinterpret_cast<unsigned int*>(ws + pl.off_gmask);
+            wp.flags = reinterpret_cast<unsigned int*>(ws + pl.off_wflags_b);
+            wp.n_mt = pl.w_nmt_b; wp.n_nt = pl.w_nnt;
+            rc = launch_wide_bwd(wp, pl.w_npass_b, st);
+            if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
+            break;
+        }
+        case Family::WideGen:
+            rc = launch_bwd_gen(d, bp, rec, pl, gy_scan, st);
+            if (rc == SNNK_OK) rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, st);
+            break;
+        case Family::TcRec:
+        case Family::NonRec:
+            // readout-adjoint scan first; dW_out / db (a contraction of it with the spike raster) beside the sweep
+            rc = launch_gy_scan(d, bp, gy_scan, st);
+            if (rc != SNNK_OK) return rc;
+            SNNK_CUDA(cudaEventRecord(fk->forked3, st));
+            SNNK_CUDA(cudaStreamWaitEvent(fk->side, fk->forked3, 0));
+            rc = launch_wout_grad(d, pl, zbits, gy_scan, pwout, pdb, fk->side);
+            if (rc != SNNK_OK) return rc;
+            SNNK_CUDA(cudaEventRecord(fk->joined3, fk->side));
+            rc = pl.family == Family::TcRec ? launch_bwd_tc(bp, gy_scan, st) : launch_nonrec_bwd(bp, gy_scan, st);
+            break;
+        case Family::Simt:
+            rc = use_lean_bwd(bp, rec, pl.R) ? launch_bwd_lean(bp, st) : launch_bwd_simt(bp, rec, pl, st);
+            break;
+        }
     }
     if (rc != SNNK_OK) return rc;
     // K4: weight-gradient GEMM (split-K partials over whole samples, then a fixed-order reduction)
@@ -1474,7 +1559,7 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
                     rc = launch_wgrad_tc_any(d, pl.tileN, gb, st_b);
                     if (rc != SNNK_OK) return rc;
                 }
-                SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));   // the gather issued beside the sweep
+                if (!done) SNNK_CUDA(cudaStreamWaitEvent(st, fk->mid, 0));   // the gather issued beside the sweep
                 WgradGeom ga{};
                 ga.x = reinterpret_cast<float*>(ws + pl.off_xu_b); ga.Ztrace = nullptr;
                 ga.g_planes = reinterpret_cast<float*>(ws + pl.off_gu); ga.g_plane_stride = pl.gu_plane;

@@ -184,10 +184,14 @@ def _head_scratch(dev, B: int) -> torch.Tensor:
 def run_forward(
 		c: LayerConsts, x, W_in, W_rec, rec_mask, beta, W_out, b_out, traces: bool = True,
 		state: Optional[Tuple[Optional[torch.Tensor], ...]] = None, labels: Optional[torch.Tensor] = None,
-		want_head_grad: bool = True,
+		want_head_grad: bool = True, sweep_scale: Optional[torch.Tensor] = None,
 ):
 	"""Calls ``snnk_forward`` -- or, with ``labels``, ``snnk_forward_nll`` (forward + fused log_softmax / NLL head).
-	Returns dict(y, V, a, Z, zbits, logits, tstar, I_in, desc[, loss, logp, g_logits])."""
+	Returns dict(y, V, a, Z, zbits, logits, tstar, I_in, desc[, loss, logp, g_logits]).
+
+	With ``sweep_scale`` (labels given, no traces): ``snnk_forward_nll_sweep``, which also runs the BPTT sweep for the
+	loss gradient ``sweep_scale`` and leaves its results in the returned ``sweep_ws`` (for ``run_backward``); V and a
+	are not produced.  Returns None when the library has no such kernel for this layer."""
 	lib = _cabi.lib()
 	_cabi.require_b200(x.device)
 	B, T, N = x.shape
@@ -203,8 +207,9 @@ def run_forward(
 	dev = x.device
 	f32 = dict(dtype=torch.float32, device=dev)
 	alif = c.layer_type != _cabi.SNNK_LIF     # three-state layers: ALIF (V, a, Z) and Izhikevich (V, u, Z)
+	sweep = sweep_scale is not None
 	V = torch.empty((B, T, H), **f32) if traces else None
-	Z = torch.empty((B, T, H), **f32) if traces else None
+	Z = torch.empty((B, T, H), **f32) if (traces or sweep) else None
 	a = torch.empty((B, T, H), **f32) if (traces and alif) else None
 	zbits = torch.empty((B, T, H // 32), dtype=torch.int32, device=dev)
 	y = torch.empty((B, T, O), **f32)
@@ -234,12 +239,19 @@ def run_forward(
 			loss = torch.empty((), **f32)
 			g = torch.empty((B, O), **f32) if want_head_grad else None
 			box = LOSS_MAILBOX if (LOSS_MAILBOX is not None and LOSS_MAILBOX[1].device == dev) else None
-			rc = lib.snnk_forward_nll(
-				*common, _cabi.ptr(labels), _cabi.ptr(logp), _cabi.ptr(loss), _cabi.ptr(g), _cabi.ptr(_head_scratch(dev, B)),
-				ctypes.c_void_p(box[0].data_ptr()) if box else None, _cabi.ptr(box[1]) if box else None,
-				_cabi.stream_ptr())
-			head = dict(loss=loss, logp=logp, g_logits=g)
-	_cabi.check(rc, "snnk_forward" if labels is None else "snnk_forward_nll")
+			head_args = (_cabi.ptr(labels), _cabi.ptr(logp), _cabi.ptr(loss), _cabi.ptr(g), _cabi.ptr(_head_scratch(dev, B)),
+				ctypes.c_void_p(box[0].data_ptr()) if box else None, _cabi.ptr(box[1]) if box else None)
+			if sweep:
+				sweep_ws = _workspace(lib.snnk_backward_workspace_bytes(ctypes.byref(desc)), dev)
+				rc = lib.snnk_forward_nll_sweep(*common, *head_args, _cabi.ptr(sweep_scale), _cabi.ptr(sweep_ws),
+					sweep_ws.numel(), _cabi.stream_ptr())
+				if rc == _cabi.SNNK_ERR_UNSUPPORTED:
+					return None
+				head["sweep_ws"] = sweep_ws
+			else:
+				rc = lib.snnk_forward_nll(*common, *head_args, _cabi.stream_ptr())
+			head.update(loss=loss, logp=logp, g_logits=g)
+	_cabi.check(rc, "snnk_forward" if labels is None else "snnk_forward_nll_sweep" if sweep else "snnk_forward_nll")
 	I_in = ws[: B * T * H * 4].view(torch.float32).view(B, T, H)
 	return dict(y=y, V=V, a=a, Z=Z, zbits=zbits, logits=logits, tstar=tstar, I_in=I_in, desc=desc, Z0=Z0, W_effT=W_effT,
 		**head)
@@ -248,10 +260,12 @@ def run_forward(
 def run_backward(
 		c: LayerConsts, x, W_rec, rec_mask, beta, W_out, V, a, zbits, g_y=None, g_logits=None, tstar=None,
 		g_V=None, g_Z=None, Z0=None, Z=None, g_scale=None, binary_input: bool = False, runs=None, W_effT=None,
+		sweep_ws=None,
 ):
 	"""Calls ``snnk_backward``.  Returns dict(dW_in, dW_rec, dW_out, db, gI) -- ``gI`` is a zero-argument callable
 	(the tensor-core mode stores it as two planes; summing them is only worth it when somebody asks).  For a
-	user-defined surrogate the ``a`` argument of the call is sigma' (surrogate_trace) instead of the saved ``a``."""
+	user-defined surrogate the ``a`` argument of the call is sigma' (surrogate_trace) instead of the saved ``a``.
+	``sweep_ws``: the workspace in which ``run_forward(sweep_scale=...)`` already ran the sweep (SNNK_F_SWEEP_DONE)."""
 	lib = _cabi.lib()
 	if c.surrogate == _cabi.SNNK_SURROGATE_TRACE:
 		a = surrogate_trace(c, V, a, beta)
@@ -267,7 +281,11 @@ def run_backward(
 	dW_rec = torch.empty((H, H), **f32) if c.recurrent else None
 	dW_out = torch.empty((H, O), **f32)
 	db = torch.empty((O,), **f32)
-	ws = _workspace(lib.snnk_backward_workspace_bytes(ctypes.byref(desc)), dev)
+	if sweep_ws is not None:
+		desc.flags |= _cabi.SNNK_F_SWEEP_DONE
+		ws = sweep_ws
+	else:
+		ws = _workspace(lib.snnk_backward_workspace_bytes(ctypes.byref(desc)), dev)
 	with torch.cuda.device(dev):
 		rc = lib.snnk_backward(
 			ctypes.byref(desc), _cabi.ptr(x), _cabi.ptr(W_rec), _cabi.ptr(rec_mask), _cabi.ptr(beta),
@@ -305,6 +323,11 @@ def run_input_grad(c: LayerConsts, gI: torch.Tensor, W_in: torch.Tensor) -> torc
 # (pinned host int64 word, device int32 counter) while a graphed training step is being built: the head kernel then
 # also posts the loss to the host word (include/snnk.h, snnk_head_nll); see modules/graphed.py
 LOSS_MAILBOX = None
+
+# The root gradient (a 0-d device tensor) of the backward call that follows while a graphed training step runs its body
+# (modules/graphed.py): SpikingSequenceNLL then runs the BPTT sweep for that gradient in its forward
+# (snnk_forward_nll_sweep), and its backward keeps the result if it receives that very tensor.
+SWEEP_SCALE = None
 
 
 def run_head_nll(logits: torch.Tensor, labels: torch.Tensor, want_grad: bool = True):
@@ -395,8 +418,15 @@ class SpikingSequenceNLL(torch.autograd.Function):
 		Hp = padded_width(H)
 		Wi, Wr, M, Wo = _pad_hidden(H, Hp, Wi, Wr, M, Wo)
 		need_grad = any(ctx.needs_input_grad)
-		out = run_forward(consts, xc, Wi, Wr, M, be, Wo, bo, traces=traces or need_grad, labels=labels,
-			want_head_grad=need_grad)
+		scale = SWEEP_SCALE
+		out = None
+		if need_grad and not traces and scale is not None and scale.device == xc.device:
+			out = run_forward(consts, xc, Wi, Wr, M, be, Wo, bo, traces=False, labels=labels, sweep_scale=scale)
+		# the sweep ran for `scale`; any other gradient recomputes the traces (same kernels, same values) in backward
+		ctx.sweep = (scale, out["sweep_ws"], Wi, bo) if out is not None else None
+		if out is None:
+			out = run_forward(consts, xc, Wi, Wr, M, be, Wo, bo, traces=traces or need_grad, labels=labels,
+				want_head_grad=need_grad)
 		loss, logp, g_logits = out["loss"], out["logp"], out["g_logits"]
 		ctx.consts, ctx.H = consts, H
 		ctx.set_materialize_grads(False)
@@ -415,9 +445,18 @@ class SpikingSequenceNLL(torch.autograd.Function):
 		xc, Wr, M, be, Wo, V, a, zbits, g_logits, tstar, Z = ctx.saved_tensors
 		if g_loss is None:
 			return (None,) * 10
+		sweep_ws, W_effT = None, ctx.W_effT
+		if ctx.sweep is not None:
+			scale, ws, Wi, bo = ctx.sweep
+			if g_loss.dtype == torch.float32 and g_loss.data_ptr() == scale.data_ptr():
+				sweep_ws = ws
+			else:
+				f = run_forward(ctx.consts, xc, Wi, Wr, M, be, Wo, bo, traces=True)
+				V, a, zbits, Z, W_effT = f["V"], f["a"], f["zbits"], f["Z"], f["W_effT"]
 		g = run_backward(
 			ctx.consts, xc, Wr, M, be, Wo, V, a, zbits, g_logits=g_logits, tstar=tstar, Z=Z,
-			g_scale=g_loss.detach().float().reshape(1), binary_input=ctx.binary, runs=ctx.runs, W_effT=ctx.W_effT)
+			g_scale=g_loss.detach().float().reshape(1), binary_input=ctx.binary, runs=ctx.runs, W_effT=W_effT,
+			sweep_ws=sweep_ws)
 		H = ctx.H
 		gX = run_input_grad(ctx.consts, g["gI"](), ctx.Wi) if ctx.Wi is not None else None
 		return (None, gX, None, g["dW_in"][:, :H], None if g["dW_rec"] is None else g["dW_rec"][:H, :H], None, None,

@@ -151,9 +151,17 @@ class GraphedTrainStep:
 
 	def _body(self, x=None, y=None) -> torch.Tensor:
 		net = self.net
-		loss = net.batch_loss(self.x if x is None else x, self.y if y is None else y, self.criterion)
-		self.optimizer.zero_grad(set_to_none=True)
-		loss.backward(gradient=_const_scalar(1.0, loss.device))     # cached root gradient: no ones_like fill per step
+		x = self.x if x is None else x
+		root = _const_scalar(1.0, x.device)      # cached root gradient: no ones_like fill per step
+		# published while the body runs: the fused training path of the loss runs the BPTT sweep for this gradient in its
+		# forward kernel, and its backward uses that sweep when it receives this tensor
+		F_.SWEEP_SCALE = root
+		try:
+			loss = net.batch_loss(x, self.y if y is None else y, self.criterion)
+			self.optimizer.zero_grad(set_to_none=True)
+			loss.backward(gradient=root)
+		finally:
+			F_.SWEEP_SCALE = None
 		net._allreduce_gradients(self.optimizer)
 		if self.step_in_graph:
 			self.optimizer.step()
