@@ -291,7 +291,10 @@ int snnk_forward_nll_sweep(const SnnkDesc* d, const float* x, const float* W_in,
  * Gradient seeds: either g_y (B,T,O) dense w.r.t. the output trace, or -- the fused-head form --
  * g_logits (B,O) with tstar (B,O) (the gradient lands on y[b,tstar[b,o],o]), optionally multiplied by
  * the device scalar g_scale (dL/dloss handed in by autograd; NULL = 1).  Exactly one of the two forms
- * must be given.  g_V, g_Z (B,T,H) are optional extra seeds on the hidden traces.
+ * must be given.  g_V, g_Z (B,T,H) are optional extra seeds on the hidden traces.  Z0 (B,H) is the initial spike
+ * state the forward was given (NULL = zeros): it stands in for Z_{-1} in dW_rec and in the ALIF adaptation.  With
+ * SNNK_F_TENSOR_CORE the weight-gradient GEMM reads Z_{-1} as zeros and the final reduction adds
+ * sum_b Z0[b]^T gI[b,0,:] to dW_rec (B*H*H extra FMAs, only when Z0 is given).
  * V, a (ALIF), Z (B,T,H) and zbits are the traces the forward wrote (Z, the fp32 spike trace, is read by the
  * tensor-core weight-gradient GEMM only and may be NULL without SNNK_F_TENSOR_CORE).
  * With surrogate SNNK_SURROGATE_TRACE, `a` instead holds sigma'_t = dZ_t/dV_t (B,T,H), the surrogate derivative the

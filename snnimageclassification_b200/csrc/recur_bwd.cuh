@@ -295,6 +295,10 @@ struct FinalizeParams {
     // frame-dedup variant (runs.cuh): when run_table says ok, dW_rec comes from its own partial buffer instead
     const int* run_table; const float* pw_rec; int S_rec; size_t rec_stride;
     int S_cmp;   // number of dW_in partials the compact GEMM wrote (same buffer and stride as the dense ones)
+    // The tcgen05 GEMMs read Z_{-1} as zeros (TMA fills t < 0), so the Z0 term of dW_rec is added here:
+    // dW_rec[j][n] += sum_b Z0[b][j] (gI + gI_lo)[b, 0, n].  Z0 is null when the partials already hold it (SIMT K4);
+    // a raised inexact flag means k_wgrad_simt redid them, Z0 included.
+    const float* Z0; const float* gI; const float* gI_lo; const unsigned int* inexact_flag; int B, H; size_t row_stride;
     // (b) warp per element, many partials:   dW_out (n_out elements, P_out partials) then db (n_b, P_b partials)
     const float* pwout; int P_out; int n_out; float* dW_out;
     const float* pdb; int P_b; int n_b; float* db;
@@ -342,8 +346,17 @@ __global__ void __launch_bounds__(256) k_finalize_grads(const FinalizeParams p)
             p.dW_in[e] = sum_partials_seq(p.pw + e, compact ? p.S_cmp : p.S, p.w_stride);
         } else if (e - p.n_in < p.n_rec) {
             const int r = e - p.n_in;
-            const float s = (compact && p.pw_rec) ? sum_partials_seq(p.pw_rec + r, p.S_rec, p.rec_stride)
-                                    : sum_partials_seq(p.pw + p.n_in + r, p.S, p.w_stride);
+            float s = (compact && p.pw_rec) ? sum_partials_seq(p.pw_rec + r, p.S_rec, p.rec_stride)
+                              : sum_partials_seq(p.pw + p.n_in + r, p.S, p.w_stride);
+            if (p.Z0 && !(p.inexact_flag && *p.inexact_flag != 0)) {
+                const int j = r / p.H, n = r - j * p.H;
+                float c = 0.f;
+                for (int b = 0; b < p.B; ++b) {
+                    const size_t g = (size_t)b * p.row_stride + n;
+                    c = fmaf(__ldg(p.Z0 + (size_t)b * p.H + j), __ldg(p.gI + g) + __ldg(p.gI_lo + g), c);
+                }
+                s += c;
+            }
             p.dW_rec[r] = p.rec_mask ? s * __ldg(p.rec_mask + r) : s;
         }
         return;

@@ -1596,6 +1596,10 @@ int snnk_backward(const SnnkDesc* d, const float* x, const float* W_rec, const f
                 fz.rec_stride = (size_t)d->H * d->H;
             }
         }
+        if (rec && Z0 && (pl.bits || pl.tc)) {   // the tcgen05 GEMMs leave out the t = 0 term of dW_rec
+            fz.Z0 = Z0; fz.gI = gI; fz.gI_lo = gI_lo; fz.inexact_flag = flag;
+            fz.B = d->B; fz.H = d->H; fz.row_stride = (size_t)d->T * d->H;
+        }
         fz.blocks_a = (fz.n_in + fz.n_rec + 255) / 256;
         const int blocks_b = (fz.n_out + fz.n_b + 7) / 8;
         return launch(SNNK_K_REDUCE_W, k_finalize_grads, fz.blocks_a + blocks_b, 256, 0, st, fz);

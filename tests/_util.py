@@ -1,5 +1,6 @@
-"""Shared helpers for the test-suite: fixture loading and parity metrics."""
+"""Shared helpers for the test-suite: fixture loading, parity metrics, kernel selection and guard bands."""
 import os
+import re
 
 import numpy as np
 
@@ -68,3 +69,57 @@ def unexplained_forks(Z_test, Z_ref, V_ref, thr_ref, tol=2e-5):
 		if np.any(np.abs(v - th) > tol * np.maximum(np.abs(th), np.abs(v))):
 			unexplained += 1
 	return forked, unexplained
+
+
+# ---- which kernels ran -----------------------------------------------------------------------------------------------
+def launched(fn):
+	"""Runs ``fn()`` under torch.profiler with CUDA activity and returns (its result, the names of the device kernels it
+	launched).  A profile without any kernel of the library fails: a selection test must not pass on an empty list."""
+	import torch
+	from torch.autograd import DeviceType
+	torch.cuda.synchronize()
+	with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+		# Late in a long session the profiler can lose the first few device records of a window (a list without the
+		# first kernels of fn, or an empty one); a few throw-away kernels take that place.
+		pad = torch.zeros(1, device="cuda")
+		for _ in range(16):
+			pad.add_(1.0)
+		torch.cuda.synchronize()
+		res = fn()
+		torch.cuda.synchronize()
+	names = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA]
+	assert any("snnk::" in n for n in names), f"the profiler reports no kernel of the library: {names[:8]}"
+	return res, names
+
+
+def ran(names, pattern):
+	return any(re.search(pattern, n) for n in names)
+
+
+# ---- guard bands -------------------------------------------------------------------------------------------------------
+GUARD = 4096          # bytes on each side
+SENT = 0xA5
+
+
+class Guarded:
+	"""A tensor of `shape` on cuda:0 carved out of a byte buffer with GUARD sentinel bytes in front of and behind it."""
+
+	def __init__(self, shape, dtype=None, fill_inside=True):
+		import torch
+		dtype = torch.float32 if dtype is None else dtype
+		n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
+		pad = (-n) % 256
+		self.raw = torch.full((GUARD + n + pad + GUARD,), SENT, dtype=torch.uint8, device="cuda:0")
+		self.n, self.pad = n, pad
+		self.t = self.raw[GUARD:GUARD + n].view(dtype).view(shape)
+
+	def check(self, name, written=True):
+		import torch
+		front, back = self.raw[:GUARD], self.raw[GUARD + self.n:]
+		assert bool((front == SENT).all()), f"{name}: write in front of the buffer"
+		assert bool((back == SENT).all()), f"{name}: write behind the buffer"
+		if written and self.t.dtype == torch.float32:
+			# 0xA5A5A5A5 as a float is -2.87e-16: exact sentinel words inside mean unwritten elements
+			words = self.raw[GUARD:GUARD + self.n].view(torch.int32)
+			assert int((words == int(np.array([0xA5A5A5A5], dtype=np.uint32).view(np.int32)[0])).sum()) == 0, f"{name}: unwritten elements"
+			assert bool(torch.isfinite(self.t).all()), f"{name}: non-finite values"

@@ -18,32 +18,9 @@ pytestmark = pytest.mark.gpu
 
 from snnimageclassification_b200 import ToSpikes, _cabi  # noqa: E402
 from snnimageclassification_b200.modules import functional as F_  # noqa: E402
+from _util import Guarded  # noqa: E402
 
 DEV = torch.device("cuda:0")
-GUARD = 4096          # bytes on each side
-SENT = 0xA5
-
-
-class Guarded:
-	"""A tensor of `shape` carved out of a byte buffer with GUARD sentinel bytes in front of and behind it."""
-
-	def __init__(self, shape, dtype=torch.float32, fill_inside=True):
-		n = int(np.prod(shape)) * torch.empty((), dtype=dtype).element_size()
-		pad = (-n) % 256
-		self.raw = torch.full((GUARD + n + pad + GUARD,), SENT, dtype=torch.uint8, device=DEV)
-		self.n, self.pad = n, pad
-		self.t = self.raw[GUARD:GUARD + n].view(dtype).view(shape)
-		assert self.t.data_ptr() % 256 == 0 or True
-
-	def check(self, name, written=True):
-		front, back = self.raw[:GUARD], self.raw[GUARD + self.n:]
-		assert bool((front == SENT).all()), f"{name}: write in front of the buffer"
-		assert bool((back == SENT).all()), f"{name}: write behind the buffer"
-		if written and self.t.dtype == torch.float32:
-			# 0xA5A5A5A5 as a float is -2.87e-16: exact sentinel words inside mean unwritten elements
-			words = self.raw[GUARD:GUARD + self.n].view(torch.int32)
-			assert int((words == int(np.array([0xA5A5A5A5], dtype=np.uint32).view(np.int32)[0])).sum()) == 0, f"{name}: unwritten elements"
-			assert bool(torch.isfinite(self.t).all()), f"{name}: non-finite values"
 
 
 def _run(B, T, N, H, O, layer, rec, tc, dedup, monkeypatch=None):

@@ -15,12 +15,11 @@ import re
 import numpy as np
 import pytest
 import torch
-from torch.autograd import DeviceType
 
 import oracle
 from oracle import OracleCfg
 from oracle.torch_port import TorchPortSNN
-from _util import elementwise_err, rel_err, unexplained_forks
+from _util import elementwise_err, launched, ran, rel_err, unexplained_forks
 
 pytestmark = pytest.mark.gpu
 
@@ -34,23 +33,6 @@ ALPHA, RHO, KAPPA = (float(np.float32(np.exp(-1 / k))) for k in (20, 200, 10))
 
 def npy(t):
 	return None if t is None else t.detach().cpu().numpy()
-
-
-# ---- which kernels ran -----------------------------------------------------------------------------------------------
-def launched(fn):
-	"""Runs ``fn()`` under torch.profiler with CUDA activity and returns (its result, the names of the device kernels it
-	launched).  A profile without any kernel of the library fails: a selection test must not pass on an empty list."""
-	torch.cuda.synchronize()
-	with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
-		res = fn()
-		torch.cuda.synchronize()
-	names = [e.name for e in prof.events() if e.device_type == DeviceType.CUDA]
-	assert any("snnk::" in n for n in names), f"the profiler reports no kernel of the library: {names[:8]}"
-	return res, names
-
-
-def ran(names, pattern):
-	return any(re.search(pattern, n) for n in names)
 
 
 def _targ(s):
